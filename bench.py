@@ -2,6 +2,7 @@
 """bench.py -- dual-arm grasp IK solves/s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dtype f32|f64] [--config 2|3|4|5]
+                    [--dump-outputs DIR]
 
 A "step" is ONE pass of the hot path over one batch of synthetic input: BASELINE config 2, 2^20 random cube
 placements over the table workspace (identity rotation, path.py:47), every problem started from q0 = 0,
@@ -15,7 +16,12 @@ the reference itself needs pinocchio, absent from this image) on the box's host 
 the rest of the metric: config 2 in fp64, config 3 (restarts, fp64, damped), config 4 (edge projection), the full
 success predicate (collision term + the reference's keep-descending tail) and, for N > 1, config 5 (the 64 Mi-problem
 strong-scaling sweep, fused scatter and NCCL gather) with a fused == all_gather check.
-`--impl reference` times the CPU port alone."""
+`--impl reference` times the CPU port alone.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (rank 0's slab) as DIR/<name>.npy,
+float64 arrays as float64 and everything else as float32, the problem index on the last axis.  The inputs are seeded,
+so two builds run with the same arguments can be compared array for array.  Above 64 MB in all, every array keeps the
+same seeded sample of problems, listed in problem_index.npy."""
 import argparse
 import json
 import os
@@ -62,7 +68,12 @@ def parse():
     ap.add_argument("--step", default="auto", choices=["auto", "cholesky"],
                     help="form of the undamped step: auto = spherical-wrist 3x3 solves where the table allows it (default), "
                          "cholesky = always the general 6x6 block-Cholesky form (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy; b200 arm only, since the "
+                         "reference arm times a CPU port whose results the tests already compare")
     args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200 and --steps >= 1")
     if args.dtype is None:
         args.dtype = "f64" if args.config == 3 else "f32"
     return args
@@ -226,7 +237,8 @@ def pose_rows_from(torch, pos):
 class Workload:
     """One BASELINE config on one rank: `launch()` enqueues the kernels of one step on the current stream and
     returns the tensors a gather would ship; `solves` = problems solved per step on this rank; `iterations()` = descent
-    iterations executed by the last step (device scalar); `converged()` = fraction converged."""
+    iterations executed by the last step (device scalar); `converged()` = fraction converged; `outputs()` = name ->
+    tensor of every result the last step returned, problem index on the last axis."""
     name = ""
     solves = 0
     kernel_choice = None
@@ -254,6 +266,9 @@ class Config2(Workload):
         q, conv, _, _ = self.solver.solve_soa(self.q0, self.pose, out=self.out, kernel=self.kernel_choice,
                                               early_stop=self.early_stop)
         return q, conv
+
+    def outputs(self):
+        return dict(zip(("q", "converged", "iterations", "residual"), self.out))
 
     def iterations(self):
         return self.out[2].sum(dtype=self.torch.int64).double()
@@ -290,6 +305,9 @@ class Config3(Workload):
         q, conv, _, resid = self.solver.solve_soa(self.q0, self.pose, out=self.out, damping=self.DAMPING, kernel=self.kernel_choice)
         self.best = self.solver.best_of_soa(q, conv, resid, self.n_place, self.R)
         return self.best[0], self.best[1]
+
+    def outputs(self):
+        return dict(zip(("q_best", "converged", "restart"), self.best))
 
     def iterations(self):
         return self.out[2].sum(dtype=self.torch.int64).double()
@@ -328,6 +346,9 @@ class Config4(Workload):
     def launch(self):
         self.res = self.solver.project_edges_soa(self.q_start, self.pose_a, self.pose_b, self.ns, self.S, kernel=self.kernel_choice)
         return self.res[0], self.res[1]
+
+    def outputs(self):
+        return dict(zip(("q_path", "n_valid", "iterations"), self.res))
 
     def executed(self):
         nv = self.res[1]
@@ -447,6 +468,28 @@ class Runner:
         if self.world > 1:
             self.dist.all_reduce(st)
         return st.tolist()
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES, seed=0):
+    """Writes every tensor of `arrays` (problem index on the last axis) as out_dir/<name>.npy: float64 tensors as
+    float64, all others as float32, and problem_index.npy (float64) with the problems kept.  When all of them would
+    exceed `budget` bytes, every array keeps the same seeded sample of problems, in ascending order."""
+    import numpy as np
+    import torch
+    n = next(iter(arrays.values())).shape[-1]
+    if any(t.shape[-1] != n for t in arrays.values()):
+        raise ValueError("dump_outputs: the arrays disagree on the problem count")
+    per_problem = 8 + sum((8 if t.dtype == torch.float64 else 4) * (t.numel() // max(n, 1)) for t in arrays.values())
+    k = min(n, (budget - 256 * (len(arrays) + 1)) // per_problem)      # 256: room for each file's .npy header
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.index_select(t.dim() - 1, torch.from_numpy(idx).to(t.device)).cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (a.double() if t.dtype == torch.float64 else a.float()).numpy())
+    np.save(os.path.join(out_dir, "problem_index.npy"), idx.astype(np.float64))
 
 
 def roofline_of(gik_b200, solver, wl, dtype, esz, kernel_ms, iters_per_launch, solves_per_launch, peak, kernel_choice):
@@ -584,6 +627,11 @@ def run_b200(args):
         sampler.stop()
     if fused is not None:     # the local flags live in the symmetric array: bring this rank's slab back for the stats
         wl.out[1].copy_(fused.conv[gather_off:gather_off + wl.solves])
+    if args.dump_outputs is not None and rank == 0:
+        outs = wl.outputs()
+        if fused is not None:
+            outs["q"] = fused.q[:, gather_off:gather_off + wl.solves]
+        dump_outputs(args.dump_outputs, outs)
     ms_per_step = ms_total / max(args.steps, 1)
     conv_solves, iters_sum, solves_all = R.stats(wl)          # per step, all ranks
     conv_frac = conv_solves / solves_all

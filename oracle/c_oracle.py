@@ -2,9 +2,12 @@
 Row-major numpy in/out, fp64.  The table argument is any ctypes struct laid out like gik_table_t."""
 from __future__ import annotations
 
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -31,9 +34,26 @@ LIB = os.path.join(_HERE, "_build", f"liboracle-{_cpu_tag()}.so")
 _lib = None
 
 
+def _writable(d):
+    try:
+        os.makedirs(d, exist_ok=True)
+    except OSError:
+        return False
+    return os.access(d, os.W_OK)
+
+
 def build(force=False):
+    """Builds the library when it is missing or older than its sources.  Where oracle/_build cannot be written (a
+    read-only checkout), it goes to a temporary directory that is removed when the process exits: bench.py's CPU
+    baseline and smoke() then run from such a checkout.  The test suite still needs a writable one (it also builds
+    tests/hostsim/_build)."""
+    global LIB
     srcs = [os.path.join(_HERE, f) for f in ("grasp_ik_oracle.c", "collision_oracle.inc")]
     if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < max(os.path.getmtime(s) for s in srcs):
+        if not _writable(os.path.dirname(LIB)):
+            d = tempfile.mkdtemp(prefix="gik-oracle-")
+            atexit.register(shutil.rmtree, d, True)
+            LIB = os.path.join(d, os.path.basename(LIB))
         subprocess.run(["make", "-C", _HERE, "-B" if force else "-s", f"OUT={LIB}"], check=True, capture_output=True)
     return LIB
 

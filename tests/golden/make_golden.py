@@ -12,6 +12,8 @@
   nextage_table.json  -- the kinematic table flattened from the reference's URDFs
                          (models/nextagea_description/urdf/NextageaOpen.urdf, models/cubes/cube_small.urdf)
                          with ROBOT_PLACEMENT (config.py:33) applied as in setup_pinocchio.py:28-32.
+  nextage_scene.json  -- the collision scene flattened from the reference's URDF/SRDF files (scene.reference_scene_from);
+                         the package ships the same file as data/nextage_scene.json.
 The fixtures are data; no reference source code is copied."""
 import json
 import os
@@ -51,11 +53,12 @@ def main(ref):
                              os.path.join(ref, "models/cubes/cube_small.urdf"))
     json.dump(tab.to_json(), open(os.path.join(HERE, "nextage_table.json"), "w"), indent=1)
     from gik_b200 import scene
+    sc = scene.reference_scene_from(ref).to_json()
+    json.dump(sc, open(os.path.join(HERE, "nextage_scene.json"), "w"))
     os.makedirs(os.path.join(HERE, "..", "..", "motion-planning-and-control-for-dual-manipulator-robot_b200", "data"), exist_ok=True)
-    json.dump(scene.reference_scene_from(ref).to_json(),
-              open(os.path.join(HERE, "..", "..", "motion-planning-and-control-for-dual-manipulator-robot_b200", "data",
-                                "nextage_scene.json"), "w"))
-    print("wrote ik_golden.json, trajectory2_reference.json, nextage_table.json, data/nextage_scene.json")
+    json.dump(sc, open(os.path.join(HERE, "..", "..", "motion-planning-and-control-for-dual-manipulator-robot_b200", "data",
+                                    "nextage_scene.json"), "w"))
+    print("wrote ik_golden.json, trajectory2_reference.json, nextage_table.json, nextage_scene.json, data/nextage_scene.json")
 
 
 if __name__ == "__main__":

@@ -31,11 +31,60 @@ def test_scene_matches_reference_construction(scene):
     assert frozenset(("CHEST_JOINT0_Link", "nextage_base")) not in links
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference checkout not present")
 def test_packaged_scene_equals_flattened_reference_urdfs(scene):
+    # nextage_scene.json: reference_scene_from(<reference checkout>).to_json(), stored by tests/golden/make_golden.py
+    ref = json.load(open(os.path.join(GOLDEN, "nextage_scene.json")))
+    assert json.dumps(ref, sort_keys=True) == json.dumps(scene.to_json(), sort_keys=True)
+
+
+def test_scene_from_urdf_geometry_order_placements_and_pairs(tmp_path):
     from gik_b200 import scene as sm
-    ref = sm.reference_scene_from("/root/reference")
-    assert json.dumps(ref.to_json(), sort_keys=True) == json.dumps(scene.to_json(), sort_keys=True)
+    from gik_b200.model import rpy_to_matrix
+
+    def write(name, text):
+        (tmp_path / name).write_text(text)
+        return str(tmp_path / name)
+
+    def col(shape, xyz="0 0 0"):
+        return f'<collision><origin xyz="{xyz}"/><geometry>{shape}</geometry></collision>'
+
+    box, sph, cyl = '<box size="0.2 0.4 0.6"/>', '<sphere radius="0.05"/>', '<cylinder radius="0.1" length="0.4"/>'
+    # children are visited in joint-name order (J0 before J1); a fixed joint's geometry joins its parent joint
+    robot = write("r.urdf", f"""<robot name="r">
+      <link name="base">{col(box, "0 0 0.1")}{col(sph)}{col(cyl, "0 0 -0.3")}</link>
+      <link name="l1">{col(cyl)}</link><link name="l1b">{col(box, "0.1 0 0")}</link><link name="l0">{col(sph, "0.1 0 0")}</link>
+      <joint name="J1" type="revolute"><parent link="base"/><child link="l1"/><origin xyz="0 1 0"/><axis xyz="0 0 1"/></joint>
+      <joint name="F" type="fixed"><parent link="l1"/><child link="l1b"/><origin xyz="0 0 0.5" rpy="0 0 1.5708"/></joint>
+      <joint name="J0" type="revolute"><parent link="base"/><child link="l0"/><origin xyz="1 0 0"/><axis xyz="1 0 0"/></joint>
+    </robot>""")
+    srdf = write("r.srdf", '<robot name="r"><disable_collisions link1="l1b" link2="l0" reason="Adjacent"/></robot>')
+    table = write("t.urdf", f'<robot name="t"><link name="baseLink">{col(box, "0 0 0.2")}</link></robot>')
+    obstacle = write("o.urdf", f'<robot name="o"><link name="obstaclebase">{col(sph)}</link></robot>')
+    cube = write("c.urdf", '<robot name="c"><link name="cubebase"><collision><geometry><mesh filename="cube.stl" '
+                           'scale="0.04 0.04 0.04"/></geometry></collision></link></robot>')
+    rz = rpy_to_matrix([0, 0, -np.pi / 2])
+    s = sm.scene_from_urdf(robot, srdf, table, obstacle, cube, robot_placement=(np.eye(3), np.array([0, 0, 0.85])),
+                           table_placement=(rz, np.array([0.8, 0, 0])), obstacle_placement=(np.eye(3), np.array([0.4, 0, 0.9])),
+                           cube_placement=(np.eye(3), np.array([0.33, -0.3, 0.93])))
+    assert [g.name for g in s.geoms] == ["base_0", "base_1", "base_2", "l0_0", "l1_0", "l1b_0", "baseLink_0",
+                                         "obstaclebase_0", "cubebase_0"]
+    assert [g.joint for g in s.geoms] == [-1, -1, -1, 0, 1, 1, -1, -1, -1]
+    assert [g.type for g in s.geoms] == [BOX, SPH, CYL, SPH, CYL, BOX, BOX, SPH, BOX]
+    assert (s.table, s.obstacle, s.cube) == (6, 7, 8)
+    assert np.allclose(s.geoms[0].size, [0.1, 0.2, 0.3]) and np.allclose(s.geoms[1].size, [0.05, 0, 0])
+    assert np.allclose(s.geoms[2].size, [0.1, 0.2, 0]) and np.allclose(s.geoms[8].size, [0.02, 0.02, 0.02])
+    # the robot placement moves only the first two root geometries
+    assert np.allclose(s.geoms[0].p, [0, 0, 0.95]) and np.allclose(s.geoms[1].p, [0, 0, 0.85])
+    assert np.allclose(s.geoms[2].p, [0, 0, -0.3])
+    # moving-joint geometries are expressed in their joint's frame, fixed-joint offsets composed in
+    assert np.allclose(s.geoms[3].p, [0.1, 0, 0]) and np.allclose(s.geoms[4].p, 0)
+    assert np.allclose(s.geoms[5].p, [0, 0.1, 0.5], atol=1e-5) and np.allclose(s.geoms[5].R, rpy_to_matrix([0, 0, 1.5708]))
+    assert np.allclose(s.geoms[6].p, [0.8, 0, 0.2]) and np.allclose(s.geoms[6].R, rz)
+    assert np.allclose(s.geoms[7].p, [0.4, 0, 0.9]) and np.allclose(s.geoms[8].p, [0.33, -0.3, 0.93])
+    # all pairs on different joints, minus the SRDF-disabled (l0, l1b), plus (obstacle, cube)
+    assert [tuple(p) for p in s.pairs] == [(0, 3), (0, 4), (0, 5), (1, 3), (1, 4), (1, 5), (2, 3), (2, 4), (2, 5), (3, 4),
+                                           (3, 6), (3, 7), (3, 8), (4, 6), (4, 7), (4, 8), (5, 6), (5, 7), (5, 8), (7, 8)]
+    assert json.dumps(sm.CollisionScene.from_json(s.to_json()).to_json()) == json.dumps(s.to_json())
 
 
 def test_oracle_pair_distances_against_closed_forms(c_oracle):
