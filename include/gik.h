@@ -315,6 +315,59 @@ int gik_bezier_fit_f64(gik_handle_t h, int64_t n_paths, int32_t n_points, int32_
                        const double* basis, const double* w0, const double* w1, const double* q0, const double* q1,
                        const double* path, double* ctrl, double* cost, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * RRT-connect trees on the device (computepath, path.py:186-278, for many queries at once).  n_trees trees of capacity
+ * cap share one set of arrays, component-major like every batch array above:
+ *   verts  [n_trees][nq][cap]   vertex configurations (nq = the handle's table)
+ *   cubes  [n_trees][12][cap]   cube placement each configuration was solved for
+ *   parent [n_trees][cap]       int32, -1 = root
+ *   n_verts[n_trees]            int32, vertices in use (a tree is reset by setting it back to 1: its root stays at 0)
+ * A planner of Q queries uses tree i as the start tree and tree Q + i as the goal tree of query i.
+ * ------------------------------------------------------------------------------------------------------- */
+
+/* Replaces the nearest-vertex query of computepath (the reference's KDTree query, path.py:186-192): for each of the
+ * n_targets rows of targets [n_targets][nq] (row-major), nearest[t] = the vertex of tree target_tree[t] with the
+ * smallest squared distance, ties to the lowest index (numpy's argmin).  Distances are fp64 whatever the storage
+ * type, summed in numpy's order for nq = 15 so that the choice is numpy's bit for bit.  nearest[t] = -1 when the tree
+ * id is out of range or the tree is empty. */
+int gik_tree_nearest_f32(gik_handle_t h, int64_t n_trees, int32_t cap, const float* verts, const int32_t* n_verts,
+                         int64_t n_targets, const float* targets, const int32_t* target_tree, int32_t* nearest, void* stream);
+int gik_tree_nearest_f64(gik_handle_t h, int64_t n_trees, int32_t cap, const double* verts, const int32_t* n_verts,
+                         int64_t n_targets, const double* targets, const int32_t* target_tree, int32_t* nearest, void* stream);
+
+/* Replaces grow() of computepath (path.py:241-244): appends the output of one gik_project_edges_* launch to the trees.
+ * Edge e belongs to tree edge_tree[e] (the edges of one tree are consecutive and are appended in edge order) and
+ * starts at vertex near[e]; q_start [nq][E], pose_a / pose_b [12][E], num_steps [E] and q_path [max_steps][nq][E] are
+ * the edge launch's inputs and output, n_valid [E] its step counts after any cut (path.py:144-156).  Each segment
+ * appends q_start[:, e] again as a child of near[e], then its n_valid[e] steps, each the child of the previous one.
+ * The placement of step j is computed as in the edge kernel (SE3 interpolation at alpha = (j+1) / num_steps[e]), so it
+ * is the placement the step was solved for.  n_valid[e] < 0 = no segment for this edge.  seg_end [E] = tree index of
+ * the segment's last vertex (-1: no segment, or its tree overflowed).  A tree whose vertices would exceed cap is left
+ * unchanged and overflow[tree] is set to 1 (never cleared here).  q_path may be NULL only when max_steps = 0. */
+int gik_tree_grow_f32(gik_handle_t h, int64_t n_trees, int32_t cap, float* verts, float* cubes, int32_t* parent,
+                      int32_t* n_verts, uint8_t* overflow, int64_t n_edges, int32_t max_steps, const int32_t* edge_tree,
+                      const int32_t* near, const float* q_start, const float* pose_a, const float* pose_b,
+                      const int32_t* num_steps, const int32_t* n_valid, const float* q_path, int32_t* seg_end,
+                      void* stream);
+int gik_tree_grow_f64(gik_handle_t h, int64_t n_trees, int32_t cap, double* verts, double* cubes, int32_t* parent,
+                      int32_t* n_verts, uint8_t* overflow, int64_t n_edges, int32_t max_steps, const int32_t* edge_tree,
+                      const int32_t* near, const double* q_start, const double* pose_a, const double* pose_b,
+                      const int32_t* num_steps, const int32_t* n_valid, const double* q_path, int32_t* seg_end,
+                      void* stream);
+
+/* The returned path of computepath (path.py:226-233, 317) for n_queries queries (2 * n_queries trees): query i
+ * connected at vertex start_end[i] of tree i and goal_end[i] of tree n_queries + i (-1 = did not connect); its path
+ * is get_path(start tree, start_end) followed by get_path(goal tree, goal_end) reversed, packed as CSR rows
+ * offsets [n_queries + 1] (int64), q [total][nq], cube [total][12] (row-major); an unconnected query has no rows.
+ * Two calls: with q = cube = NULL the lengths are computed and offsets written (offsets[n_queries] = total, the one
+ * value the caller reads back to size q / cube); then, with q and cube, the rows are written at those offsets. */
+int gik_tree_paths_f32(gik_handle_t h, int64_t n_queries, int32_t cap, const float* verts, const float* cubes,
+                       const int32_t* parent, const int32_t* n_verts, const int32_t* start_end, const int32_t* goal_end,
+                       int64_t* offsets, float* q, float* cube, void* stream);
+int gik_tree_paths_f64(gik_handle_t h, int64_t n_queries, int32_t cap, const double* verts, const double* cubes,
+                       const int32_t* parent, const int32_t* n_verts, const int32_t* start_end, const int32_t* goal_end,
+                       int64_t* offsets, double* q, double* cube, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -95,3 +95,53 @@ def rrt_connect_trials(robot, cubeplacementq0, cubeplacementqgoal, std_devs=STD_
                         "max_iterations": int(np.max(iters)), "min_iterations": int(np.min(iters)),
                         "std_iterations": float(np.std(iters))})
     return results
+
+
+def random_endpoints(robot, cubeplacementq0, cubeplacementqgoal, std_dev, n, *, dtype=torch.float64, generator=None,
+                     oversample=4):
+    """n endpoints of path_TESTS.sample_random_cube_placement drawn in batch with the acceptance rule of
+    `_random_endpoint` (valid grasp, cube and robot collision-free, 0.04 m clearance): candidates are drawn and
+    validated `oversample * n` at a time and the valid ones are taken in draw order.  -> (q [n,nq], placements [n,3])."""
+    solver = solver_for(robot)
+    solver._need_scene()
+    qs, ps, need = [], [], n
+    while need > 0:
+        m = max(need * oversample, 256)
+        pl = sample_gaussian_placements(m, cubeplacementq0, cubeplacementqgoal, std_dev, device=solver.device, dtype=dtype,
+                                        generator=generator)
+        p12 = as_pose12(pl, dtype=dtype, device=solver.device).t().contiguous()
+        q0 = torch.zeros((solver.nq, m), dtype=dtype, device=solver.device)
+        q, succ, _, _, _ = solver.solve_success_soa(q0, p12, descend_while_colliding=False, early_stop=True)
+        ok = succ.bool() & ~solver.cube_collision_soa(p12).bool() & solver.clearance_soa(q, p12, 0.04).bool()
+        idx = torch.nonzero(ok).flatten()[:need]
+        qs.append(q.t()[idx]); ps.append(pl[idx])
+        need -= idx.numel()
+    return torch.cat(qs), torch.cat(ps)
+
+
+def rrt_connect_trials_batch(robot, cubeplacementq0, cubeplacementqgoal, std_devs=STD_DEVS[:4], trials=100, *,
+                             dtype=torch.float64, generator=None, expand=8):
+    """`rrt_connect_trials` with every query of a spread in ONE computepath_batch call: the same dict keys per spread.
+    Times are AMORTISED per query -- the device-synchronised wall time of the batched call divided by `trials` -- so
+    avg_time = max_time = min_time and std_time = 0; the iteration statistics are per query."""
+    import time
+    from .planner import computepath_batch
+    solver = solver_for(robot)
+    solver._need_scene()
+    results = []
+    for sd in std_devs:
+        q, pl = random_endpoints(solver, cubeplacementq0, cubeplacementqgoal, sd, 2 * trials, dtype=dtype,
+                                 generator=generator)
+        torch.cuda.synchronize(solver.device)
+        t0 = time.perf_counter()
+        _, _, offsets, stats = computepath_batch(q[:trials], q[trials:], pl[:trials], pl[trials:], robot=solver,
+                                                 generator=generator, dtype=dtype, expand=expand)
+        torch.cuda.synchronize(solver.device)
+        t = (time.perf_counter() - t0) / trials
+        wins = int((offsets[1:] > offsets[:-1]).sum().item())
+        iters = stats["iterations"].cpu().numpy()
+        results.append({"std_dev": tuple(sd), "success_rate": 100.0 * wins / trials,
+                        "avg_time": t, "max_time": t, "min_time": t, "std_time": 0.0,
+                        "avg_iterations": float(np.mean(iters)), "max_iterations": int(np.max(iters)),
+                        "min_iterations": int(np.min(iters)), "std_iterations": float(np.std(iters))})
+    return results

@@ -352,6 +352,95 @@ class GraspIK:
             self.launches += 1
         return ctrl, cost
 
+    # ------------------------------------------------------------------ RRT-connect trees on the device (csrc/gik_tree.cuh)
+    # verts [n_trees][nq][cap], cubes [n_trees][12][cap], parent i32 [n_trees][cap], n_verts i32 [n_trees]
+    def _chk_tree(self, verts, n_verts, cubes=None, parent=None):
+        self._chk_dev(verts, n_verts, cubes, parent)
+        _sfx(verts.dtype)
+        n_trees, nq, cap = verts.shape
+        if nq != self.nq or n_verts.shape != (n_trees,) or n_verts.dtype != torch.int32 or \
+                (cubes is not None and (cubes.shape != (n_trees, 12, cap) or cubes.dtype != verts.dtype)) or \
+                (parent is not None and (parent.shape != (n_trees, cap) or parent.dtype != torch.int32)):
+            raise ValueError("trees: expected verts [n_trees][nq][cap], cubes [n_trees][12][cap] (same dtype), "
+                             "parent int32 [n_trees][cap], n_verts int32 [n_trees]")
+        if not all(t is None or t.is_contiguous() for t in (verts, n_verts, cubes, parent)):
+            raise ValueError("tree arrays must be contiguous")
+        return n_trees, cap
+
+    def tree_nearest(self, verts, n_verts, targets, target_tree) -> torch.Tensor:
+        """Nearest vertex of tree target_tree[t] to each row of targets [n,nq] (gik_tree_nearest_*): squared distances
+        in fp64, numpy's sum order and argmin's tie rule (lowest index).  -> nearest int32 [n] (-1: empty tree)."""
+        n_trees, cap = self._chk_tree(verts, n_verts)
+        self._chk_dev(targets, target_tree)
+        n = targets.shape[0]
+        tg = targets.to(verts.dtype).contiguous()
+        tt = target_tree.to(torch.int32).contiguous()
+        if tg.shape != (n, self.nq) or tt.shape != (n,):
+            raise ValueError("tree_nearest: expected targets [n][nq] and target_tree [n]")
+        out = torch.empty((n,), dtype=torch.int32, device=self.device)
+        f = getattr(self._lib, f"gik_tree_nearest_{_sfx(verts.dtype)}")
+        _cabi.check(f(self._h, n_trees, cap, self._ptr(verts), self._ptr(n_verts), n, self._ptr(tg), self._ptr(tt),
+                      self._ptr(out), self._stream()), "gik_tree_nearest")
+        if n:
+            self.launches += 1
+        return out
+
+    def tree_grow(self, verts, cubes, parent, n_verts, overflow, edge_tree, near, q_start, pose_a, pose_b, num_steps,
+                  n_valid, q_path) -> torch.Tensor:
+        """Append the output of one edge launch to the trees in place (gik_tree_grow_*; grow() of computepath).
+        Edge e (the edges of one tree consecutive) belongs to tree edge_tree[e] and starts at vertex near[e];
+        q_start [nq][E], pose_a / pose_b [12][E], num_steps i32 [E] and q_path [S][nq][E] are project_edges_soa's
+        inputs and output, n_valid i32 [E] its step counts (< 0: no segment).  overflow u8 [n_trees] is set for a tree
+        that would exceed its capacity (left unchanged).  -> seg_end int32 [E] (tree index of each segment's last
+        vertex, -1 without a segment)."""
+        n_trees, cap = self._chk_tree(verts, n_verts, cubes, parent)
+        self._chk_dev(overflow, edge_tree, near, q_start, pose_a, pose_b, num_steps, n_valid, q_path)
+        E = q_start.shape[1]
+        S = q_path.shape[0]
+        dt = verts.dtype
+        if overflow.shape != (n_trees,) or overflow.dtype != torch.uint8:
+            raise ValueError("tree_grow: overflow must be uint8 [n_trees]")
+        if q_start.shape != (self.nq, E) or pose_a.shape != (12, E) or pose_b.shape != (12, E) or \
+                q_path.shape != (S, self.nq, E) or any(t.shape != (E,) for t in (edge_tree, near, num_steps, n_valid)):
+            raise ValueError("tree_grow: inconsistent edge shapes")
+        if any(t.dtype != dt for t in (q_start, pose_a, pose_b, q_path)) or \
+                any(t.dtype != torch.int32 for t in (edge_tree, near, num_steps, n_valid)):
+            raise TypeError("tree_grow: float arrays must share the trees' dtype, index arrays must be int32")
+        seg_end = torch.empty((E,), dtype=torch.int32, device=self.device)
+        args = [x.contiguous() for x in (edge_tree, near, q_start, pose_a, pose_b, num_steps, n_valid, q_path)]
+        f = getattr(self._lib, f"gik_tree_grow_{_sfx(dt)}")
+        _cabi.check(f(self._h, n_trees, cap, self._ptr(verts), self._ptr(cubes), self._ptr(parent), self._ptr(n_verts),
+                      self._ptr(overflow), E, S, *[self._ptr(x) for x in args], self._ptr(seg_end), self._stream()),
+                    "gik_tree_grow")
+        if E:
+            self.launches += 1
+        return seg_end
+
+    def tree_paths(self, verts, cubes, parent, n_verts, start_end, goal_end):
+        """Paths of Q queries (2Q trees: start tree i, goal tree Q + i) that connected at (start_end[i], goal_end[i])
+        (-1 = did not connect): get_path(start) + get_path(goal)[::-1] (path.py:226-233, 317) as packed rows
+        (gik_tree_paths_*).  -> (q [total][nq], cube [total][12], offsets int64 [Q+1]); query i owns rows
+        offsets[i]:offsets[i+1].  One host synchronisation (reading the total)."""
+        n_trees, cap = self._chk_tree(verts, n_verts, cubes, parent)
+        Q = n_trees // 2
+        self._chk_dev(start_end, goal_end)
+        if n_trees != 2 * Q or start_end.shape != (Q,) or goal_end.shape != (Q,):
+            raise ValueError("tree_paths: expected 2Q trees and start_end / goal_end [Q]")
+        se, ge = start_end.to(torch.int32).contiguous(), goal_end.to(torch.int32).contiguous()
+        offsets = torch.zeros((Q + 1,), dtype=torch.int64, device=self.device)
+        f = getattr(self._lib, f"gik_tree_paths_{_sfx(verts.dtype)}")
+        tree = [self._ptr(x) for x in (verts, cubes, parent, n_verts, se, ge)]
+        _cabi.check(f(self._h, Q, cap, *tree, self._ptr(offsets), None, None, self._stream()), "gik_tree_paths")
+        total = int(offsets[-1].item()) if Q else 0
+        q = torch.empty((total, self.nq), dtype=verts.dtype, device=self.device)
+        cube = torch.empty((total, 12), dtype=verts.dtype, device=self.device)
+        if total:
+            _cabi.check(f(self._h, Q, cap, *tree, self._ptr(offsets), self._ptr(q), self._ptr(cube), self._stream()),
+                        "gik_tree_paths")
+        if Q:
+            self.launches += 3 if total else 2
+        return q, cube, offsets
+
     def cube_collision_soa(self, cube_pose_soa: torch.Tensor) -> torch.Tensor:
         """The cube's own collision test (cube vs table / obstacle, path.py:51-52): cube_pose [12][n] -> u8 [n]."""
         self._need_scene()

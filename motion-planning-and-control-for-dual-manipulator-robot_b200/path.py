@@ -16,7 +16,10 @@ Deliberate differences from the reference loop (never unsafe: every returned ver
     (inverse_geometry.py:70) -- it may find a free q there and carry on with it as the next warm start, so its edges
     can be longer than the ones returned here, never shorter;
   * the sampler abandons stalled descents early (GIK_F_EARLY_STOP) and skips the extra descent on colliding samples:
-    accepted samples satisfy the reference's acceptance rule; which candidates are accepted can differ."""
+    accepted samples satisfy the reference's acceptance rule; which candidates are accepted can differ;
+  * the batched planner (planner.computepath_batch) draws a fixed number of candidates (16) per extension slot and
+    iteration instead of rejecting until a valid sample turns up: a slot whose candidates all fail stays idle for that
+    iteration -- no edge, and no connect test for that slot."""
 from __future__ import annotations
 
 import numpy as np
@@ -31,11 +34,19 @@ STEP_SIZE = 0.025                 # path.py:125, 203-206
 
 def sample_cube_placements(n, p0, p1, *, z_range=(Z_MIN, Z_MAX), device="cuda", dtype=torch.float32, generator=None):
     """n translations uniform in the box of path.py:35-45: x, y between the two given cube translations, z in
-    `z_range`; identity rotation (path.py:47).  Returns [n,3]."""
-    p0 = np.asarray(p0, float).reshape(-1)[-3:]
-    p1 = np.asarray(p1, float).reshape(-1)[-3:]
-    lo = torch.tensor([min(p0[0], p1[0]), min(p0[1], p1[1]), z_range[0]], dtype=dtype, device=device)
-    hi = torch.tensor([max(p0[0], p1[0]), max(p0[1], p1[1]), z_range[1]], dtype=dtype, device=device)
+    `z_range`; identity rotation (path.py:47).  `p0` / `p1` are one placement each (translation last), or per-row
+    placements [n,3|12] (tensors or arrays): row i is then drawn from its own box.  Returns [n,3]."""
+    if getattr(p0, "ndim", 1) == 2:
+        a = torch.as_tensor(p0, device=device)[:, -3:].to(dtype)
+        b = torch.as_tensor(p1, device=device)[:, -3:].to(dtype)
+        z = torch.tensor(z_range, dtype=dtype, device=device).expand(a.shape[0], 2)
+        lo = torch.cat([torch.minimum(a[:, :2], b[:, :2]), z[:, :1]], dim=1)
+        hi = torch.cat([torch.maximum(a[:, :2], b[:, :2]), z[:, 1:]], dim=1)
+    else:
+        p0 = np.asarray(p0, float).reshape(-1)[-3:]
+        p1 = np.asarray(p1, float).reshape(-1)[-3:]
+        lo = torch.tensor([min(p0[0], p1[0]), min(p0[1], p1[1]), z_range[0]], dtype=dtype, device=device)
+        hi = torch.tensor([max(p0[0], p1[0]), max(p0[1], p1[1]), z_range[1]], dtype=dtype, device=device)
     u = torch.rand((n, 3), dtype=dtype, device=device, generator=generator)
     return lo + u * (hi - lo)
 
@@ -59,6 +70,16 @@ def sample_grasp_poses_batch(robot, n, cubeplacementq0, cubeplacementqgoal, *, q
     b = _pose_to_array(cubeplacementqgoal)
     pl = sample_cube_placements(n, a[9:], b[9:], device=solver.device, dtype=dtype, generator=generator)
     qi = torch.zeros(solver.nq, dtype=dtype, device=solver.device) if q0 is None else torch.as_tensor(q0, device=solver.device).to(dtype)
+    q, ok = _grasp_filter(solver, pl, qi, dtype, cube_collision=cube_collision, collision=collision,
+                          min_obstacle_distance=min_obstacle_distance, eps=eps, dt=dt, max_iters=max_iters, damping=damping)
+    return q, pl, ok
+
+
+def _grasp_filter(solver, pl, qi, dtype, *, cube_collision="scene", collision="scene",
+                  min_obstacle_distance=MIN_OBSTACLE_DISTANCE, eps=EPSILON, dt=DT, max_iters=MAX_ITERS, damping=0.0):
+    """Steps 2-4 of sample_grasp_poses_batch on the placements pl [n,3] with IK from qi [nq]: cube collision, IK with
+    the success predicate, clearance.  Returns (q [n,nq], ok bool [n]).  Shared with the batched planner's sampler."""
+    n = pl.shape[0]
     p12 = as_pose12(pl, dtype=dtype, device=solver.device)
     pose_soa = p12.t().contiguous()
     if collision == "scene":
@@ -83,7 +104,7 @@ def sample_grasp_poses_batch(robot, n, cubeplacementq0, cubeplacementqgoal, *, q
         ok = ok & ~solver.cube_collision_soa(pose_soa).bool()
     elif callable(cube_collision):
         ok = ok & ~torch.as_tensor(cube_collision(pl), device=solver.device).bool()
-    return q, pl, ok
+    return q, ok
 
 
 def edge_num_steps(cube_a12: torch.Tensor, cube_b12: torch.Tensor, step_size=STEP_SIZE) -> torch.Tensor:
@@ -129,22 +150,32 @@ def project_edges_batch(robot, q_start, cube_a, cube_b, *, num_steps=None, step_
     return out
 
 
-def _cut_at_first_collision(solver, path, nv, a12, b12, ns, S):
+def _cut_at_first_collision(solver, path, nv, a12, b12, ns, S, dense=False):
     """path [S][nq][E] (zero beyond n_valid), nv [E] -> nv cut at the first step whose cube placement or robot
-    configuration collides with the attached scene; rows beyond the new nv are zeroed."""
+    configuration collides with the attached scene; rows beyond the new nv are zeroed.  `dense=True` tests all S steps
+    of every edge and masks the result instead of gathering the valid ones first: more collision work, no host
+    synchronisation (the gather sizes its output); same result."""
     solver._need_scene()
     E = a12.shape[0]
     dev = a12.device
     k = torch.arange(S, device=dev)
     valid = k[None, :] < nv[:, None]                                            # [E,S]
-    e_idx, k_idx = torch.nonzero(valid, as_tuple=True)
+    if dense:
+        e_idx = torch.arange(E, device=dev).repeat_interleave(S)
+        k_idx = k.repeat(E)
+    else:
+        e_idx, k_idx = torch.nonzero(valid, as_tuple=True)
     bad = torch.zeros((E, S), dtype=torch.bool, device=dev)
     if e_idx.numel():
-        alpha = (k_idx + 1).to(a12.dtype) / ns[e_idx].to(a12.dtype)
+        # (dense: the clamps keep the unused steps' placements finite; a valid step's alpha is unchanged)
+        alpha = ((k_idx + 1).to(a12.dtype) / ns[e_idx].clamp_min(1).to(a12.dtype)).clamp(max=1.0)
         poses = se3_interpolate(a12[e_idx], b12[e_idx], alpha).t().contiguous()   # [12][M]
         q = path[k_idx, :, e_idx].t().contiguous()                                # [nq][M]
         hit = solver.cube_collision_soa(poses).bool() | solver.collision_soa(q, poses).bool()
-        bad[e_idx, k_idx] = hit
+        if dense:
+            bad = hit.reshape(E, S) & valid
+        else:
+            bad[e_idx, k_idx] = hit
     first_bad = torch.where(bad.any(dim=1), bad.to(torch.int32).argmax(dim=1), torch.full((E,), S, device=dev)).to(nv.dtype)
     nv_new = torch.minimum(nv, first_bad)
     path.mul_((k[None, :] < nv_new[:, None]).t()[:, None, :].to(path.dtype))      # zero the rows that were cut
