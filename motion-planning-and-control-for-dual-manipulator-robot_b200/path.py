@@ -365,12 +365,19 @@ def _like(template, pose12):
 def se3_interpolate(a12: torch.Tensor, b12: torch.Tensor, alpha) -> torch.Tensor:
     """pin.SE3.Interpolate(A, B, alpha) = A exp6(alpha log6(A^-1 B)) on [B,12] host/device tensors; alpha a float or a
     [B] tensor (bookkeeping for the returned cube paths and the scene tests; the kernel has its own copy in
-    gik_core.cuh)."""
-    alpha = torch.as_tensor(alpha, dtype=a12.dtype, device=a12.device).reshape(-1, 1)
+    gik_core.cuh).  log3 follows pinocchio, including its form for rotations within 1e-2 of pi: |w_i| from the
+    diagonal, the sign of w_i from the antisymmetric part.  At exactly pi about an axis that is not a coordinate axis
+    the signs are rounding noise in pinocchio too.  log6(A^-1 B) is evaluated in fp64 whatever the input dtype (an
+    fp32 log3 cannot resolve the axis near pi) and rounded to the input dtype; exp6 and the product with A run in the
+    input dtype, so that an edge without rotation gives the kernel's placements bit for bit.  Returned on the input's
+    device."""
+    dtype = a12.dtype
+    alpha = torch.as_tensor(alpha, dtype=dtype, device=a12.device).reshape(-1, 1)
     Ra, pa = a12[:, :9].reshape(-1, 3, 3), a12[:, 9:]
-    Rb, pb = b12[:, :9].reshape(-1, 3, 3), b12[:, 9:]
-    R = Ra.transpose(1, 2) @ Rb
-    p = (Ra.transpose(1, 2) @ (pb - pa).unsqueeze(-1)).squeeze(-1)
+    Ra64, pa64 = Ra.to(torch.float64), pa.to(torch.float64)
+    Rb64, pb64 = b12[:, :9].reshape(-1, 3, 3).to(torch.float64), b12[:, 9:].to(torch.float64)
+    R = Ra64.transpose(1, 2) @ Rb64
+    p = (Ra64.transpose(1, 2) @ (pb64 - pa64).unsqueeze(-1)).squeeze(-1)
     # log3
     v = torch.stack([R[:, 2, 1] - R[:, 1, 2], R[:, 0, 2] - R[:, 2, 0], R[:, 1, 0] - R[:, 0, 1]], dim=1)
     c = ((R.diagonal(dim1=1, dim2=2).sum(1) - 1) * 0.5).clamp(-1, 1)
@@ -378,21 +385,30 @@ def se3_interpolate(a12: torch.Tensor, b12: torch.Tensor, alpha) -> torch.Tensor
     th = torch.atan2(s, c)
     fac = torch.where(s > 1e-12, 0.5 * th / s.clamp_min(1e-300), torch.full_like(s, 0.5))
     w = fac.unsqueeze(1) * v
+    # near pi, v = 2 sin(theta) u loses the axis to rounding: pinocchio's form, selected without a host synchronisation
+    near_pi = (th >= np.pi - 1e-2).unsqueeze(1)
+    w_pi = ((R.diagonal(dim1=1, dim2=2) - c.unsqueeze(1)) * (th * th / (1 - c).clamp_min(1)).unsqueeze(1)).clamp_min(0).sqrt()
+    w = torch.where(near_pi, torch.where(v > 0, w_pi, -w_pi), w)
     t2 = th * th
     small = t2 < 1e-8
-    half_cot = torch.where(small, torch.ones_like(th), 0.5 * th * (1 + c) / s.clamp_min(1e-300))
+    # (theta/2) cot(theta/2) = (theta/2) (1 + c) / s = (theta/2) s / (1 - c): the second form keeps its accuracy near pi
+    half_cot = torch.where(small, torch.ones_like(th),
+                           0.5 * th * torch.where(c >= 0, (1 + c) / s.clamp_min(1e-300), s / (1 - c).clamp_min(1e-300)))
     alpha_c = torch.where(small, 1 - t2 / 12, half_cot)
     beta_c = torch.where(small, torch.full_like(th, 1.0 / 12), (1 - alpha_c) / t2.clamp_min(1e-300))
     lin = alpha_c.unsqueeze(1) * p - 0.5 * torch.cross(w, p, dim=1) + (beta_c * (w * p).sum(1)).unsqueeze(1) * w
-    # exp6(alpha * [lin; w])
-    lv, lw = alpha * lin, alpha * w
+    # exp6(alpha * [lin; w]) in the input dtype
+    lv, lw = alpha * lin.to(dtype), alpha * w.to(dtype)
     t2 = (lw * lw).sum(1)
     t = t2.sqrt()
-    small = t2 < 1e-8
-    ts = t.clamp_min(1e-300)
-    ca = torch.where(small, 1 - t2 / 6, torch.sin(t) / ts)
-    cb = torch.where(small, 0.5 - t2 / 24, (1 - torch.cos(t)) / ts ** 2)
-    cc = torch.where(small, 1.0 / 6 - t2 / 120, (t - torch.sin(t)) / ts ** 3)
+    # series below the kernel's threshold (se3_advance): in fp32 (t - sin t) / t^3 cancels up to t^2 = 0.25
+    small = t2 < (1e-8 if dtype == torch.float64 else 0.25)
+    ts = t.clamp_min(torch.finfo(dtype).tiny)
+    ca = torch.where(small, 1 - t2 * (1 / 6 - t2 * (1 / 120 - t2 * (1 / 5040 - t2 / 362880))), torch.sin(t) / ts)
+    cb = torch.where(small, 0.5 - t2 * (1 / 24 - t2 * (1 / 720 - t2 * (1 / 40320 - t2 / 3628800))),
+                     (1 - torch.cos(t)) / ts ** 2)
+    cc = torch.where(small, 1 / 6 - t2 * (1 / 120 - t2 * (1 / 5040 - t2 * (1 / 362880 - t2 / 39916800))),
+                     (t - torch.sin(t)) / ts ** 3)
     W = torch.zeros((lw.shape[0], 3, 3), dtype=lw.dtype, device=lw.device)
     W[:, 0, 1], W[:, 0, 2], W[:, 1, 0] = -lw[:, 2], lw[:, 1], lw[:, 2]
     W[:, 1, 2], W[:, 2, 0], W[:, 2, 1] = -lw[:, 0], -lw[:, 1], lw[:, 0]
