@@ -111,23 +111,15 @@ GIK_HD float rsqrt_(float x) {
 #endif
 }
 // fp64 device versions: MUFU seed (rsqrt/rcp.approx.ftz.f64, ~2^-22 relative) + ONE third-order correction step
-// (5 / 3 FP64-pipe instructions; two Newton steps, 7 / 4, behind GIK_NEWTON2_F64).  Accuracy measured on B200 over
+// (5 / 3 FP64-pipe instructions; two Newton steps, 7 / 4, measured no more accurate).  Accuracy measured on B200 over
 // 1e-12..1e12 by tools/probes/f64_approx.cu (see DESIGN.md); no special-case paths: operands are floored.
 GIK_HD double rsqrt_(double x) {
 #ifdef __CUDA_ARCH__
   double y;
   asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
-#ifdef GIK_NEWTON2_F64
-  const double h = 0.5 * x;
-  double e = fma(-h * y, y, 0.5);
-  y = fma(y, e, y);
-  e = fma(-h * y, y, 0.5);
-  return fma(y, e, y);
-#else
   // one third-order step: y (1 + e/2 + 3 e^2 / 8), e = 1 - x y^2; seed error 2^-22 -> ~1e-20 before rounding
   const double e = fma(-(x * y), y, 1.0);
   return fma(y * e, fma(e, 0.375, 0.5), y);
-#endif
 #else
   return 1.0 / sqrt(x);
 #endif
@@ -145,16 +137,9 @@ GIK_HD double rcp_(double b) {
 #ifdef __CUDA_ARCH__
   double y;
   asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(b));
-#ifdef GIK_NEWTON2_F64
-  double e = fma(-b, y, 1.0);
-  y = fma(y, e, y);
-  e = fma(-b, y, 1.0);
-  return fma(y, e, y);
-#else
   // one third-order step: y (1 + e + e^2), e = 1 - b y
   const double e = fma(-b, y, 1.0);
   return fma(fma(y, e, y), e, y);
-#endif
 #else
   return 1.0 / b;
 #endif
@@ -208,13 +193,10 @@ GIK_HD float atan2_pos(float y, float x) {
   -0.3333333333333333, 0.1999999999999552, -0.14285714284666542, 0.11111111015256361, -0.09090904578123903,  \
       0.07692183190826087, -0.06664511447381948, 0.0585814891280221, -0.0508544973794026, 0.03923165829558719, \
       -0.01917688711906226
-#if defined(__CUDACC__) && !defined(GIK_LIB_ATAN64)
+#if defined(__CUDACC__)
 static __constant__ double kAtan64[11] = {GIK_ATAN64_COEFFS};
 #endif
 GIK_HD double atan2_pos(double y, double x) {
-#if defined(GIK_LIB_ATAN64)
-  return atan2(y, x);
-#else
 #ifdef __CUDA_ARCH__
   const double* K = kAtan64;
 #else
@@ -232,7 +214,6 @@ GIK_HD double atan2_pos(double y, double x) {
   r = big ? r + 0.78539816339744831 : r;
   r = y > ax ? 1.57079632679489662 - r : r;
   return x < 0.0 ? 3.14159265358979324 - r : r;
-#endif
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -333,7 +314,6 @@ GIK_HD void sincos_(float x, float& s, float& c) {
 // 15 % of the loop's issue slots in the round-1 fp64 capture) and carries a slow-path branch for huge arguments.
 // Valid for |x| < 2^50 (far beyond any joint range); NaN/inf propagate.
 #if defined(__CUDACC__)
-#ifndef GIK_LIB_SINCOS64
 static __constant__ double kSinCos64[18] = {
     6.36619772367581382433e-01,   // 0: 2/pi
     6755399441055744.0,           // 1: 1.5 * 2^52 (round-to-nearest-integer magic)
@@ -353,10 +333,9 @@ static __constant__ double kSinCos64[18] = {
     -1.13596475577881948265e-11,  // 15: C6
     -0.5, 1.0};
 #endif
-#endif
 template <bool FAST>
 GIK_HD void sincos_(double x, double& s, double& c) {
-#if defined(__CUDA_ARCH__) && !defined(GIK_LIB_SINCOS64)
+#ifdef __CUDA_ARCH__
   if (FAST) {
     const double* K = kSinCos64;
     const double t = fma(x, K[0], K[1]);
@@ -380,8 +359,6 @@ GIK_HD void sincos_(double x, double& s, double& c) {
   } else {
     sincos(x, &s, &c);
   }
-#elif defined(__CUDA_ARCH__)
-  sincos(x, &s, &c);
 #else
   s = sin(x); c = cos(x);
 #endif
@@ -475,13 +452,6 @@ GIK_HD void log6_pre_v(F2 vx, F2 vy, F2 vz, F2 tr, Log6Mid<F2>& m) {
   const F2 den = sel_(front, s, F2(1.0f) - c);
   const F2 alpha_g = F2(0.5f) * theta * (num * rcp_(max_(den, tiny)));
   const F2 beta_g = (F2(1.0f) - alpha_g) * rcp_(max_(t2, tiny));
-#ifdef GIK_LOG6_SERIES_F32
-  const F2 alpha_s = F2(1.0f) - t2 * (F2(1.0f / 12) + t2 * (F2(1.0f / 720) + t2 * F2(1.0f / 30240)));
-  const F2 beta_s = F2(1.0f / 12) + t2 * (F2(1.0f / 720) + t2 * (F2(1.0f / 30240) + t2 * F2(1.0f / 1209600)));
-  const B2 small = lt_(t2, F2(Num<float>::kSeriesT2));
-  m.alpha = sel_(small, alpha_s, alpha_g);
-  m.beta = sel_(small, beta_s, beta_g);
-#else
   // The packed kernel is bound by FMA-pipe slots, and fp32 needs no series near theta = 0: alpha = (theta / s) (1 + c) / 2
   // is a product of factors that each keep their relative accuracy (theta is computed FROM s, so the ratio is clean),
   // and beta = (1 - alpha) / theta^2 -- whose cancellation costs it ~1e-7 / theta^2 absolute -- enters e only as
@@ -489,7 +459,6 @@ GIK_HD void log6_pre_v(F2 vx, F2 vy, F2 vz, F2 tr, Log6Mid<F2>& m) {
   // selects less per iteration: config 2 45.8 -> 47.1 M solves/s.
   m.alpha = sel_(gt_(s, tiny), alpha_g, F2(1.0f));     // (exactly zero rotation error: theta = 0 would zero the product)
   m.beta = beta_g;
-#endif
   m.vx = vx; m.vy = vy; m.vz = vz;
   m.c = c; m.theta = theta;
 }
@@ -1067,6 +1036,13 @@ GIK_HD void se3_advance(const T (&A)[12], const T (&xi)[6], T alpha, T (&out)[12
       out[3 * r + cc] = A[3 * r] * E[cc] + A[3 * r + 1] * E[3 + cc] + A[3 * r + 2] * E[6 + cc];
     out[9 + r] = A[9 + r] + A[3 * r] * d[0] + A[3 * r + 1] * d[1] + A[3 * r + 2] * d[2];
   }
+}
+
+// Placement of step s of an edge marched in nsteps steps, xi = se3_delta(A, B): A * exp6((s / nsteps) xi).  The edge
+// kernels solve each step for it and the tree kernels store it with the step's configuration.
+template <typename T>
+GIK_HD void edge_placement(const T (&A)[12], const T (&xi)[6], int s, int nsteps, T (&out)[12]) {
+  se3_advance(A, xi, T(s) / T(nsteps), out);
 }
 
 }  // namespace gik

@@ -18,20 +18,14 @@
 
 namespace gik {
 
-#ifndef GIK_THREADS
-#define GIK_THREADS 128
-#endif
-#ifndef GIK_MINB_F32
-#define GIK_MINB_F32 4   // 4 x 128 threads / SM -> <= 128 registers per thread
-#endif
-#ifndef GIK_MINB_F64
-#define GIK_MINB_F64 3   // 3 x 128 threads / SM -> 168 registers per thread; spills go to L1 and cost LSU issue slots, which the
-                         // FP64-pipe-bound loop has to spare (measured +7 % over 2 blocks, -10 % at 4 blocks)
-#endif
+constexpr int kThreads = 128;   // threads per block of the persistent solve kernels
 
+// resident blocks per SM of the scalar lane kernel
 template <typename T> struct Launch;
-template <> struct Launch<float>  { static constexpr int kMinBlocks = GIK_MINB_F32; };
-template <> struct Launch<double> { static constexpr int kMinBlocks = GIK_MINB_F64; };
+template <> struct Launch<float>  { static constexpr int kMinBlocks = 4; };   // 4 x 128 threads / SM -> <= 128 registers per thread
+template <> struct Launch<double> { static constexpr int kMinBlocks = 3; };   // 3 x 128 threads / SM -> 168 registers per thread;
+    // spills go to L1 and cost LSU issue slots, which the FP64-pipe-bound loop has to spare (measured +7 % over 2 blocks,
+    // -10 % at 4 blocks)
 
 enum { MODE_BATCH = 0, MODE_EDGES = 1 };
 #define GIK_FLOPS_EXEC_F32_WRIST 945    // see gik_flops_per_iter_executed()
@@ -166,10 +160,7 @@ __device__ __forceinline__ int64_t queue_take(const SolveArgs<T>& a, int64_t n, 
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kChunkShift = 10;
 constexpr int kChunk = 1 << kChunkShift;
-#ifndef GIK_MARK_SHIFT
-#define GIK_MARK_SHIFT 13
-#endif
-constexpr int kMarkShift = GIK_MARK_SHIFT;
+constexpr int kMarkShift = 13;
 constexpr int kMarkDone = 0x7fffffff;
 
 __device__ __forceinline__ int ld_relaxed(const int32_t* p) {
@@ -199,7 +190,7 @@ __device__ __forceinline__ int warp_slot() {
 struct MarkState { int pub = 0, pending = 0, events = 0; };
 template <typename T>
 __device__ __forceinline__ int mark_slot(const SolveArgs<T>& a) {          // the leading blocks hold the pushers
-  return ((int)blockIdx.x - a.push_blocks) * (GIK_THREADS / 32) + ((int)threadIdx.x >> 5);
+  return ((int)blockIdx.x - a.push_blocks) * (kThreads / 32) + ((int)threadIdx.x >> 5);
 }
 // a lane of this warp finished: called BEFORE the results of this event are stored
 template <typename T>
@@ -339,7 +330,7 @@ __device__ __forceinline__ bool push_chunk(const SolveArgs<T>& a, int nq, int64_
 // 19 ms at 8, because F sweeps the last 10 % of the slab at the very end.]
 template <typename T>
 __device__ __noinline__ void pusher_loop(const SolveArgs<T>& a, int nq, int64_t n) {
-  const int lane = threadIdx.x & 31, warp = (int)blockIdx.x * (GIK_THREADS / 32) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31, warp = (int)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5);
   const int64_t n_chunks = (n + kChunk - 1) >> kChunkShift;
   unsigned long long t_a = 0, t_b = 0;    // measurement hook (GIK_FUSED_STATS): lookout: looking / sleeping; pushers: pushing / waiting
   int count = 0;                          // looks / chunks pushed
@@ -448,11 +439,126 @@ __global__ void __launch_bounds__(128) gik_push_rest_kernel(const __grid_constan
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Per-problem code of the three solve kernels: what runs when a lane (lane pair) takes a work item, and when its problem
+// or one step of its edge ends.  These rules define the results -- the start iteration, the placement of each edge step,
+// when the passive joints are clamped, how n_valid counts -- so all kernels run this one copy of them.  Each kernel
+// loads and stores its own ACTIVE joints, whose layout differs: load_q(idx) reads them from q_init, store_q(dst, sc, si,
+// col) writes them to column col of dst (component stride sc, column stride si).  `owner` is the lane that writes the
+// per-problem fields: every lane of the lane kernels, the even lane of a pair.
+// ---------------------------------------------------------------------------------------------------------------
+template <typename T>
+struct Work {
+  int64_t idx = -1;          // column of the problem (or edge) this lane works on
+  bool active = false;
+  int it = 0;                // descent iterations of the problem (edge: of the current step)
+  T r_mark = T(3.0e38);      // early stop: squared residual sum at the last 64-iteration checkpoint
+  int step = 0, nsteps = 0, it_total = 0;   // edge mode: current step (from 1), steps of the edge, iterations so far
+};
+
+// cube placement of step `step` of edge idx
+template <typename T>
+__device__ __forceinline__ void edge_step_cube(const SolveArgs<T>& a, int64_t idx, int step, int nsteps, T (&cube)[12]) {
+  T ca[12], cb[12], xi[6];
+  load_cube(a.pose, a.pose_sc, a.pose_si, idx, ca);
+  load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
+  se3_delta(ca, cb, xi);
+  edge_placement(ca, xi, step, nsteps, cube);
+}
+
+// The lane takes work item `cand`: its column, start iteration and active joints, and in `cube` the placement its hooks
+// aim at (edges: that of step 1).  An edge with nothing to march ends at once with no valid step: the reference loop
+// body never runs (path.py:137).
+template <typename T, int MODE, typename LoadQ>
+__device__ __forceinline__ void work_start(const SolveArgs<T>& a, int64_t cand, bool owner, Work<T>& w, LoadQ load_q,
+                                           T (&cube)[12]) {
+  w.idx = a.sel ? a.sel[cand] : cand;
+  w.active = true;
+  w.it = a.it0 ? a.it0[w.idx] : 0;
+  w.r_mark = T(3.0e38);
+  load_q(w.idx);
+  if (MODE == MODE_BATCH) {
+    load_cube(a.pose, a.pose_sc, a.pose_si, w.idx, cube);
+    return;
+  }
+  w.nsteps = ld_in(a.num_steps + w.idx);
+  w.step = 1;
+  w.it_total = 0;
+  edge_step_cube(a, w.idx, 1, w.nsteps, cube);
+  if (w.nsteps < 1) {
+    if (owner) {
+      a.n_valid[w.idx] = 0;
+      if (a.iters) a.iters[w.idx] = 0;
+    }
+    w.active = false;
+  }
+}
+
+// passive joints of a result: q_init, clamped to their limits if an update has been applied (`moved`: the first update
+// clamps the whole q, :89)
+template <typename T>
+__device__ __forceinline__ void store_passive(const DevTable<T>& tab, const SolveArgs<T>& a, int64_t idx, bool moved, T* dst,
+                                              int64_t sc, int64_t si, int64_t col) {
+  for (int p = 0; p < tab.n_passive; ++p) {
+    const int j = tab.passive_q[p];
+    T v = ld_in(a.q_init + (int64_t)j * a.q_sc + idx * a.q_si);
+    if (moved) v = min_(max_(tab.qlo[j], v), tab.qhi[j]);
+    dst[(int64_t)j * sc + col * si] = v;
+  }
+}
+
+// Batch mode: the lane's problem ended (ok: converged).  Its result goes to this rank's own arrays (peers: the pushers of
+// block 0) -- joints, flag, iteration count, and the residual norm of each hand this lane solved (r[k]: hand h0 + k) --
+// and the lane is free.
+template <typename T, int NH, typename StoreQ>
+__device__ __forceinline__ void batch_finish(const DevTable<T>& tab, const SolveArgs<T>& a, Work<T>& w, bool ok, bool owner,
+                                             StoreQ store_q, int h0, const T (&r)[NH]) {
+  const int64_t col = a.out_off + w.idx;
+  T* qo = a.q_dst[0];
+  store_q(qo, a.out_sc, a.out_si, col);
+  if (owner) {
+    store_passive(tab, a, w.idx, w.it > 0, qo, a.out_sc, a.out_si, col);
+    a.conv_dst[0][col] = ok ? 1 : 0;
+    if (a.iters) a.iters[w.idx] = w.it;
+  }
+  if (a.resid)
+#pragma unroll
+    for (int k = 0; k < NH; ++k) a.resid[(int64_t)(h0 + k) * a.res_sc + w.idx * a.res_si] = sqrt_(r[k]);
+  w.active = false;
+}
+
+// Edge mode: the solve of step w.step ended (ok: converged).  A converged step stores its path row, the passive joints
+// clamped once any update has been applied on this edge.  Then the lane either goes on to the next step -- returns true
+// with its placement in `cube` -- or the edge is finished: n_valid = the steps that converged, iters = the iterations of
+// the whole edge.
+template <typename T, typename StoreQ>
+__device__ __forceinline__ bool edge_step_end(const DevTable<T>& tab, const SolveArgs<T>& a, Work<T>& w, bool ok, bool owner,
+                                              StoreQ store_q, T (&cube)[12]) {
+  w.it_total += w.it;
+  if (ok) {
+    T* dst = a.q_out + (int64_t)(w.step - 1) * tab.nq * a.n;
+    store_q(dst, a.n, 1, w.idx);
+    if (owner) store_passive(tab, a, w.idx, w.it_total > 0, dst, a.n, 1, w.idx);
+  }
+  if (ok && w.step < w.nsteps) {
+    ++w.step;
+    w.it = 0;
+    w.r_mark = T(3.0e38);
+    edge_step_cube(a, w.idx, w.step, w.nsteps, cube);
+    return true;
+  }
+  if (owner) {
+    a.n_valid[w.idx] = ok ? w.step : w.step - 1;
+    if (a.iters) a.iters[w.idx] = w.it_total;
+  }
+  w.active = false;
+  return false;
+}
+
 template <typename T, int MODE, uint32_t TZ, bool WRIST = false>
-__global__ void __launch_bounds__(GIK_THREADS, Launch<T>::kMinBlocks)
+__global__ void __launch_bounds__(kThreads, Launch<T>::kMinBlocks)
 gik_solve_kernel(const __grid_constant__ DevTable<T> tab, const __grid_constant__ SolveArgs<T> a) {
   const int lane = threadIdx.x & 31;
-  const int64_t n_cols = a.n;                                                 // columns of the arrays
   const int64_t n = a.n_sel ? min(a.n, (int64_t)*a.n_sel) : a.n;          // work items of this launch
   if (MODE == MODE_BATCH && a.n_dst > 1 && (int)blockIdx.x < a.push_blocks) {   // fused all-gather: the leading blocks push, the others solve
     pusher_loop(a, tab.nq, n);
@@ -470,14 +576,21 @@ gik_solve_kernel(const __grid_constant__ DevTable<T> tab, const __grid_constant_
   for (int h = 0; h < 2; ++h)
 #pragma unroll
     for (int c = 0; c < 12; ++c) tgt[h][c] = (c % 4 == 0 && c < 9) ? T(1) : T(0);
+  auto load_q = [&](int64_t idx) {
+#pragma unroll
+    for (int i = 0; i < kActive; ++i) q[i] = ld_in(a.q_init + (int64_t)tab.act_q[i] * a.q_sc + idx * a.q_si);
+  };
+  auto store_q = [&](T* dst, int64_t sc, int64_t si, int64_t col) {
+#pragma unroll
+    for (int i = 0; i < kActive; ++i) dst[(int64_t)tab.act_q[i] * sc + col * si] = q[i];
+  };
+  auto set_targets = [&](const T (&cube)[12]) {
+    hook_target(tab.arm[0], cube, tgt[0]);
+    hook_target(tab.arm[1], cube, tgt[1]);
+  };
 
-  int64_t idx = -1;     // problem (or edge) this lane works on
-  bool active = false;
+  Work<T> w;
   bool exhausted = false;   // warp-uniform: the queue has handed out every problem
-  int it = 0;
-  T r_mark = T(3.0e38);      // early stop: squared residual sum at the last 64-iteration checkpoint
-  // edge mode state
-  int step = 0, nsteps = 0, it_total = 0;
   MarkState ms;             // fused all-gather: this warp's low-water mark
 
   for (;;) {
@@ -486,111 +599,45 @@ gik_solve_kernel(const __grid_constant__ DevTable<T> tab, const __grid_constant_
     // order to whichever lane frees up first: the tail of the launch is bounded by ONE problem's duration instead
     // of by the slowest statically assigned lane.  The first refill of a warp takes 32 consecutive problems
     // (coalesced loads).  A problem's arithmetic does not depend on the lane it lands on: results are bit-identical.
-    const unsigned need = exhausted ? 0u : __ballot_sync(0xffffffffu, enabled && !active);
+    const unsigned need = exhausted ? 0u : __ballot_sync(0xffffffffu, enabled && !w.active);
     if (need) {
       const int64_t cand = queue_take(a, n, need, lane, __popc(need & ((1u << lane) - 1u)), from_top, exhausted);
-      if (enabled && !active) {
-        if (cand >= 0) {
-          idx = a.sel ? a.sel[cand] : cand;
-          active = true;
-          it = a.it0 ? a.it0[idx] : 0;
-          r_mark = T(3.0e38);
-#pragma unroll
-          for (int i = 0; i < kActive; ++i) q[i] = ld_in(a.q_init + (int64_t)tab.act_q[i] * a.q_sc + idx * a.q_si);
-          T cube[12];
-          load_cube(a.pose, a.pose_sc, a.pose_si, idx, cube);
-          if (MODE == MODE_EDGES) {
-            nsteps = ld_in(a.num_steps + idx);
-            step = 1;
-            it_total = 0;
-            T cb[12], xi[6], ca[12];
-#pragma unroll
-            for (int c = 0; c < 12; ++c) ca[c] = cube[c];
-            load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
-            se3_delta(ca, cb, xi);
-            se3_advance(ca, xi, T(1) / T(nsteps), cube);
-            if (nsteps < 1) {  // nothing to march: reference loop body never runs (path.py:137)
-              a.n_valid[idx] = 0;
-              if (a.iters) a.iters[idx] = 0;
-              active = false;
-            }
-          }
-          hook_target(tab.arm[0], cube, tgt[0]);
-          hook_target(tab.arm[1], cube, tgt[1]);
-        }
+      if (enabled && !w.active && cand >= 0) {
+        T cube[12];
+        work_start<T, MODE>(a, cand, true, w, load_q, cube);
+        set_targets(cube);
       }
     }
-    if (exhausted && !__any_sync(0xffffffffu, active)) break;
+    if (exhausted && !__any_sync(0xffffffffu, w.active)) break;
 
     // ---------------- one descent iteration for every lane ----------------
     T dq[kActive], rL, rR;
     ik_iteration<T, true, TZ, WRIST>(tab, q, tgt, a.lambda, dq, rL, rR);
-    const bool ok = (rL < a.eps2) && (rR < a.eps2) && (it < a.max_iters);
+    const bool ok = (rL < a.eps2) && (rR < a.eps2) && (w.it < a.max_iters);
     bool stalled = false;
-    if (a.early_stop && (it & 63) == 63) {
+    if (a.early_stop && (w.it & 63) == 63) {
       const T rs = rL + rR;
-      stalled = rs > T(0.9) * r_mark;
-      r_mark = rs;
+      stalled = rs > T(0.9) * w.r_mark;
+      w.r_mark = rs;
     }
-    const bool done = ok || (it >= a.max_iters) || stalled;
+    const bool done = ok || (w.it >= a.max_iters) || stalled;
 
-    const bool fused_event = MODE == MODE_BATCH && a.n_dst > 1 && __any_sync(0xffffffffu, done && active);
+    const bool fused_event = MODE == MODE_BATCH && a.n_dst > 1 && __any_sync(0xffffffffu, done && w.active);
     if (fused_event && !from_top) mark_publish(a, ms, lane);
     if (!done) {
       apply_step(tab, q, dq, a.dt);
-      ++it;
-    } else if (active) {
-      // ---------------- rare path: this lane's problem ended ----------------
+      ++w.it;
+    } else if (w.active) {
+      // ---------------- rare path: this lane's problem (edge step) ended ----------------
+      T cube[12];
       if (MODE == MODE_BATCH) {
-        const int64_t col = a.out_off + idx;
-        {                                       // this rank's own result arrays (peers: the pushers of block 0)
-          T* qo = a.q_dst[0];
-#pragma unroll
-          for (int i = 0; i < kActive; ++i) qo[(int64_t)tab.act_q[i] * a.out_sc + col * a.out_si] = q[i];
-          for (int p = 0; p < tab.n_passive; ++p) {
-            const int j = tab.passive_q[p];
-            T v = ld_in(a.q_init + (int64_t)j * a.q_sc + idx * a.q_si);
-            if (it > 0) v = min_(max_(tab.qlo[j], v), tab.qhi[j]);   // clamped by the first update (:89)
-            qo[(int64_t)j * a.out_sc + col * a.out_si] = v;
-          }
-          a.conv_dst[0][col] = ok ? 1 : 0;
-        }
-        if (a.iters) a.iters[idx] = it;
-        if (a.resid) { a.resid[idx * a.res_si] = sqrt_(rL); a.resid[a.res_sc + idx * a.res_si] = sqrt_(rR); }
-        active = false;
-      } else {
-        it_total += it;
-        if (ok) {
-          T* dst = a.q_out + (int64_t)(step - 1) * tab.nq * n_cols;
-#pragma unroll
-          for (int i = 0; i < kActive; ++i) dst[(int64_t)tab.act_q[i] * n_cols + idx] = q[i];
-          for (int p = 0; p < tab.n_passive; ++p) {
-            const int j = tab.passive_q[p];
-            // passive joints: clamped once any update has been applied on this edge
-            T v = ld_in(a.q_init + (int64_t)j * a.q_sc + idx * a.q_si);
-            if (it_total > 0) v = min_(max_(tab.qlo[j], v), tab.qhi[j]);
-            dst[(int64_t)j * n_cols + idx] = v;
-          }
-        }
-        if (ok && step < nsteps) {
-          ++step;
-          it = 0;
-          r_mark = T(3.0e38);
-          T ca[12], cb[12], xi[6], cube[12];
-          load_cube(a.pose, a.pose_sc, a.pose_si, idx, ca);
-          load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
-          se3_delta(ca, cb, xi);
-          se3_advance(ca, xi, T(step) / T(nsteps), cube);
-          hook_target(tab.arm[0], cube, tgt[0]);
-          hook_target(tab.arm[1], cube, tgt[1]);
-        } else {
-          a.n_valid[idx] = ok ? step : step - 1;
-          if (a.iters) a.iters[idx] = it_total;
-          active = false;
-        }
+        const T r[2] = {rL, rR};
+        batch_finish(tab, a, w, ok, true, store_q, 0, r);
+      } else if (edge_step_end(tab, a, w, ok, true, store_q, cube)) {
+        set_targets(cube);
       }
     }
-    if (fused_event) mark_update(ms, active, idx);      // (from_top warps: statistics only)
+    if (fused_event) mark_update(ms, w.active, w.idx);      // (from_top warps: statistics only)
   }
   if (MODE == MODE_BATCH && a.n_dst > 1) mark_exit(a, lane);
 }
@@ -601,24 +648,16 @@ gik_solve_kernel(const __grid_constant__ DevTable<T> tab, const __grid_constant_
 // chain walks, Gram matrices, Cholesky factorisations and solves of both hands issue as FFMA2 / FMUL2 / FADD2 --
 // half the issue slots of the scalar lane kernel for the same arithmetic (gik_core.cuh "F2").  Scheduling (global
 // work queue, lane refill) is the scalar lane kernel's.
+// Resident blocks per SM: 3 (168 registers) for the block-Cholesky step; 4 for the spherical-wrist step (128 registers,
+// ~190 B of spills outside the iteration).  2^20 problems, packed log6: 42.2 M solves/s against 41.2 M at 3 blocks
+// (144 registers, none) and 38.0 M at 5 (96 registers).
 // ========================================================================================================
-#ifndef GIK_MINB_LANE2
-#define GIK_MINB_LANE2 3
-#endif
-#ifndef GIK_LANE2_INNER
-#define GIK_LANE2_INNER true   // measured against the single-loop form on 2^20 problems: 38.30 -> 36.75 ms (27.3 -> 28.5 M solves/s)
-#endif
-#ifndef GIK_MINB_LANE2_WRIST
-#define GIK_MINB_LANE2_WRIST 4   // 128 registers (~190 B of spills outside the iteration).  2^20 problems, packed log6: 42.2 M solves/s
-                                 // against 41.2 M at 3 blocks (144 registers, none) and 38.0 M at 5 (96 registers)
-#endif
 template <int MODE, uint32_t TZ, bool WRIST = false>
-__global__ void __launch_bounds__(GIK_THREADS, (WRIST ? GIK_MINB_LANE2_WRIST : GIK_MINB_LANE2))
+__global__ void __launch_bounds__(kThreads, (WRIST ? 4 : 3))
 gik_solve_lane2_kernel(const __grid_constant__ DevTable<float> tab, const __grid_constant__ PackedTable pt,
                        const __grid_constant__ SolveArgs<float> a) {
   using T = float;
   const int lane = threadIdx.x & 31;
-  const int64_t n_cols = a.n;                                                 // columns of the arrays
   const int64_t n = a.n_sel ? min(a.n, (int64_t)*a.n_sel) : a.n;          // work items of this launch
   if (MODE == MODE_BATCH && a.n_dst > 1 && (int)blockIdx.x < a.push_blocks) {   // fused all-gather: the leading blocks push, the others solve
     pusher_loop(a, tab.nq, n);
@@ -635,12 +674,11 @@ gik_solve_lane2_kernel(const __grid_constant__ DevTable<float> tab, const __grid
   for (int k = 0; k < 6; ++k) q2[k] = F2(0.0f);
 #pragma unroll
   for (int c = 0; c < 12; ++c) tgt2[c] = F2((c % 4 == 0 && c < 9) ? 1.0f : 0.0f);
-  auto set_targets = [&](const T (&cube)[12]) {
-    T tl[12], tr[12];
-    hook_target(tab.arm[0], cube, tl);
-    hook_target(tab.arm[1], cube, tr);
+  auto load_q = [&](int64_t idx) {
+    q0 = ld_in(a.q_init + (int64_t)tab.act_q[0] * a.q_sc + idx * a.q_si);
 #pragma unroll
-    for (int c = 0; c < 12; ++c) tgt2[c] = F2(tl[c], tr[c]);
+    for (int k = 0; k < 6; ++k)
+      q2[k] = F2(ld_in(a.q_init + (int64_t)tab.act_q[1 + k] * a.q_sc + idx * a.q_si), ld_in(a.q_init + (int64_t)tab.act_q[7 + k] * a.q_sc + idx * a.q_si));
   };
   auto store_q = [&](T* dst, int64_t sc, int64_t si, int64_t col) {
     dst[(int64_t)tab.act_q[0] * sc + col * si] = q0;
@@ -650,144 +688,75 @@ gik_solve_lane2_kernel(const __grid_constant__ DevTable<float> tab, const __grid
       dst[(int64_t)tab.act_q[7 + k] * sc + col * si] = q2[k].y;
     }
   };
+  auto set_targets = [&](const T (&cube)[12]) {
+    T tl[12], tr[12];
+    hook_target(tab.arm[0], cube, tl);
+    hook_target(tab.arm[1], cube, tr);
+#pragma unroll
+    for (int c = 0; c < 12; ++c) tgt2[c] = F2(tl[c], tr[c]);
+  };
 
-  int64_t idx = -1;     // problem (or edge) this lane works on
-  bool active = false;
+  Work<T> w;
   bool exhausted = false;   // warp-uniform: the queue has handed out every problem
-  int it = 0;
-  T r_mark = T(3.0e38);      // early stop: squared residual sum at the last 64-iteration checkpoint
-  // edge mode state
-  int step = 0, nsteps = 0, it_total = 0;
   MarkState ms;             // fused all-gather: this warp's low-water mark
 
   for (;;) {
     // ---------------- refill: lanes without work pull the next problems from the global queue ----------------
-    // One atomicAdd per warp per refill (leader lane, count = lanes in need), so problems are handed out in index
-    // order to whichever lane frees up first: the tail of the launch is bounded by ONE problem's duration instead
-    // of by the slowest statically assigned lane.  The first refill of a warp takes 32 consecutive problems
-    // (coalesced loads).  A problem's arithmetic does not depend on the lane it lands on: results are bit-identical.
-    const unsigned need = exhausted ? 0u : __ballot_sync(0xffffffffu, enabled && !active);
+    // (as in the scalar lane kernel)
+    const unsigned need = exhausted ? 0u : __ballot_sync(0xffffffffu, enabled && !w.active);
     if (need) {
       const int64_t cand = queue_take(a, n, need, lane, __popc(need & ((1u << lane) - 1u)), from_top, exhausted);
-      if (enabled && !active) {
-        if (cand >= 0) {
-          idx = a.sel ? a.sel[cand] : cand;
-          active = true;
-          it = a.it0 ? a.it0[idx] : 0;
-          r_mark = T(3.0e38);
-          q0 = ld_in(a.q_init + (int64_t)tab.act_q[0] * a.q_sc + idx * a.q_si);
-#pragma unroll
-          for (int k = 0; k < 6; ++k)
-            q2[k] = F2(ld_in(a.q_init + (int64_t)tab.act_q[1 + k] * a.q_sc + idx * a.q_si), ld_in(a.q_init + (int64_t)tab.act_q[7 + k] * a.q_sc + idx * a.q_si));
-          T cube[12];
-          load_cube(a.pose, a.pose_sc, a.pose_si, idx, cube);
-          if (MODE == MODE_EDGES) {
-            nsteps = ld_in(a.num_steps + idx);
-            step = 1;
-            it_total = 0;
-            T cb[12], xi[6], ca[12];
-#pragma unroll
-            for (int c = 0; c < 12; ++c) ca[c] = cube[c];
-            load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
-            se3_delta(ca, cb, xi);
-            se3_advance(ca, xi, T(1) / T(nsteps), cube);
-            if (nsteps < 1) {  // nothing to march: reference loop body never runs (path.py:137)
-              a.n_valid[idx] = 0;
-              if (a.iters) a.iters[idx] = 0;
-              active = false;
-            }
-          }
-          set_targets(cube);
-        }
+      if (enabled && !w.active && cand >= 0) {
+        T cube[12];
+        work_start<T, MODE>(a, cand, true, w, load_q, cube);
+        set_targets(cube);
       }
     }
-    if (GIK_LANE2_INNER) {
-      if (!__any_sync(0xffffffffu, active)) {
-        if (exhausted) break;
-        continue;                                // (edges with nothing to march) back to the queue
-      }
-    } else {
-      if (exhausted && !__any_sync(0xffffffffu, active)) break;
+    if (!__any_sync(0xffffffffu, w.active)) {
+      if (exhausted) break;
+      continue;                                // (edges with nothing to march) back to the queue
     }
 
     // ---------------- one descent iteration for every lane ----------------
-    // GIK_LANE2_INNER: the iteration repeats in a loop of its own until an active lane finishes -- arithmetic, one vote
-    // and the back edge per trip; the queue / store logic above and below runs only then (as in the pair kernel)
+    // The iteration repeats in a loop of its own until an active lane finishes -- arithmetic, one vote and the back edge
+    // per trip; the queue / store logic above and below runs only then (as in the pair kernel).  Measured against the
+    // single-loop form on 2^20 problems: 38.30 -> 36.75 ms (27.3 -> 28.5 M solves/s).
     T rL, rR;
     bool ok, done;
     for (;;) {
       T dq0;
       F2 dq2[6];
       ik_iteration_packed<TZ, WRIST>(pt, q0, q2, tgt2, a.lambda, dq0, dq2, rL, rR);
-      ok = (rL < a.eps2) && (rR < a.eps2) && (it < a.max_iters);
+      ok = (rL < a.eps2) && (rR < a.eps2) && (w.it < a.max_iters);
       bool stalled = false;
-      if (a.early_stop && (it & 63) == 63) {
+      if (a.early_stop && (w.it & 63) == 63) {
         const T rs = rL + rR;
-        stalled = rs > T(0.9) * r_mark;
-        r_mark = rs;
+        stalled = rs > T(0.9) * w.r_mark;
+        w.r_mark = rs;
       }
-      done = ok || (it >= a.max_iters) || stalled;
+      done = ok || (w.it >= a.max_iters) || stalled;
       if (!done) {
         q0 = min_(max_(pt.lo0, q0 + a.dt * dq0), pt.hi0);
         const F2 dt2 = F2(a.dt);
 #pragma unroll
         for (int k = 0; k < 6; ++k) q2[k] = min_(max_(pt.lo[k], q2[k] + dt2 * dq2[k]), pt.hi[k]);
-        ++it;
+        ++w.it;
       }
-      if (!GIK_LANE2_INNER) break;
-      if (__any_sync(0xffffffffu, done && active)) break;
+      if (__any_sync(0xffffffffu, done && w.active)) break;
     }
-    const bool fused_event = MODE == MODE_BATCH && a.n_dst > 1 && __any_sync(0xffffffffu, done && active);
+    const bool fused_event = MODE == MODE_BATCH && a.n_dst > 1 && __any_sync(0xffffffffu, done && w.active);
     if (fused_event && !from_top) mark_publish(a, ms, lane);
-    if (done && active) {
-      // ---------------- rare path: this lane's problem ended ----------------
+    if (done && w.active) {
+      // ---------------- rare path: this lane's problem (edge step) ended ----------------
+      T cube[12];
       if (MODE == MODE_BATCH) {
-        const int64_t col = a.out_off + idx;
-        {                                       // this rank's own result arrays (peers: the pushers of block 0)
-          T* qo = a.q_dst[0];
-          store_q(qo, a.out_sc, a.out_si, col);
-          for (int p = 0; p < tab.n_passive; ++p) {
-            const int j = tab.passive_q[p];
-            T v = ld_in(a.q_init + (int64_t)j * a.q_sc + idx * a.q_si);
-            if (it > 0) v = min_(max_(tab.qlo[j], v), tab.qhi[j]);   // clamped by the first update (:89)
-            qo[(int64_t)j * a.out_sc + col * a.out_si] = v;
-          }
-          a.conv_dst[0][col] = ok ? 1 : 0;
-        }
-        if (a.iters) a.iters[idx] = it;
-        if (a.resid) { a.resid[idx * a.res_si] = sqrt_(rL); a.resid[a.res_sc + idx * a.res_si] = sqrt_(rR); }
-        active = false;
-      } else {
-        it_total += it;
-        if (ok) {
-          T* dst = a.q_out + (int64_t)(step - 1) * tab.nq * n_cols;
-          store_q(dst, n_cols, 1, idx);
-          for (int p = 0; p < tab.n_passive; ++p) {
-            const int j = tab.passive_q[p];
-            // passive joints: clamped once any update has been applied on this edge
-            T v = ld_in(a.q_init + (int64_t)j * a.q_sc + idx * a.q_si);
-            if (it_total > 0) v = min_(max_(tab.qlo[j], v), tab.qhi[j]);
-            dst[(int64_t)j * n_cols + idx] = v;
-          }
-        }
-        if (ok && step < nsteps) {
-          ++step;
-          it = 0;
-          r_mark = T(3.0e38);
-          T ca[12], cb[12], xi[6], cube[12];
-          load_cube(a.pose, a.pose_sc, a.pose_si, idx, ca);
-          load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
-          se3_delta(ca, cb, xi);
-          se3_advance(ca, xi, T(step) / T(nsteps), cube);
-          set_targets(cube);
-        } else {
-          a.n_valid[idx] = ok ? step : step - 1;
-          if (a.iters) a.iters[idx] = it_total;
-          active = false;
-        }
+        const T r[2] = {rL, rR};
+        batch_finish(tab, a, w, ok, true, store_q, 0, r);
+      } else if (edge_step_end(tab, a, w, ok, true, store_q, cube)) {
+        set_targets(cube);
       }
     }
-    if (fused_event) mark_update(ms, active, idx);      // (from_top warps: statistics only)
+    if (fused_event) mark_update(ms, w.active, w.idx);      // (from_top warps: statistics only)
   }
   if (MODE == MODE_BATCH && a.n_dst > 1) mark_stats(a, ms, lane, from_top);
   if (MODE == MODE_BATCH && a.n_dst > 1) mark_exit(a, lane);
@@ -806,35 +775,23 @@ gik_solve_lane2_kernel(const __grid_constant__ DevTable<float> tab, const __grid
 // register-resident in the latency-bound instantiations, lane-indexed constant loads in the large-batch fp64 one
 // (HOIST below).
 // ========================================================================================================
-#ifndef GIK_MINB_PAIR_F32
-#define GIK_MINB_PAIR_F32 3   // 165 registers: the hand's constants live in registers (HOIST below).  Measured against the
-                              // 96-register build with lane-indexed constant loads: config 4 40.1 -> 32.0 ms, 16 Ki problems
-                              // 1.33 -> 1.02 ms, 2 Ki problems 0.89 -> 0.67 ms (the same code capped at 96 registers: 44.5 ms)
-#endif
-#ifndef GIK_MINB_PAIR_F64
-#define GIK_MINB_PAIR_F64 3   // 168 registers, 12 warps / SM.  With the constant-bank sincos / atan2 the loop is bound by its FP64-pipe
-                              // instruction count, not by latency: 8, 9, 10, 11, 12 warps / SM all measure 9.2-9.5 M solves/s
-                              // (2^20 problems), 14 and 16 warps (144 / 128 registers + spills) 9.1 / 8.9 M
-#endif
-#ifndef GIK_PAIR_INNER
-#define GIK_PAIR_INNER true   // measured against the single-loop form: config 4 29.97 -> 27.12 ms, 2 Ki fp32 problems 0.64 -> 0.58 ms,
-                              // 16 Ki 1.00 -> 0.93 ms, fp64 small batches unchanged
-#endif
-#ifndef GIK_F64_HOIST_WARPS
-#define GIK_F64_HOIST_WARPS 8   // warps per SM (= its two resident blocks) up to which an fp64 launch takes the register-resident
-                                // instantiation: 12 Ki / 18 Ki problems 2.64 -> 2.47 ms against the 168-register one
-#endif
-#ifndef GIK_MINB_PAIR_F64_HOIST
-#define GIK_MINB_PAIR_F64_HOIST 1   // launches of <= GIK_F64_HOIST_WARPS warps per SM only: registers are free (252 used, two blocks per SM)
-#endif
-#ifndef GIK_MINB_PAIR_F64_WRIST
-#define GIK_MINB_PAIR_F64_WRIST 4   // large-batch fp64 instantiation of the spherical-wrist step
-#endif
+// Resident blocks per SM:
+//   fp32: 3 -- 165 registers: the hand's constants live in registers (HOIST below).  Measured against the 96-register
+//     build with lane-indexed constant loads: config 4 40.1 -> 32.0 ms, 16 Ki problems 1.33 -> 1.02 ms, 2 Ki problems
+//     0.89 -> 0.67 ms (the same code capped at 96 registers: 44.5 ms).
+//   fp64: 3 -- 168 registers, 12 warps / SM.  With the constant-bank sincos / atan2 the loop is bound by its FP64-pipe
+//     instruction count, not by latency: 8, 9, 10, 11, 12 warps / SM all measure 9.2-9.5 M solves/s (2^20 problems),
+//     14 and 16 warps (144 / 128 registers + spills) 9.1 / 8.9 M.
+//   fp64, spherical-wrist step: 4 (large batches).
+//   fp64 HOIST: 1 -- launches of <= kF64HoistWarps warps per SM only: registers are free (252 used, two blocks per SM).
 template <typename T, bool HOIST, bool WRIST> struct LaunchPair;
-template <bool HOIST, bool WRIST> struct LaunchPair<float, HOIST, WRIST>  { static constexpr int kMinBlocks = GIK_MINB_PAIR_F32; };
-template <> struct LaunchPair<double, false, false> { static constexpr int kMinBlocks = GIK_MINB_PAIR_F64; };
-template <> struct LaunchPair<double, false, true> { static constexpr int kMinBlocks = GIK_MINB_PAIR_F64_WRIST; };
-template <bool WRIST> struct LaunchPair<double, true, WRIST>  { static constexpr int kMinBlocks = GIK_MINB_PAIR_F64_HOIST; };
+template <bool HOIST, bool WRIST> struct LaunchPair<float, HOIST, WRIST>  { static constexpr int kMinBlocks = 3; };
+template <> struct LaunchPair<double, false, false> { static constexpr int kMinBlocks = 3; };
+template <> struct LaunchPair<double, false, true> { static constexpr int kMinBlocks = 4; };
+template <bool WRIST> struct LaunchPair<double, true, WRIST>  { static constexpr int kMinBlocks = 1; };
+// warps per SM (= its two resident blocks) up to which an fp64 launch takes the register-resident instantiation:
+// 12 Ki / 18 Ki problems 2.64 -> 2.47 ms against the 168-register one
+constexpr int kF64HoistWarps = 8;
 
 // HOIST: the hand's constants are selected into registers once instead of being fetched by lane-indexed constant loads
 // (39 LDC + their scoreboard waits per iteration), and the tip joint's constant outer product then comes from the table
@@ -843,13 +800,12 @@ template <bool WRIST> struct LaunchPair<double, true, WRIST>  { static constexpr
 // its two resident blocks per SM (<= 8 warps per SM); the large-batch fp64 kernel is bound by the FP64 pipe at 168 registers and keeps
 // the constant loads.
 template <typename T, int MODE, uint32_t TZ, bool HOIST = (sizeof(T) == 4), bool WRIST = false>
-__global__ void __launch_bounds__(GIK_THREADS, (LaunchPair<T, HOIST, WRIST>::kMinBlocks))
+__global__ void __launch_bounds__(kThreads, (LaunchPair<T, HOIST, WRIST>::kMinBlocks))
 gik_solve_pair_kernel(const __grid_constant__ DevTable<T> tab, const __grid_constant__ SolveArgs<T> a) {
   const int lane = threadIdx.x & 31;
   const int h = lane & 1;                       // hand of this lane
   const int off = 1 + 6 * h;                    // first active-joint slot of this hand's arm
   const unsigned lower_pairs = (1u << (lane & ~1)) - 1u;
-  const int64_t n_cols = a.n;
   const int64_t n = a.n_sel ? min(a.n, (int64_t)*a.n_sel) : a.n;
   if (MODE == MODE_BATCH && a.n_dst > 1 && (int)blockIdx.x < a.push_blocks) {   // fused all-gather: the leading blocks push, the others solve
     pusher_loop(a, tab.nq, n);
@@ -888,75 +844,60 @@ gik_solve_pair_kernel(const __grid_constant__ DevTable<T> tab, const __grid_cons
   for (int i = 0; i < 7; ++i) q[i] = T(0);
 #pragma unroll
   for (int c = 0; c < 12; ++c) tgt[c] = (c % 4 == 0 && c < 9) ? T(1) : T(0);
+  auto load_q = [&](int64_t idx) {
+    q[0] = ld_in(a.q_init + (int64_t)tab.act_q[0] * a.q_sc + idx * a.q_si);
+#pragma unroll
+    for (int k = 0; k < 6; ++k) q[1 + k] = ld_in(a.q_init + (int64_t)tab.act_q[off + k] * a.q_sc + idx * a.q_si);
+  };
+  auto store_q = [&](T* dst, int64_t sc, int64_t si, int64_t col) {   // this hand's arm; the chest from the even lane
+#pragma unroll
+    for (int k = 0; k < 6; ++k) dst[(int64_t)tab.act_q[off + k] * sc + col * si] = q[1 + k];
+    if (h == 0) dst[(int64_t)tab.act_q[0] * sc + col * si] = q[0];
+  };
 
-  int64_t idx = -1;
-  bool active = false, exhausted = false;
-  int it = 0, step = 0, nsteps = 0, it_total = 0;
+  Work<T> w;
+  bool exhausted = false;
   MarkState ms;              // fused all-gather: this warp's low-water mark
-  T r_mark = T(3.0e38);      // early stop: squared residual sum at the last 64-iteration checkpoint
 
   // `refill` (warp-uniform): some lane pair finished a problem in the previous trip (or the loop is starting), so the
   // queue / exit logic has to run.  GATED (the throughput-bound fp64 instantiation): while it is false -- almost every
   // trip -- the loop is the iteration, one vote and the back edge (measured +1.8 % on 2^20 fp64 problems).  The
   // latency-bound instantiations run the queue check every trip: gating it measured 6 % SLOWER on config 4 (30.0 ->
   // 31.8 ms; code layout of a 11 KB loop running from the instruction cache with one warp per sub-partition).
+  // INNER (the latency-bound instantiations): the iteration repeats in a loop of its own until an active pair finishes
+  // -- its trip is the arithmetic, one vote and the back edge; the queue / store logic above and below runs only then.
+  // Stall samples of the single-loop form put 14 % of a lone chain's time on its four branches per trip
+  // (branch_resolving + instruction fetch at the targets).  Measured against the single-loop form: config 4 29.97 ->
+  // 27.12 ms, 2 Ki fp32 problems 0.64 -> 0.58 ms, 16 Ki 1.00 -> 0.93 ms, fp64 small batches unchanged.  [The same idea
+  // as a FLAG in the single loop measured slower, 30.0 -> 31.8 ms.]
   constexpr bool GATED = !HOIST;
-  constexpr bool INNER = HOIST && GIK_PAIR_INNER;
+  constexpr bool INNER = HOIST;
   const T dt = a.dt, eps2 = a.eps2, lambda = a.lambda;
   const int max_iters = a.max_iters;
   bool refill = true;
   for (;;) {
-    const unsigned need = ((GATED && !refill) || exhausted) ? 0u : (__ballot_sync(0xffffffffu, enabled && !active) & 0x55555555u);
+    const unsigned need = ((GATED && !refill) || exhausted) ? 0u : (__ballot_sync(0xffffffffu, enabled && !w.active) & 0x55555555u);
     bool again = false;
     if (need) {
       const int64_t cand = queue_take(a, n, need, lane, __popc(need & lower_pairs), from_top, exhausted);
-      if (enabled && !active) {
-        if (cand >= 0) {
-          idx = a.sel ? a.sel[cand] : cand;
-          active = true;
-          it = a.it0 ? a.it0[idx] : 0;
-          r_mark = T(3.0e38);
-          q[0] = ld_in(a.q_init + (int64_t)tab.act_q[0] * a.q_sc + idx * a.q_si);
-#pragma unroll
-          for (int k = 0; k < 6; ++k) q[1 + k] = ld_in(a.q_init + (int64_t)tab.act_q[off + k] * a.q_sc + idx * a.q_si);
-          T cube[12];
-          load_cube(a.pose, a.pose_sc, a.pose_si, idx, cube);
-          if (MODE == MODE_EDGES) {
-            nsteps = ld_in(a.num_steps + idx);
-            step = 1;
-            it_total = 0;
-            T cb[12], xi[6], ca[12];
-#pragma unroll
-            for (int c = 0; c < 12; ++c) ca[c] = cube[c];
-            load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
-            se3_delta(ca, cb, xi);
-            se3_advance(ca, xi, T(1) / T(nsteps), cube);
-            if (nsteps < 1) {
-              if (h == 0) { a.n_valid[idx] = 0; if (a.iters) a.iters[idx] = 0; }
-              active = false;
-            }
-          }
-          hook_target(ac, cube, tgt);
-        }
+      if (enabled && !w.active && cand >= 0) {
+        T cube[12];
+        work_start<T, MODE>(a, cand, h == 0, w, load_q, cube);
+        hook_target(ac, cube, tgt);
       }
       // an edge with nothing to march leaves its pair idle although the queue has more: come back next trip
-      if (GATED && MODE == MODE_EDGES) again = !exhausted && __any_sync(0xffffffffu, enabled && !active);
+      if (GATED && MODE == MODE_EDGES) again = !exhausted && __any_sync(0xffffffffu, enabled && !w.active);
     }
     if constexpr (INNER) {
-      if (!__any_sync(0xffffffffu, active)) {
+      if (!__any_sync(0xffffffffu, w.active)) {
         if (exhausted) break;
         continue;                                // (edges with nothing to march) back to the queue
       }
     } else {
-      if ((!GATED || refill) && exhausted && !__any_sync(0xffffffffu, active)) break;
+      if ((!GATED || refill) && exhausted && !__any_sync(0xffffffffu, w.active)) break;
     }
 
     // ---------------- one descent iteration: this lane's hand ----------------
-    // INNER (the latency-bound instantiations): the iteration repeats in a loop of its own until an active pair
-    // finishes -- its trip is the arithmetic, one vote and the back edge; the queue / store logic above and below runs
-    // only then.  Stall samples of the single-loop form put 14 % of a lone chain's time on its four branches per trip
-    // (branch_resolving + instruction fetch at the targets).  [The same idea as a FLAG in the single loop measured
-    // slower, 30.0 -> 31.8 ms; as a loop it is 27.1 ms.]
     bool ok, done;
     T r;
     for (;;) {
@@ -975,15 +916,15 @@ gik_solve_pair_kernel(const __grid_constant__ DevTable<T> tab, const __grid_cons
       if constexpr (WRIST) hand_wrist_phase2(wst, kappa, dqa);
       else hand_phase2(hs, kappa, dqa);
       const T rL = h ? r_o : r, rR = h ? r : r_o;
-      ok = (rL < eps2) && (rR < eps2) && (it < max_iters);
+      ok = (rL < eps2) && (rR < eps2) && (w.it < max_iters);
       bool stalled = false;
-      if (a.early_stop && (it & 63) == 63) {
+      if (a.early_stop && (w.it & 63) == 63) {
         const T rs = rL + rR;
-        stalled = rs > T(0.9) * r_mark;
-        r_mark = rs;
+        stalled = rs > T(0.9) * w.r_mark;
+        w.r_mark = rs;
       }
-      done = ok || (it >= max_iters) || stalled;
-      if constexpr (GATED) refill = __any_sync(0xffffffffu, done && active) || again;
+      done = ok || (w.it >= max_iters) || stalled;
+      if constexpr (GATED) refill = __any_sync(0xffffffffu, done && w.active) || again;
       if (!done) {
         if constexpr (HOIST) {
           q[0] = min_(max_(lim_lo[0], q[0] + dt * kappa), lim_hi[0]);
@@ -995,56 +936,23 @@ gik_solve_pair_kernel(const __grid_constant__ DevTable<T> tab, const __grid_cons
           for (int k = 0; k < 6; ++k)
             q[1 + k] = min_(max_(tab.lo[off + k], q[1 + k] + dt * dqa[k]), tab.hi[off + k]);
         }
-        ++it;
+        ++w.it;
       }
       if (!INNER) break;
-      if (__any_sync(0xffffffffu, done && active)) break;
+      if (__any_sync(0xffffffffu, done && w.active)) break;
     }
-    const bool fused_event = MODE == MODE_BATCH && a.n_dst > 1 && __any_sync(0xffffffffu, done && active);
+    const bool fused_event = MODE == MODE_BATCH && a.n_dst > 1 && __any_sync(0xffffffffu, done && w.active);
     if (fused_event && !from_top) mark_publish(a, ms, lane);
-    if (done && active) {
-      const bool batch = (MODE == MODE_BATCH);
-      if (!batch) it_total += it;
-      if (batch || ok) {                        // store q: batch result, or path row of a converged edge step
-        const bool moved = batch ? (it > 0) : (it_total > 0);
-        const int64_t ld = batch ? a.out_sc : n_cols, cs_ = batch ? a.out_si : 1, col = batch ? a.out_off + idx : idx;
-        {                                       // batch: this rank's own result arrays (peers: the pushers of block 0)
-          constexpr int d = 0;
-          T* dst = batch ? a.q_dst[d] : a.q_out + (int64_t)(step - 1) * tab.nq * n_cols;
-#pragma unroll
-          for (int k = 0; k < 6; ++k) dst[(int64_t)tab.act_q[off + k] * ld + col * cs_] = q[1 + k];
-          if (h == 0) {
-            dst[(int64_t)tab.act_q[0] * ld + col * cs_] = q[0];
-            for (int p = 0; p < tab.n_passive; ++p) {
-              const int j = tab.passive_q[p];
-              T v = ld_in(a.q_init + (int64_t)j * a.q_sc + idx * a.q_si);
-              if (moved) v = min_(max_(tab.qlo[j], v), tab.qhi[j]);   // clamped by the first update (:89)
-              dst[(int64_t)j * ld + col * cs_] = v;
-            }
-            if (batch) a.conv_dst[d][col] = ok ? 1 : 0;
-          }
-        }
-      }
-      if (batch) {
-        if (h == 0 && a.iters) a.iters[idx] = it;
-        if (a.resid) a.resid[(int64_t)h * a.res_sc + idx * a.res_si] = sqrt_(r);
-        active = false;
-      } else if (ok && step < nsteps) {
-        ++step;
-        it = 0;
-        r_mark = T(3.0e38);
-        T ca[12], cb[12], xi[6], cube[12];
-        load_cube(a.pose, a.pose_sc, a.pose_si, idx, ca);
-        load_cube(a.pose_b, a.pose_sc, a.pose_si, idx, cb);
-        se3_delta(ca, cb, xi);
-        se3_advance(ca, xi, T(step) / T(nsteps), cube);
+    if (done && w.active) {
+      T cube[12];
+      if (MODE == MODE_BATCH) {
+        const T rh[1] = {r};
+        batch_finish(tab, a, w, ok, h == 0, store_q, h, rh);
+      } else if (edge_step_end(tab, a, w, ok, h == 0, store_q, cube)) {
         hook_target(ac, cube, tgt);
-      } else {
-        if (h == 0) { a.n_valid[idx] = ok ? step : step - 1; if (a.iters) a.iters[idx] = it_total; }
-        active = false;
       }
     }
-    if (fused_event) mark_update(ms, active, idx);      // (from_top warps: statistics only)
+    if (fused_event) mark_update(ms, w.active, w.idx);      // (from_top warps: statistics only)
   }
   if (MODE == MODE_BATCH && a.n_dst > 1) mark_exit(a, lane);
 }
@@ -1203,18 +1111,14 @@ template <typename Kernel>
 int grid_dims(gik_handle_t h, Kernel kernel, int64_t n, int max_per_warp, int* blocks, int* per_warp, int64_t* max_warps_out,
               int reserve = 0) {   // reserve: resident block slots kept free (the pusher block of a fused launch)
   int occ = 0;
-  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, GIK_THREADS, 0);
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, kThreads, 0);
   if (e != cudaSuccess) return (int)e;
   if (occ < 1) occ = 1;
-  const int64_t warps_per_block = GIK_THREADS / 32;
+  const int64_t warps_per_block = kThreads / 32;
   const int64_t max_blocks = (int64_t)h->sm_count * occ - reserve;
   const int64_t max_warps = max_blocks * warps_per_block;
   const int64_t target_warps = (int64_t)h->sm_count * 4;      // one warp per SM sub-partition
   int64_t Lw = (n + target_warps - 1) / target_warps;
-  if (const char* env = getenv("GIK_PER_WARP")) {              // experiment hook: problems (pairs) per warp
-    const int v = atoi(env);
-    if (v > 0) Lw = v;
-  }
   int L = (int)(Lw < 1 ? 1 : (Lw > max_per_warp ? max_per_warp : Lw));
   int64_t warps = (n + L - 1) / L;
   int64_t b = (warps + warps_per_block - 1) / warps_per_block;
@@ -1226,10 +1130,6 @@ int grid_dims(gik_handle_t h, Kernel kernel, int64_t n, int max_per_warp, int* b
   return GIK_OK;
 }
 
-// fp32: lane kernel when the batch can give (at least) half of the lanes of every resident warp a problem, pair kernel
-// below that.  fp64: always the pair kernel -- one hand per lane halves the live state, which at 2 registers per value
-// is worth more than the shared chest work (measured 7.0M vs 6.0M solves/s on 2^20 problems).
-// params.flags can force either (GIK_F_LANE_KERNEL / GIK_F_PAIR_KERNEL) for A/B measurements.
 // Which form of the step a launch runs: the spherical-wrist form (two 3x3 solves per hand) needs an undamped step and
 // a table with the wrist's zero pattern (instantiated for the Nextage pattern); everything else -- damping > 0, other
 // tables of the compiled topology, GIK_F_CHOLESKY -- takes the block Cholesky + Sherman-Morrison form.
@@ -1239,41 +1139,64 @@ bool use_wrist(gik_handle_t h, const gik_params_t* prm) {
   return (tab.tzero & kNextageTZ) == kNextageTZ && prm->damping == 0.0 && !(prm->flags & GIK_F_CHOLESKY);
 }
 
+// The solve kernel instantiation one launch runs.  choose_launch picks it; the grid is sized, the kernel launched and
+// its name reported from this one choice.
+struct SolveKernel {
+  enum Family { LANE, LANE2, PAIR } family;   // scalar lane kernel, packed fp32 lane kernel, pair kernel
+  bool nx;      // TZ = kNextageTZ: the table has (at least) the Nextage zero pattern, so those FMAs are skipped
+  bool wrist;   // WRIST: the spherical-wrist step (implies nx)
+  bool hoist;   // pair kernel, HOIST: the hand's constants in registers (fp32: always)
+};
+
+// f(kernel) for the instantiation k names
+template <typename T, int MODE, typename F>
+int with_kernel(const SolveKernel& k, F&& f) {
+  constexpr uint32_t NX = kNextageTZ;
+  if (k.family == SolveKernel::PAIR) {
+    if constexpr (sizeof(T) == 8) {
+      if (!k.hoist) return k.wrist ? f(gik_solve_pair_kernel<T, MODE, NX, false, true>)
+                           : k.nx  ? f(gik_solve_pair_kernel<T, MODE, NX, false>) : f(gik_solve_pair_kernel<T, MODE, 0, false>);
+    }
+    return k.wrist ? f(gik_solve_pair_kernel<T, MODE, NX, true, true>)
+         : k.nx  ? f(gik_solve_pair_kernel<T, MODE, NX, true>) : f(gik_solve_pair_kernel<T, MODE, 0, true>);
+  }
+  if constexpr (sizeof(T) == 4) {
+    if (k.family == SolveKernel::LANE2)
+      return k.wrist ? f(gik_solve_lane2_kernel<MODE, NX, true>)
+           : k.nx  ? f(gik_solve_lane2_kernel<MODE, NX>) : f(gik_solve_lane2_kernel<MODE, 0>);
+  }
+  return k.wrist ? f(gik_solve_kernel<T, MODE, NX, true>) : k.nx ? f(gik_solve_kernel<T, MODE, NX>) : f(gik_solve_kernel<T, MODE, 0>);
+}
+
 // fp32: lane kernel when the batch can give (at least) half of the lanes of every resident warp a problem, pair kernel
 // below that.  fp64: always the pair kernel -- one hand per lane halves the live state, which at 2 registers per value
 // is worth more than the shared chest work (measured 7.0M vs 6.0M solves/s on 2^20 problems).
-// params.flags can force either (GIK_F_LANE_KERNEL / GIK_F_PAIR_KERNEL) for A/B measurements.
+// flags can force either (GIK_F_LANE_KERNEL / GIK_F_PAIR_KERNEL) for A/B measurements, and the scalar fp32 lane kernel
+// (GIK_F_SCALAR_LANE).  `reserve`: resident block slots kept free (the pusher blocks of a fused launch).
 template <typename T, int MODE>
-int choose_launch(gik_handle_t h, int64_t n, int flags, bool wrist, int* blocks, int* per_warp, bool* pair, bool* hoist = nullptr,
-                  int reserve = 0) {
+int choose_launch(gik_handle_t h, int64_t n, int flags, bool wrist, int reserve, SolveKernel* k, int* blocks, int* per_warp) {
+  const bool nx = (table_of<T>(h).tzero & kNextageTZ) == kNextageTZ;
+  *k = {sizeof(T) == 4 && !(flags & GIK_F_SCALAR_LANE) ? SolveKernel::LANE2 : SolveKernel::LANE, nx, wrist, false};
   int64_t max_warps = 0;
-  int rc;
-  if constexpr (sizeof(T) == 4) {
-    if (flags & GIK_F_SCALAR_LANE) rc = grid_dims(h, gik_solve_kernel<T, MODE, 0>, n, 32, blocks, per_warp, &max_warps, reserve);
-    else if (wrist) rc = grid_dims(h, gik_solve_lane2_kernel<MODE, kNextageTZ, true>, n, 32, blocks, per_warp, &max_warps, reserve);
-    else rc = grid_dims(h, gik_solve_lane2_kernel<MODE, 0>, n, 32, blocks, per_warp, &max_warps, reserve);
-  } else {
-    rc = grid_dims(h, gik_solve_kernel<T, MODE, 0>, n, 32, blocks, per_warp, &max_warps, reserve);
-  }
+  int rc = with_kernel<T, MODE>(*k, [&](auto kern) { return grid_dims(h, kern, n, 32, blocks, per_warp, &max_warps, reserve); });
   if (rc) return rc;
-  *pair = sizeof(T) == 8 || n <= 16 * max_warps;
-  if (flags & GIK_F_LANE_KERNEL) *pair = false;
-  if (flags & GIK_F_PAIR_KERNEL) *pair = true;
+  bool pair = sizeof(T) == 8 || n <= 16 * max_warps;
+  if (flags & GIK_F_LANE_KERNEL) pair = false;
+  if (flags & GIK_F_PAIR_KERNEL) pair = true;
+  if (!pair) return GIK_OK;
+  k->family = SolveKernel::PAIR;
   // fp64 pair kernel with register-resident constants: launches of at most one full warp per SM sub-partition
-  const bool hz = *pair && sizeof(T) == 8 && n <= (int64_t)16 * GIK_F64_HOIST_WARPS * h->sm_count;
-  if (hoist) *hoist = hz;
-  if (*pair) {
-    if constexpr (sizeof(T) == 8) {
-      if (wrist) rc = hz ? grid_dims(h, gik_solve_pair_kernel<T, MODE, kNextageTZ, true, true>, n, 16, blocks, per_warp, nullptr, reserve)
-                         : grid_dims(h, gik_solve_pair_kernel<T, MODE, kNextageTZ, false, true>, n, 16, blocks, per_warp, nullptr, reserve);
-      else rc = hz ? grid_dims(h, gik_solve_pair_kernel<T, MODE, 0, true>, n, 16, blocks, per_warp, nullptr, reserve)
-                   : grid_dims(h, gik_solve_pair_kernel<T, MODE, 0, false>, n, 16, blocks, per_warp, nullptr, reserve);
-    } else {
-      rc = wrist ? grid_dims(h, gik_solve_pair_kernel<T, MODE, kNextageTZ, true, true>, n, 16, blocks, per_warp, nullptr, reserve)
-                 : grid_dims(h, gik_solve_pair_kernel<T, MODE, 0>, n, 16, blocks, per_warp, nullptr, reserve);
-    }
-  }
-  return rc;
+  k->hoist = sizeof(T) == 4 || n <= (int64_t)16 * kF64HoistWarps * h->sm_count;
+  return with_kernel<T, MODE>(*k, [&](auto kern) { return grid_dims(h, kern, n, 16, blocks, per_warp, nullptr, reserve); });
+}
+
+template <typename T>
+void launch_kernel(void (*kern)(DevTable<T>, SolveArgs<T>), int blocks, cudaStream_t st, gik_handle_t h, const SolveArgs<T>& a) {
+  kern<<<blocks, kThreads, 0, st>>>(table_of<T>(h), a);
+}
+void launch_kernel(void (*kern)(DevTable<float>, PackedTable, SolveArgs<float>), int blocks, cudaStream_t st, gik_handle_t h,
+                   const SolveArgs<float>& a) {
+  kern<<<blocks, kThreads, 0, st>>>(h->tab32, h->pt32, a);
 }
 
 // force: a continuation launch that must run every problem to the iteration cap -- eps^2 = 0 can never be undercut
@@ -1287,60 +1210,40 @@ int launch_solve(gik_handle_t h, SolveArgs<T>& a, const gik_params_t* prm, void*
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
   int blocks = 0, lanes = 32;
-  bool pair = false, hoist = false;
-  const bool wrist = use_wrist<T>(h, prm);
+  SolveKernel k;
   const int pushers = (MODE == MODE_BATCH && a.n_dst > 1) ? a.push_blocks : 0;   // fused all-gather: the leading blocks push (see "Fused all-gather")
-  int rc = choose_launch<T, MODE>(h, a.n, prm->flags, wrist, &blocks, &lanes, &pair, &hoist, pushers);
+  int rc = choose_launch<T, MODE>(h, a.n, prm->flags, use_wrist<T>(h, prm), pushers, &k, &blocks, &lanes);
   if (rc) return rc;
   if (pushers) {
-    a.n_marks = blocks * (GIK_THREADS / 32);
+    a.n_marks = blocks * (kThreads / 32);
     // the warps in the upper half of the SM's occupied warp slots -- the low-priority ones -- work from the top of the slab
     // (queue_take); needs both counters in one 64-bit word and a device-resident batch handed out by index
-    const bool two_ended = a.n < (1ll << 31) && !a.ready && !a.sel && !getenv("GIK_FUSED_ONE_ENDED");
+    const bool two_ended = a.n < (1ll << 31) && !a.ready && !a.sel;
     const int per_sm = (blocks + pushers + h->sm_count - 1) / h->sm_count;     // blocks per SM of this launch
-    a.top_from = (two_ended && per_sm >= 2) ? (per_sm + 1) / 2 * (GIK_THREADS / 32) : 0;
+    a.top_from = (two_ended && per_sm >= 2) ? (per_sm + 1) / 2 * (kThreads / 32) : 0;
     blocks += pushers;
   }
   a.lanes = lanes;
   a.queue = h->queues + (h->next_queue.fetch_add(1, std::memory_order_relaxed) % kQueueSlots);
   cudaError_t qe = cudaMemsetAsync(a.queue, 0, sizeof(unsigned long long), (cudaStream_t)stream);
   if (qe != cudaSuccess) return (int)qe;
-  const DevTable<T>& tab = table_of<T>(h);
-  const bool nx = (tab.tzero & kNextageTZ) == kNextageTZ;   // table has (at least) the Nextage zero pattern: skip those FMAs
-  cudaStream_t st = (cudaStream_t)stream;
-  constexpr uint32_t NX = kNextageTZ;
-  if (pair) {
-    if constexpr (sizeof(T) == 8) {
-      if (hoist) {
-        if (wrist) gik_solve_pair_kernel<T, MODE, NX, true, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-        else if (nx) gik_solve_pair_kernel<T, MODE, NX, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-        else gik_solve_pair_kernel<T, MODE, 0, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-      } else {
-        if (wrist) gik_solve_pair_kernel<T, MODE, NX, false, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-        else if (nx) gik_solve_pair_kernel<T, MODE, NX, false><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-        else gik_solve_pair_kernel<T, MODE, 0, false><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-      }
-    } else {
-      if (wrist) gik_solve_pair_kernel<T, MODE, NX, true, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-      else if (nx) gik_solve_pair_kernel<T, MODE, NX><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-      else gik_solve_pair_kernel<T, MODE, 0><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-    }
-  } else if constexpr (sizeof(T) == 4) {
-    if (prm->flags & GIK_F_SCALAR_LANE) {
-      if (wrist) gik_solve_kernel<T, MODE, NX, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-      else if (nx) gik_solve_kernel<T, MODE, NX><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-      else gik_solve_kernel<T, MODE, 0><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-    } else {                                             // packed FFMA2 lane kernel (default for fp32)
-      if (wrist) gik_solve_lane2_kernel<MODE, NX, true><<<blocks, GIK_THREADS, 0, st>>>(tab, h->pt32, a);
-      else if (nx) gik_solve_lane2_kernel<MODE, NX><<<blocks, GIK_THREADS, 0, st>>>(tab, h->pt32, a);
-      else gik_solve_lane2_kernel<MODE, 0><<<blocks, GIK_THREADS, 0, st>>>(tab, h->pt32, a);
-    }
-  } else {
-    if (wrist) gik_solve_kernel<T, MODE, NX, true><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-    else if (nx) gik_solve_kernel<T, MODE, NX><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-    else gik_solve_kernel<T, MODE, 0><<<blocks, GIK_THREADS, 0, st>>>(tab, a);
-  }
-  return (int)cudaGetLastError();
+  return with_kernel<T, MODE>(k, [&](auto kern) {
+    launch_kernel(kern, blocks, (cudaStream_t)stream, h, a);
+    return (int)cudaGetLastError();
+  });
+}
+
+// The launch gik_solve_f32/f64 makes for n problems with the default parameters and these flags (GIK_F_CHOLESKY selects
+// the step form, the kernel flags the kernel)
+int batch_launch(gik_handle_t h, int elem_size, int64_t n, int flags, SolveKernel* k, int* blocks) {
+  DeviceGuard g(h->device);
+  if (g.err != cudaSuccess) return (int)g.err;
+  gik_params_t dp;
+  gik_default_params(&dp);
+  dp.flags = flags & GIK_F_CHOLESKY;
+  int lanes = 0;
+  if (elem_size == 4) return choose_launch<float, MODE_BATCH>(h, n, flags, use_wrist<float>(h, &dp), 0, k, blocks, &lanes);
+  return choose_launch<double, MODE_BATCH>(h, n, flags, use_wrist<double>(h, &dp), 0, k, blocks, &lanes);
 }
 
 template <typename T>
@@ -1426,7 +1329,7 @@ int scatter_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const
   // scratch: marks (one per warp of the largest grid any solve kernel takes; zero = "nothing finished yet"), the pushers'
   // control words + statistics, one flag per chunk
   const int64_t n_chunks = (n + kChunk - 1) / kChunk;
-  const int64_t n_marks = (int64_t)h->sm_count * 16 * (GIK_THREADS / 32);
+  const int64_t n_marks = (int64_t)h->sm_count * 16 * (kThreads / 32);
   const size_t marks_bytes = ((size_t)n_marks * sizeof(int32_t) + 255) / 256 * 256, ctl_bytes = 2048;
   char* scratch = nullptr;
   cudaError_t e = cudaMallocAsync((void**)&scratch, marks_bytes + ctl_bytes + (size_t)n_chunks, st);
@@ -1439,7 +1342,6 @@ int scatter_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const
   // pusher blocks: one (a lookout + three pushing warps) keeps pace with one or two destinations; more destinations
   // mean more stores per chunk
   a.push_blocks = n_peers <= 3 ? 1 : 2;
-  if (const char* env = getenv("GIK_PUSH_BLOCKS")) { const int v = atoi(env); if (v >= 1 && v <= 8) a.push_blocks = v; }
   const bool stats = getenv("GIK_FUSED_STATS") != nullptr;     // measurement hook (synchronises the stream)
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   if (stats) {
@@ -1466,7 +1368,7 @@ int scatter_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const
               (long long)k, (long long)n_chunks, t_solve, (long long)r, t_rest);
       long long pw[28];
       if (a.n_marks > 0 && cudaMemcpy(pw, a.push_ctl, sizeof(pw), cudaMemcpyDeviceToHost) == cudaSuccess)
-        for (int w = 0; w < 8 && w < a.push_blocks * (GIK_THREADS / 32); ++w)
+        for (int w = 0; w < 8 && w < a.push_blocks * (kThreads / 32); ++w)
           fprintf(stderr, w == 0 ? "  lookout warp: %lld looks, looking %lld us, sleeping %lld us\n" : "  pusher warp: %lld chunks, pushing %lld us, waiting %lld us\n",
                   pw[4 + 3 * w + 2], pw[4 + 3 * w], pw[4 + 3 * w + 1]);
       if (a.warp_stats && a.n_marks > 0 && 2 * a.n_marks <= n_marks / 2) {
@@ -1479,9 +1381,9 @@ int scatter_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const
           fprintf(stderr, "  finish events per compute warp: min %d, mean %.1f, max %d; histogram over [min, max] in 8 bins:", lo, (double)sum / a.n_marks, hi);
           for (int b = 0; b < 8; ++b) fprintf(stderr, " %d", hist[b]);
           fprintf(stderr, "\n  by sub-partition slot (warp index in block), mean events:");
-          for (int k = 0; k < GIK_THREADS / 32; ++k) {
+          for (int k = 0; k < kThreads / 32; ++k) {
             long long sk = 0; int nk = 0;
-            for (int w = k; w < a.n_marks; w += GIK_THREADS / 32) { sk += ws[2 * w]; ++nk; }
+            for (int w = k; w < a.n_marks; w += kThreads / 32) { sk += ws[2 * w]; ++nk; }
             fprintf(stderr, " %.1f", nk ? (double)sk / nk : 0.0);
           }
           fprintf(stderr, "\n  by launch order of the block (quarters of the compute grid), mean events:");
@@ -1737,41 +1639,31 @@ int gik_solve_launch_dims(gik_handle_t h, int elem_size, int64_t n, int32_t* blo
   if (bad_handle(h)) return GIK_E_HANDLE;
   if (!blocks || !threads) return GIK_E_NULL;
   if (n < 0) return GIK_E_SIZE;
-  DeviceGuard g(h->device);
-  if (g.err != cudaSuccess) return (int)g.err;
-  int b = 0, l = 32, rc;
-  bool pair = false;
-  gik_params_t dp;
-  gik_default_params(&dp);
-  if (elem_size == 4) rc = choose_launch<float, MODE_BATCH>(h, n, 0, use_wrist<float>(h, &dp), &b, &l, &pair);
-  else if (elem_size == 8) rc = choose_launch<double, MODE_BATCH>(h, n, 0, use_wrist<double>(h, &dp), &b, &l, &pair);
-  else return GIK_E_PARAM;
+  if (elem_size != 4 && elem_size != 8) return GIK_E_PARAM;
+  SolveKernel k;
+  int b = 0;
+  const int rc = batch_launch(h, elem_size, n, 0, &k, &b);
   if (rc) return rc;
-  *blocks = b; *threads = GIK_THREADS;
+  *blocks = b; *threads = kThreads;
   return GIK_OK;
 }
 
 const char* gik_solve_kernel_name(gik_handle_t h, int elem_size, int64_t n, int flags) {
   if (bad_handle(h) || n < 0 || (elem_size != 4 && elem_size != 8)) return "";
-  DeviceGuard g(h->device);
-  if (g.err != cudaSuccess) return "";
-  int b = 0, l = 32, rc;
-  bool pair = false;
-  gik_params_t dp;
-  gik_default_params(&dp);
-  dp.flags = flags & GIK_F_CHOLESKY;
-  if (elem_size == 4) rc = choose_launch<float, MODE_BATCH>(h, n, flags, use_wrist<float>(h, &dp), &b, &l, &pair);
-  else rc = choose_launch<double, MODE_BATCH>(h, n, flags, use_wrist<double>(h, &dp), &b, &l, &pair);
-  if (rc) return "";
-  const bool wrist = elem_size == 4 ? use_wrist<float>(h, &dp) : use_wrist<double>(h, &dp);
-  if (wrist) {
-    if (pair) return elem_size == 4 ? "gik_solve_pair_kernel<float, wrist>" : "gik_solve_pair_kernel<double, wrist>";
-    if (elem_size == 8) return "gik_solve_kernel<double, wrist>";
-    return (flags & GIK_F_SCALAR_LANE) ? "gik_solve_kernel<float, wrist>" : "gik_solve_lane2_kernel<wrist>";
+  SolveKernel k;
+  int b = 0;
+  if (batch_launch(h, elem_size, n, flags, &k, &b)) return "";
+  const bool f64 = elem_size == 8;
+  switch (k.family) {
+    case SolveKernel::PAIR:
+      if (k.wrist) return f64 ? "gik_solve_pair_kernel<double, wrist>" : "gik_solve_pair_kernel<float, wrist>";
+      return f64 ? "gik_solve_pair_kernel<double>" : "gik_solve_pair_kernel<float>";
+    case SolveKernel::LANE:
+      if (k.wrist) return f64 ? "gik_solve_kernel<double, wrist>" : "gik_solve_kernel<float, wrist>";
+      return f64 ? "gik_solve_kernel<double>" : "gik_solve_kernel<float>";
+    default:
+      return k.wrist ? "gik_solve_lane2_kernel<wrist>" : "gik_solve_lane2_kernel";
   }
-  if (pair) return elem_size == 4 ? "gik_solve_pair_kernel<float>" : "gik_solve_pair_kernel<double>";
-  if (elem_size == 8) return "gik_solve_kernel<double>";
-  return (flags & GIK_F_SCALAR_LANE) ? "gik_solve_kernel<float>" : "gik_solve_lane2_kernel";
 }
 
 const char* gik_strerror(int code) {

@@ -77,9 +77,8 @@ GIK_HD void tree_scan_nearest(const T* tree, int64_t cap, int nv, const T* targe
 
 // grow() of path.computepath (path.py:241-244) for the edges [e0, e1) of ONE tree (in edge order).  Edge e appends
 // its start configuration q_start[:, e] again, with placement pose_a[:, e], as a child of near[e], then its
-// n_valid[e] steps q_path[j][:, e], each the child of the previous vertex; step j was solved for the placement
-// pose_a * exp6(alpha log6(pose_a^-1 pose_b)), alpha = (j+1) / num_steps[e] -- the same se3_delta / se3_advance
-// calls and the same expression as the edge kernel, so the stored placement is the one the step was solved for.
+// n_valid[e] steps q_path[j][:, e], each the child of the previous vertex; step j stores edge_placement of step j + 1,
+// the placement the edge kernel solved that step for.
 // n_valid[e] < 0 marks an edge that was not projected: it appends nothing and seg_end[e] = -1.  Otherwise seg_end[e]
 // is the index of the segment's last vertex.  If the vertices would exceed cap, the tree is left unchanged, every
 // seg_end of the range is -1 and the function returns false.  q_path is [max_steps][nq][E]; a step count above
@@ -106,7 +105,7 @@ GIK_HD bool tree_append(int nq, int64_t cap, int max_steps, int64_t E, int64_t e
     ++n;
     if (m > 0) se3_delta(a, b, xi);
     for (int j = 0; j < m; ++j) {
-      se3_advance(a, xi, T(j + 1) / T(num_steps[e]), cube);
+      edge_placement(a, xi, j + 1, num_steps[e], cube);
       for (int c = 0; c < nq; ++c) verts[c * cap + n] = q_path[((int64_t)j * nq + c) * E + e];
       for (int c = 0; c < 12; ++c) cubes[c * cap + n] = cube[c];
       parent[n] = (int32_t)(n - 1);

@@ -67,7 +67,7 @@ static int solve_impl(const gik_table_t* tab, int64_t n, const T* q_init, const 
     int it = 0;
     bool ok = false;
     for (;;) {
-      // same specialisation rule as launch_solve() in csrc/gik_kernels.cu
+      // same specialisation rule as choose_launch() in csrc/gik_kernels.cu
       const bool nx = (d.tzero & kNextageTZ) == kNextageTZ && !generic;
       bool done_packed = false;
       if constexpr (sizeof(T) == 4) {
