@@ -4,6 +4,7 @@
   inverse_geometry.py:105-120  -> grasp poses q0 / qe for CUBE_PLACEMENT / CUBE_PLACEMENT_TARGET
   path.py:282-303              -> RRT-connect path that carries the cube over the obstacle
   control.py:431-452           -> Bezier trajectory through the path (closed-form fit)
+  control.py:416-463           -> can the trajectory be executed?  (checked at the controller's 1501 sample times)
 
     python examples/grasp_and_plan.py            (needs a CUDA device)
 """
@@ -43,6 +44,10 @@ def main():
     q_of_t, vq_of_t, vvq_of_t = trajs
     print(f"trajectory: degree {q_of_t.degree_}, fit accepted {ok}  ({(t3 - t2) * 1e3:.1f} ms); "
           f"|v(0)| {np.abs(vq_of_t(0.0)).max():.1e}, |a(T)| {np.abs(vvq_of_t(15.0)).max():.1e}")
+    verdict = gik_b200.check_trajectory(q_of_t)
+    t4 = time.perf_counter()
+    print(f"check: valid {verdict['valid']}, first bad sample {verdict['first_bad']} (reason {verdict['reason']}: "
+          f"1 limits, 2 grasp, 4 collision), max grasp error {verdict['grasp_err']:.2e}  ({(t4 - t3) * 1e3:.1f} ms)")
     return 0
 
 

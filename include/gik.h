@@ -368,6 +368,42 @@ int gik_tree_paths_f64(gik_handle_t h, int64_t n_queries, int32_t cap, const dou
                        const int32_t* parent, const int32_t* n_verts, const int32_t* start_end, const int32_t* goal_end,
                        int64_t* offsets, double* q, double* cube, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Trajectory check: can a fitted trajectory be executed?  The reference finds out only by running its 1500 pybullet
+ * control steps (control.py:416-463): between the path vertices the least-squares curve lies on no grasp manifold, and
+ * its free control points are unconstrained.  This checks the curve itself at the controller's sample times.
+ *
+ * Input: n_traj trajectories as Bezier control points ctrl [n_traj][n_ctrl][nq] (row-major, what gik_bezier_fit_*
+ * writes) and the Bernstein weights of n_samples parameters u_k = k / (n_samples - 1): weights [n_samples][n_ctrl],
+ * weights[k][i] = C(n_ctrl - 1, i) u_k^i (1 - u_k)^(n_ctrl - 1 - i), computed by the caller (in fp64, then rounded to
+ * the kernel's type).  The controller runs 1500 steps of 0.01 s over T = 15 s, so 1501 samples cover every step and the
+ * end point; time only rescales u, so positions need no T.  For every sample (n, k):
+ *   1. q = sum_i weights[k][i] * ctrl[n][i]  (i ascending).
+ *   2. bit 0 (joint limits): some q_j < lower_j - limit_tol or q_j > upper_j + limit_tol (a NaN q_j counts).  limit_tol
+ *      absorbs the round-off of the weights on a curve that lies on a limit.
+ *   3. bit 1 (grasp): hand frames H_h = oMi[hand_joint[h]] * hand offset (LARM_EFF / RARM_EFF), the cube placement each
+ *      hand implies C_h = H_h * hook_h^-1, and the grasp error g = ||log6(C_L^-1 * C_R)||_2 -- zero exactly when both
+ *      hands sit on the hooks of one rigid cube; the same norm as the IK residual, and the same log6, near-pi form
+ *      included.  The bit is set when g > grasp_tol (or g is NaN).
+ *   4. bit 2 (collisions): the carried cube is placed at C_L (the left hand carries the pose; the right hand's deviation
+ *      is g) and some pair of "list 3" intersects.  List 3, built by gik_scene_attach, is every pair of the scene except
+ *      the pairs of the cube with a geometry attached to hand_joint[0] or hand_joint[1] (that contact is what bit 1
+ *      judges: the cube sits about a millimetre from the finger faces), plus the cube's own pairs with the table and
+ *      the obstacle (gik_cube_collision_*) when the scene does not list them.
+ * Outputs per trajectory: valid [n_traj] u8 = no sample has a bit set; first_bad [n_traj] i32 = the first sample with
+ * a bit set, -1 if none; reason [n_traj] u8 = the bits of that sample (0 if none); grasp_err [n_traj] = max of g over
+ * all samples (+inf where g is NaN).  sample_flags [n_traj][n_samples] u8 (may be NULL = not written): every sample's
+ * bits.  Every output is a min / max reduction: independent of the launch configuration, identical between runs.
+ * Errors: GIK_E_SIZE (n_traj < 0, n_ctrl < 2, n_samples < 2 or > 2^28 - 1), GIK_E_PARAM (a negative or NaN
+ * tolerance), GIK_E_NULL (a required pointer is NULL and n_traj > 0), GIK_E_HANDLE, GIK_E_NOSCENE; n_traj = 0 is a
+ * no-op. */
+int gik_traj_check_f32(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_samples, const float* weights,
+                       const float* ctrl, double limit_tol, double grasp_tol, uint8_t* valid, int32_t* first_bad,
+                       uint8_t* reason, float* grasp_err, uint8_t* sample_flags, void* stream);
+int gik_traj_check_f64(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_samples, const double* weights,
+                       const double* ctrl, double limit_tol, double grasp_tol, uint8_t* valid, int32_t* first_bad,
+                       uint8_t* reason, double* grasp_err, uint8_t* sample_flags, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -13,7 +13,8 @@ from .inverse_geometry import apply_collision, computeqgrasppose, computeqgraspp
 from .path import (computepath, edge_num_steps, project_edges_batch, project_path, sample_cube_placements,  # noqa: F401
                    sample_grasp_poses_batch, se3_interpolate)
 from .planner import computepath_batch                                                # noqa: F401
-from .trajectory import Bezier, maketraj, maketraj_batch                                        # noqa: F401
+from .trajectory import (Bezier, check_trajectories_batch, check_trajectory, maketraj, maketraj_batch,  # noqa: F401
+                         maketraj_paths)
 from . import tools                                                                   # noqa: F401
 from . import experiments                                                             # noqa: F401
 from . import dist                                                                     # noqa: F401

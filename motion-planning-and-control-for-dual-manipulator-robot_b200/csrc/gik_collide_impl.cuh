@@ -495,11 +495,17 @@ gik_tail_kernel(const __grid_constant__ DevTable<T> tab, const DevScene<T>* __re
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
+namespace gik {
+constexpr int kTrajPairCap = GIK_MAX_PAIRS + 2;   // list 3: at most list 0 plus the cube's two own pairs
+}
+
 struct gik_scene_dev {
   gik::DevScene<float>* sc32 = nullptr;
   gik::DevScene<double>* sc64 = nullptr;
-  uint8_t* pairs = nullptr;   // [3 lists][2][GIK_MAX_PAIRS]: all pairs | table/obstacle pairs | cube vs table, obstacle
-  int n_list[3] = {0, 0, 0};
+  // [3 lists][2][GIK_MAX_PAIRS]: all pairs | table/obstacle pairs | cube vs table, obstacle; then list 3 as
+  // [2][kTrajPairCap]: the trajectory check's pairs (gik_traj.cuh)
+  uint8_t* pairs = nullptr;
+  int n_list[4] = {0, 0, 0, 0};
 };
 
 namespace {
@@ -673,7 +679,8 @@ int gik_scene_attach(gik_handle_t h, const gik_scene_t* scene) {
   if (!sd) return (int)cudaErrorMemoryAllocation;
   gik::DevScene<float>* h32 = new (std::nothrow) gik::DevScene<float>();
   gik::DevScene<double>* h64 = new (std::nothrow) gik::DevScene<double>();
-  uint8_t* hp = new (std::nothrow) uint8_t[3 * 2 * GIK_MAX_PAIRS]();
+  const size_t pair_bytes = (size_t)6 * GIK_MAX_PAIRS + 2 * gik::kTrajPairCap;
+  uint8_t* hp = new (std::nothrow) uint8_t[pair_bytes]();
   cudaError_t e = (h32 && h64 && hp) ? cudaSuccess : cudaErrorMemoryAllocation;
   if (e == cudaSuccess) {
     gik::fill_dev_scene(h->host, *scene, *h32);
@@ -690,12 +697,32 @@ int gik_scene_attach(gik_handle_t h, const gik_scene_t* scene) {
       if (env[k] >= 0 && scene->cube_geom >= 0) {
         hp[4 * GIK_MAX_PAIRS + sd->n_list[2]] = (uint8_t)env[k]; hp[5 * GIK_MAX_PAIRS + sd->n_list[2]++] = (uint8_t)scene->cube_geom;
       }
+    // list 3 (gik_traj_check_*): list 0 without the pairs of the cube with a geometry on either hand joint -- the grasp
+    // error judges that contact, GJK would only measure the millimetre between the fingers and the cube -- plus the
+    // pairs of list 2 that list 0 lacks
+    uint8_t* l3a = hp + 6 * GIK_MAX_PAIRS;
+    uint8_t* l3b = l3a + gik::kTrajPairCap;
+    auto on_hand = [&](int g) {
+      return scene->geoms[g].joint == h->host.hand_joint[0] || scene->geoms[g].joint == h->host.hand_joint[1];
+    };
+    for (int k = 0; k < sd->n_list[0]; ++k) {
+      const int a = hp[k], b = hp[GIK_MAX_PAIRS + k];
+      if ((a == scene->cube_geom && on_hand(b)) || (b == scene->cube_geom && on_hand(a))) continue;
+      l3a[sd->n_list[3]] = (uint8_t)a; l3b[sd->n_list[3]++] = (uint8_t)b;
+    }
+    for (int k = 0; k < sd->n_list[2]; ++k) {
+      const int a = hp[4 * GIK_MAX_PAIRS + k], b = hp[5 * GIK_MAX_PAIRS + k];
+      bool listed = false;
+      for (int j = 0; j < sd->n_list[3] && !listed; ++j)
+        listed = (l3a[j] == a && l3b[j] == b) || (l3a[j] == b && l3b[j] == a);
+      if (!listed) { l3a[sd->n_list[3]] = (uint8_t)a; l3b[sd->n_list[3]++] = (uint8_t)b; }
+    }
     if ((e = cudaMalloc(&sd->sc32, sizeof(*h32))) == cudaSuccess &&
         (e = cudaMalloc(&sd->sc64, sizeof(*h64))) == cudaSuccess &&
-        (e = cudaMalloc(&sd->pairs, 3 * 2 * GIK_MAX_PAIRS)) == cudaSuccess &&
+        (e = cudaMalloc(&sd->pairs, pair_bytes)) == cudaSuccess &&
         (e = cudaMemcpy(sd->sc32, h32, sizeof(*h32), cudaMemcpyHostToDevice)) == cudaSuccess &&
         (e = cudaMemcpy(sd->sc64, h64, sizeof(*h64), cudaMemcpyHostToDevice)) == cudaSuccess)
-      e = cudaMemcpy(sd->pairs, hp, 3 * 2 * GIK_MAX_PAIRS, cudaMemcpyHostToDevice);
+      e = cudaMemcpy(sd->pairs, hp, pair_bytes, cudaMemcpyHostToDevice);
   }
   delete h32; delete h64; delete[] hp;
   if (e != cudaSuccess) { free_scene(sd); return (int)e; }

@@ -352,6 +352,34 @@ class GraspIK:
             self.launches += 1
         return ctrl, cost
 
+    def check_trajectories(self, ctrl: torch.Tensor, weights, *, limit_tol: float, grasp_tol: float, per_sample=False):
+        """Validity of many Bezier trajectories at the sample times of `weights` (gik_traj_check_*, semantics in
+        include/gik.h): joint limits, grasp error between the cube placements the two hands imply, collisions with the
+        carried cube at the left hand's placement.  ctrl [N, n_ctrl, nq] on this device; weights [M, n_ctrl]: Bernstein
+        weights of the samples (trajectory.sample_weights).  -> (valid u8 [N], first_bad i32 [N] (-1 = none), reason u8
+        [N] (flags of the first bad sample: 1 limits | 2 grasp | 4 collision), grasp_err [N] (max over the samples),
+        sample_flags u8 [N, M] or None)."""
+        self._need_scene()
+        self._chk_dev(ctrl)
+        dt = ctrl.dtype
+        N, n_ctrl, nq = ctrl.shape
+        W = torch.as_tensor(weights, dtype=dt, device=self.device).contiguous()
+        if nq != self.nq or W.dim() != 2 or W.shape[1] != n_ctrl:
+            raise ValueError(f"check_trajectories: expected ctrl [N, n_ctrl, {self.nq}] and weights [M, n_ctrl]")
+        M = W.shape[0]
+        valid = torch.empty((N,), dtype=torch.uint8, device=self.device)
+        first_bad = torch.empty((N,), dtype=torch.int32, device=self.device)
+        reason = torch.empty((N,), dtype=torch.uint8, device=self.device)
+        grasp_err = torch.empty((N,), dtype=dt, device=self.device)
+        flags = torch.empty((N, M), dtype=torch.uint8, device=self.device) if per_sample else None
+        f = getattr(self._lib, f"gik_traj_check_{_sfx(dt)}")
+        _cabi.check(f(self._h, N, n_ctrl, M, self._ptr(W), self._ptr(ctrl.contiguous()), float(limit_tol),
+                      float(grasp_tol), self._ptr(valid), self._ptr(first_bad), self._ptr(reason), self._ptr(grasp_err),
+                      self._ptr(flags), self._stream()), "gik_traj_check")
+        if N:
+            self.launches += 3
+        return valid, first_bad, reason, grasp_err, flags
+
     # ------------------------------------------------------------------ RRT-connect trees on the device (csrc/gik_tree.cuh)
     # verts [n_trees][nq][cap], cubes [n_trees][12][cap], parent i32 [n_trees][cap], n_verts i32 [n_trees]
     def _chk_tree(self, verts, n_verts, cubes=None, parent=None):

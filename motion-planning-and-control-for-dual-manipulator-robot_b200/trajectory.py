@@ -124,6 +124,76 @@ def maketraj_batch(q0, q1, path_points, degree=DEGREE, solver=None):
     return torch.cat([rep0, Pf, rep1], dim=-2), cost
 
 
+def maketraj_paths(q0, q1, q, offsets, degree=DEGREE, solver=None):
+    """Fit CSR-packed paths, e.g. computepath_batch's (q [total, nq], offsets [Q+1]): path i is
+    q[offsets[i]:offsets[i+1]].  q0, q1 [Q, nq].  One host read of `offsets`, then one maketraj_batch per distinct path
+    length (one gik_bezier_fit_* launch for CUDA tensors).  -> (control points [Q, degree+1, nq], cost [Q]); a query
+    without a path gets NaN control points and cost +inf."""
+    import torch
+    off = offsets.cpu().numpy() if torch.is_tensor(offsets) else np.asarray(offsets)
+    Q, nq = len(off) - 1, q.shape[-1]
+    lens = np.diff(off)
+    ctrl = torch.full((Q, degree + 1, nq), float("nan"), dtype=q.dtype, device=q.device)
+    cost = torch.full((Q,), float("inf"), dtype=q.dtype, device=q.device)
+    for n in np.unique(lens[lens > 0]):
+        rows = np.nonzero(lens == n)[0]
+        idx = torch.as_tensor(off[rows][:, None] + np.arange(n)[None, :], device=q.device)
+        r = torch.as_tensor(rows, device=q.device)
+        c, k = maketraj_batch(q0[r], q1[r], q[idx], degree, solver)
+        ctrl[r], cost[r] = c, k
+    return ctrl, cost
+
+
+CHECK_SAMPLES = 1501     # the controller's 1500 steps of 0.01 s over T = 15 s (control.py:416-463), plus the end point
+GRASP_TOL = 1e-2         # policy default, not derived from the controller: see DESIGN.md "Trajectory check"
+LIMIT_TOL = 1e-6         # rad: round-off of the weights on a curve that lies on a joint limit
+
+
+def sample_weights(n_ctrl: int, n_samples: int) -> np.ndarray:
+    """Bernstein weights [n_samples, n_ctrl] (fp64) of the parameters u_k = k / (n_samples - 1)."""
+    return bernstein_matrix(n_ctrl - 1, np.arange(n_samples) / (n_samples - 1))
+
+
+def check_trajectories_batch(ctrl, *, n_samples=CHECK_SAMPLES, grasp_tol=GRASP_TOL, limit_tol=LIMIT_TOL, per_sample=False,
+                             solver=None):
+    """Can these fitted trajectories be executed?  ctrl [N, n_ctrl, nq] Bezier control points (maketraj_batch /
+    maketraj_paths), checked at u_k = k / (n_samples - 1) in one gik_traj_check_* call (semantics in include/gik.h):
+    joint limits (flag 1), grasp error between the cube placements the two hands imply (flag 2), collisions with the
+    carried cube at the left hand's placement (flag 4).  `solver`: a GraspIK (default: the built-in Nextage solver on
+    ctrl's CUDA device, or the current one); ctrl is moved to its device.  -> dict of tensors on that device: valid
+    bool [N], first_bad int32 [N] (-1 = none), reason uint8 [N] (flags of the first bad sample), grasp_err [N] (max over
+    the samples) and, with per_sample, sample_flags uint8 [N, n_samples]."""
+    import torch
+    from .ops import default_solver
+    ctrl = torch.as_tensor(ctrl)
+    s = solver if solver is not None else default_solver(ctrl.device if ctrl.is_cuda else None)
+    ctrl = ctrl.to(s.device)
+    W = sample_weights(ctrl.shape[-2], int(n_samples))
+    valid, first_bad, reason, grasp_err, flags = s.check_trajectories(ctrl, W, limit_tol=limit_tol, grasp_tol=grasp_tol,
+                                                                       per_sample=per_sample)
+    out = {"valid": valid.bool(), "first_bad": first_bad, "reason": reason, "grasp_err": grasp_err}
+    if per_sample:
+        out["sample_flags"] = flags
+    return out
+
+
+def check_trajectory(q_of_t, *, n_samples=CHECK_SAMPLES, grasp_tol=GRASP_TOL, limit_tol=LIMIT_TOL, per_sample=False,
+                     solver=None, dtype=None):
+    """check_trajectories_batch for one reference-style Bezier (maketraj's q_of_t): sampled at n_samples evenly spaced
+    times over [t_min, t_max].  -> dict with valid (bool), first_bad (int), reason (int), grasp_err (float) and, with
+    per_sample, sample_flags (uint8 tensor [n_samples])."""
+    import torch
+    P = np.array(q_of_t.control_points_, dtype=float) * q_of_t.mult_T_
+    ctrl = torch.as_tensor(P[None], dtype=dtype if dtype is not None else torch.float64)
+    r = check_trajectories_batch(ctrl, n_samples=n_samples, grasp_tol=grasp_tol, limit_tol=limit_tol,
+                                 per_sample=per_sample, solver=solver)
+    out = {"valid": bool(r["valid"][0]), "first_bad": int(r["first_bad"][0]), "reason": int(r["reason"][0]),
+           "grasp_err": float(r["grasp_err"][0])}
+    if per_sample:
+        out["sample_flags"] = r["sample_flags"][0]
+    return out
+
+
 def save_trajectory_to_json(filename, q_of_t, vq_of_t, vvq_of_t):
     """control.save_trajectory_to_json (control.py:203-216), same file format."""
     data = {"q_control_points": [p.tolist() for p in q_of_t.control_points_],
