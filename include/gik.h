@@ -368,6 +368,37 @@ int gik_tree_paths_f64(gik_handle_t h, int64_t n_queries, int32_t cap, const dou
                        const int32_t* parent, const int32_t* n_verts, const int32_t* start_end, const int32_t* goal_end,
                        int64_t* offsets, double* q, double* cube, void* stream);
 
+/* Shortcutting of planned paths, one round for n_paths paths (what gik_tree_paths_* returns: CSR rows offsets
+ * [n_paths + 1] int64, q [total][nq], cube [total][12], row-major).  Path p has n = offsets[p+1] - offsets[p] rows and
+ * K = n_cand candidates; candidate k is edge e = p * K + k of one gik_project_edges_* launch of E = n_paths * K edges
+ * (max_steps, q_path [max_steps][nq][E]) from (q_i, cube_i) towards cube_j, (i, j) = (pair_i[e], pair_j[e]), with
+ * num_steps[e] = ns steps and n_valid[e] = nv its converged, collision-free steps.  Let s_m be the q of step m and
+ * ||.|| the fp64 norm of the fp64 difference, squares summed left to right.  Candidate k is accepted when
+ *   0 <= i, i + 2 <= j <= n - 1, 1 <= ns <= max_steps, nv == ns, ||s_ns - q_j|| < join_tol, and
+ *   gain = L_old - L_new > 0, where L_old = sum_{k=i}^{j-1} ||q_{k+1} - q_k|| and
+ *   L_new = ||s_1 - q_i|| + sum_{m=1}^{ns-2} ||s_{m+1} - s_m|| + ||q_j - s_{ns-1}||  (ns = 1: ||q_j - q_i||),
+ * every sum in fp64, left to right, without contraction.  Of the accepted candidates the one with the largest gain is
+ * chosen, ties to the lowest k; chosen[p] = k, or -1.  The chosen candidate replaces rows i+1 .. j-1 with steps
+ * 1 .. ns-1 (s_ns is dropped, q_j kept); the placement stored with step m is cube_i * exp6((m / ns) xi),
+ * xi = log6(cube_i^-1 cube_j): the placement the edge kernel solved it for.  length[p] = joint-space length of the
+ * output path (sum of ||q_{r+1} - q_r|| over its rows, left to right).  K <= 32; K = 0 computes lengths only.
+ * Two calls: with q_out = cube_out = NULL, chosen, length and offsets_out [n_paths + 1] are written (offsets_out[n_paths]
+ * = the new total, the one value the caller reads back to size q_out / cube_out); then, with q_out and cube_out, the
+ * rows are written at offsets_out.
+ * Errors: GIK_E_SIZE (n_paths < 0, n_cand < 0 or > 32, max_steps < 0), GIK_E_PARAM (join_tol negative or NaN),
+ * GIK_E_NULL (a required pointer is NULL and n_paths > 0; the candidate arrays are required when n_cand > 0, q_path
+ * when also max_steps > 0; q_out without cube_out or the reverse), GIK_E_HANDLE; n_paths = 0 is a no-op. */
+int gik_path_shortcut_f32(gik_handle_t h, int64_t n_paths, int32_t n_cand, int32_t max_steps, const int64_t* offsets,
+                          const float* q, const float* cube, const int32_t* pair_i, const int32_t* pair_j,
+                          const int32_t* num_steps, const int32_t* n_valid, const float* q_path, double join_tol,
+                          int32_t* chosen, double* length, int64_t* offsets_out, float* q_out, float* cube_out,
+                          void* stream);
+int gik_path_shortcut_f64(gik_handle_t h, int64_t n_paths, int32_t n_cand, int32_t max_steps, const int64_t* offsets,
+                          const double* q, const double* cube, const int32_t* pair_i, const int32_t* pair_j,
+                          const int32_t* num_steps, const int32_t* n_valid, const double* q_path, double join_tol,
+                          int32_t* chosen, double* length, int64_t* offsets_out, double* q_out, double* cube_out,
+                          void* stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * Trajectory check: can a fitted trajectory be executed?  The reference finds out only by running its 1500 pybullet
  * control steps (control.py:416-463): between the path vertices the least-squares curve lies on no grasp manifold, and

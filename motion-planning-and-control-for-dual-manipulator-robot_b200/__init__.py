@@ -12,7 +12,7 @@ from .ops import (DT, EPSILON, MAX_ITERS, GraspIK, SolveInfo, as_pose12, bytes_p
 from .inverse_geometry import apply_collision, computeqgrasppose, computeqgrasppose_batch, solver_for  # noqa: F401
 from .path import (computepath, edge_num_steps, project_edges_batch, project_path, sample_cube_placements,  # noqa: F401
                    sample_grasp_poses_batch, se3_interpolate)
-from .planner import computepath_batch                                                # noqa: F401
+from .planner import computepath_batch, shortcut_paths_batch                          # noqa: F401
 from .trajectory import (Bezier, check_trajectories_batch, check_trajectory, maketraj, maketraj_batch,  # noqa: F401
                          maketraj_paths)
 from . import tools                                                                   # noqa: F401

@@ -32,7 +32,7 @@ class GikError(RuntimeError):
 def _sources():
     return [os.path.join(CSRC, f) for f in ("gik_kernels.cu", "gik_core.cuh", "gik_table.h", "gik_collide.cuh",
                                             "gik_collide_impl.cuh", "gik_bezier.cuh", "gik_tree.cuh",
-                                            "gik_traj.cuh")] + \
+                                            "gik_shortcut.cuh", "gik_traj.cuh")] + \
            [os.path.join(_HERE, "..", "include", "gik.h")]
 
 
@@ -103,6 +103,7 @@ def lib() -> ctypes.CDLL:
         getattr(L, f"gik_tree_nearest_{sfx}").argtypes = [_P, _I64, _I32, _P, _P, _I64, _P, _P, _P, _P]
         getattr(L, f"gik_tree_grow_{sfx}").argtypes = [_P, _I64, _I32, _P, _P, _P, _P, _P, _I64, _I32] + [_P] * 10
         getattr(L, f"gik_tree_paths_{sfx}").argtypes = [_P, _I64, _I32] + [_P] * 10
+        getattr(L, f"gik_path_shortcut_{sfx}").argtypes = [_P, _I64, _I32, _I32] + [_P] * 8 + [ctypes.c_double] + [_P] * 6
         getattr(L, f"gik_traj_check_{sfx}").argtypes = [_P, _I64, _I32, _I32, _P, _P, ctypes.c_double, ctypes.c_double] + [_P] * 6
     L.gik_solve_success_scratch_bytes.argtypes = [_P, _I64, ctypes.c_int]
     L.gik_solve_success_scratch_bytes.restype = ctypes.c_size_t
@@ -128,7 +129,7 @@ EXPORTS = [
     "gik_cube_collision_f32", "gik_cube_collision_f64", "gik_obstacle_distance_f32", "gik_obstacle_distance_f64",
     "gik_bezier_fit_f32", "gik_bezier_fit_f64",
     "gik_tree_nearest_f32", "gik_tree_nearest_f64", "gik_tree_grow_f32", "gik_tree_grow_f64",
-    "gik_tree_paths_f32", "gik_tree_paths_f64", "gik_traj_check_f32", "gik_traj_check_f64",
+    "gik_tree_paths_f32", "gik_tree_paths_f64", "gik_path_shortcut_f32", "gik_path_shortcut_f64", "gik_traj_check_f32", "gik_traj_check_f64",
     "gik_flops_per_iter", "gik_flops_per_iter_executed", "gik_bytes_per_solve", "gik_measure_fma_peak", "gik_solve_launch_dims",
     "gik_solve_kernel_name",
     "gik_strerror", "gik_version",

@@ -1689,5 +1689,6 @@ const char* gik_version(void) { return "gik 0.1 (sm_100a)"; }
 #include "gik_collide_impl.cuh"
 #include "gik_bezier.cuh"
 #include "gik_tree.cuh"
+#include "gik_shortcut.cuh"
 #include "gik_traj.cuh"
 static void gik_free_scene_of(gik_handle_s* h) { free_scene(h->scene); h->scene = nullptr; }

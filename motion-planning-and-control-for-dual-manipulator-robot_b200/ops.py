@@ -469,6 +469,41 @@ class GraspIK:
             self.launches += 3 if total else 2
         return q, cube, offsets
 
+    def path_shortcut(self, q, cube, offsets, pair_i, pair_j, num_steps, n_valid, q_path, *, join_tol: float):
+        """One shortcut round for CSR paths (gik_path_shortcut_*, semantics in include/gik.h): q [total][nq], cube
+        [total][12], offsets int64 [Q+1] (tree_paths' form); candidate k of path p is edge p * K + k of one
+        project_edges_soa launch: pair_i / pair_j / num_steps / n_valid int32 [Q, K] and q_path [S][nq][Q*K].
+        -> (q [total'][nq], cube [total'][12], offsets int64 [Q+1], chosen int32 [Q] (-1 = none), length float64 [Q]
+        (joint-space length of each output path)).  One host synchronisation (reading the new total)."""
+        self._chk_dev(q, cube, offsets, pair_i, pair_j, num_steps, n_valid, q_path)
+        dt = q.dtype
+        Q = offsets.shape[0] - 1
+        K = pair_i.shape[1] if pair_i.dim() == 2 else -1
+        S = q_path.shape[0]
+        if Q < 0 or offsets.dtype != torch.int64 or q.shape[1:] != (self.nq,) or cube.shape != (q.shape[0], 12) or \
+                any(t.shape != (Q, K) for t in (pair_i, pair_j, num_steps, n_valid)) or q_path.shape != (S, self.nq, Q * K):
+            raise ValueError("path_shortcut: expected q [total][nq], cube [total][12], offsets int64 [Q+1], candidate "
+                             "arrays [Q, K] and q_path [S][nq][Q*K]")
+        if cube.dtype != dt or q_path.dtype != dt or any(t.dtype != torch.int32 for t in (pair_i, pair_j, num_steps, n_valid)):
+            raise TypeError("path_shortcut: float arrays must share q's dtype, candidate arrays must be int32")
+        args = [x.contiguous() for x in (offsets, q, cube, pair_i, pair_j, num_steps, n_valid, q_path)]
+        chosen = torch.empty((Q,), dtype=torch.int32, device=self.device)
+        length = torch.empty((Q,), dtype=torch.float64, device=self.device)
+        off_out = torch.empty((Q + 1,), dtype=torch.int64, device=self.device)
+        f = getattr(self._lib, f"gik_path_shortcut_{_sfx(dt)}")
+        head = [self._ptr(x) for x in args]
+        tail = [self._ptr(chosen), self._ptr(length), self._ptr(off_out)]
+        _cabi.check(f(self._h, Q, K, S, *head, float(join_tol), *tail, None, None, self._stream()), "gik_path_shortcut")
+        total = int(off_out[-1].item()) if Q else 0
+        q_out = torch.empty((total, self.nq), dtype=dt, device=self.device)
+        cube_out = torch.empty((total, 12), dtype=dt, device=self.device)
+        if total:
+            _cabi.check(f(self._h, Q, K, S, *head, float(join_tol), *tail, self._ptr(q_out), self._ptr(cube_out),
+                          self._stream()), "gik_path_shortcut")
+        if Q:
+            self.launches += 3 if total else 2
+        return q_out, cube_out, off_out, chosen, length
+
     def cube_collision_soa(self, cube_pose_soa: torch.Tensor) -> torch.Tensor:
         """The cube's own collision test (cube vs table / obstacle, path.py:51-52): cube_pose [12][n] -> u8 [n]."""
         self._need_scene()

@@ -159,3 +159,85 @@ def computepath_batch(qinit, qgoal, cube0, cube1, robot=None, cube=None, *, step
     stats["retries"] = retry
     q, cube_rows, offsets = solver.tree_paths(verts, cubes, parent, n_verts, start_end, goal_end)
     return q, cube_rows, offsets, stats
+
+
+# ------------------------------------------------------------------------------------------------ path shortcutting
+SHORTCUT_ROUNDS = 16        # defaults chosen from the length-per-round curve of tools/bench_shortcut.py: DESIGN.md
+SHORTCUT_CANDIDATES = 16    # "Path shortcutting"
+
+
+def _draw_pairs(n, K, generator):
+    """K candidate pairs per path: n int64 [Q] path lengths -> (i, j) int32 [Q, K], uniform over the pairs with
+    0 <= i and i + 2 <= j <= n - 1 (two distinct slots x != y of n - 1, i = min, j = max + 1); -1 for a path with fewer
+    than 3 vertices.  Drawn on n's device from `generator`."""
+    Q, dev = n.shape[0], n.device
+    u = torch.rand((Q, K, 2), dtype=torch.float64, device=dev, generator=generator)
+    m = (n - 1).clamp_min(2)[:, None]
+    x = torch.minimum((u[..., 0] * m).long(), m - 1)                                # [0, n-1)
+    y = torch.minimum((u[..., 1] * (m - 1)).long(), m - 2)                          # [0, n-2)
+    y = y + (y >= x).long()
+    i, j = torch.minimum(x, y), torch.maximum(x, y) + 1
+    ok = (n >= 3)[:, None]
+    return torch.where(ok, i, -1).to(torch.int32), torch.where(ok, j, -1).to(torch.int32)
+
+
+def shortcut_paths_batch(q, cube, offsets, robot=None, *, rounds=SHORTCUT_ROUNDS, candidates=SHORTCUT_CANDIDATES,
+                         step_size=STEP_SIZE, join_tol=GOAL_TOLERANCE, generator=None):
+    """Shortcut CSR paths as computepath_batch returns them: q [total, nq], cube [total, 12], offsets int64 [Q+1].
+
+    Each round draws `candidates` (K <= 32) pairs (i, j), j >= i + 2, per path of at least 3 vertices (_draw_pairs),
+    marches each as one edge from (q_i, cube_i) towards cube_j in _num_steps(cube_i, cube_j) steps (all Q·K edges in
+    one edge launch, cut at the first collision), and accepts a candidate when every step converged collision-free,
+    the last step lands within join_tol of q_j and the joint-space length strictly drops.  Per path the accepted
+    candidate with the largest gain (ties: the lowest index) replaces vertices i+1 .. j-1 with the edge's steps but
+    the last, each stored with the placement it was solved for (gik_path_shortcut_*, semantics in include/gik.h).
+    The end rows of every path are kept bit for bit; lengths never increase; no cube move above step_size is added.
+
+    Returns (q, cube, offsets, stats) in the same form; stats holds shortcuts int32 [Q] (splices accepted) and
+    length float64 [Q] (joint-space length after the last round).  Host synchronisations: one before the loop (the
+    step bound S, from the largest cube-translation bounding-box diagonal of a path) and one per round (the new row
+    count).  A candidate needing more than S steps (possible only when a path rotates the cube) is dropped: it
+    marches no step."""
+    solver = solver_for(robot, None)
+    solver._need_scene()
+    dev = solver.device
+    q = torch.as_tensor(q, device=dev)
+    cube = torch.as_tensor(cube, device=dev).to(q.dtype)
+    offsets = torch.as_tensor(offsets, device=dev).to(torch.int64)
+    K = int(candidates)
+    if not 0 <= K <= 32:
+        raise ValueError("shortcut_paths_batch: candidates must be in [0, 32]")
+    Q, total = offsets.shape[0] - 1, q.shape[0]
+    stats = {"shortcuts": torch.zeros(Q, dtype=torch.int32, device=dev),
+             "length": torch.zeros(Q, dtype=torch.float64, device=dev)}
+    if Q == 0 or total == 0:
+        return q, cube, offsets, stats
+    # step bound: the largest bounding-box diagonal of a path's cube translations (the one read before the loop)
+    pid = torch.searchsorted(offsets[1:], torch.arange(total, device=dev), right=True)[:, None].expand(total, 3)
+    p = cube[:, 9:].double()
+    lo = torch.zeros((Q, 3), dtype=torch.float64, device=dev).scatter_reduce(0, pid, p, "amin", include_self=False)
+    hi = torch.zeros((Q, 3), dtype=torch.float64, device=dev).scatter_reduce(0, pid, p, "amax", include_self=False)
+    S = int(torch.linalg.vector_norm(hi - lo, dim=1).max().item() * (1 + 1e-6) / step_size) + 1
+    i32 = dict(dtype=torch.int32, device=dev)
+    if rounds <= 0 or K == 0:                               # lengths only
+        none = torch.zeros((Q, 0), **i32)
+        q, cube, offsets, _, stats["length"] = solver.path_shortcut(
+            q, cube, offsets, none, none, none, none, torch.zeros((0, solver.nq, 0), dtype=q.dtype, device=dev),
+            join_tol=join_tol)
+        return q, cube, offsets, stats
+    for _ in range(int(rounds)):
+        n = offsets[1:] - offsets[:-1]
+        pi, pj = _draw_pairs(n, K, generator)
+        has = (pi >= 0).reshape(-1)
+        last = q.shape[0] - 1
+        ri = (offsets[:-1, None] + pi.long()).clamp(0, last).reshape(-1)
+        rj = (offsets[:-1, None] + pj.long()).clamp(0, last).reshape(-1)
+        ca, cb = cube[ri], cube[rj]
+        ns = _num_steps(ca, cb, step_size)
+        ns = torch.where(has & (ns <= S), ns, 0)
+        path, nv, _ = solver.project_edges_soa(q[ri].t().contiguous(), ca.t().contiguous(), cb.t().contiguous(), ns, S)
+        nv = _cut_at_first_collision(solver, path, nv, ca, cb, ns, S, dense=True)
+        q, cube, offsets, chosen, stats["length"] = solver.path_shortcut(
+            q, cube, offsets, pi, pj, ns.reshape(Q, K), nv.reshape(Q, K), path, join_tol=join_tol)
+        stats["shortcuts"] += (chosen >= 0).to(torch.int32)
+    return q, cube, offsets, stats
