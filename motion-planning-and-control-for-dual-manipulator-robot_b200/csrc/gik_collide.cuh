@@ -200,6 +200,28 @@ GIK_HD Shape<T> make_shape(const DevGeom<T>& g, const T* M) {
   return S;
 }
 
+// World placement of geometry g: oMi[joint] * placement (pin.updateGeometryPlacements).  The cube takes the problem's
+// pose cube[k * ld + i], k < 12 (cube = nullptr: the scene's own).  oMi = nullptr (no configuration): every geometry
+// keeps its placement in its joint's frame.
+template <typename T>
+GIK_HD void place_geom(const DevScene<T>* sc, int g, const T* cube, int64_t ld, int64_t i, const T (*oMi)[12], T* out) {
+  const DevGeom<T>& G = sc->g[g];
+  T P[12];
+  if (g == sc->cube_geom && cube) {
+#pragma unroll
+    for (int k = 0; k < 12; ++k) P[k] = cube[k * ld + i];
+  } else {
+#pragma unroll
+    for (int k = 0; k < 9; ++k) P[k] = G.R[k];
+    P[9] = G.p[0]; P[10] = G.p[1]; P[11] = G.p[2];
+  }
+  if (G.joint >= 0 && oMi) se3_mul12(&oMi[G.joint][0], P, out);
+  else {
+#pragma unroll
+    for (int k = 0; k < 12; ++k) out[k] = P[k];
+  }
+}
+
 // The shape ERODED by `shrink` (the points whose shrink-ball lies inside it): box -> smaller box, sphere -> smaller
 // sphere, cylinder -> thinner and shorter cylinder.  Returns false when nothing is left.
 template <typename T>

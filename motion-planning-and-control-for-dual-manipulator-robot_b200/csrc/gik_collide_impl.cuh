@@ -1,9 +1,10 @@
 // gik_collide_impl.cuh -- collision kernels + their C ABI (included at the end of gik_kernels.cu: one translation
-// unit, one library).  Mapping: ONE CONFIGURATION PER WARP.  The kinematic tree is walked level by level (one joint per lane),
-// the lanes place the geometries (oMg = oMi[parent] * placement, pin.updateGeometryPlacements), then the collision
-// pairs are dealt round-robin to the 32 lanes for the bounding-sphere test, the survivors are compacted into a per-warp
-// list and boolean GJK runs on full warps of candidates, with one __any_sync per round for the early exit.  The scene (geometries, pair lists) lives in global memory and is read
-// through the read-only path; per-configuration traffic is q in (60 B) and one flag out.
+// unit, one library).  Mapping: ONE CONFIGURATION PER WARP.  The kinematic tree is walked level by level (one joint per
+// lane, warp_tree_fk), the lanes place the geometries (place_geom, gik_collide.cuh), then the collision pairs are dealt
+// round-robin to the 32 lanes for the bounding-sphere test, the survivors are compacted into a per-warp list and boolean
+// GJK runs on full warps of candidates, with one __any_sync per round for the early exit (warp_any_pair_hits, shared
+// with the trajectory check).  The scene (geometries, pair lists) lives in global memory and is read through the
+// read-only path; per-configuration traffic is q in (60 B) and one flag out.
 #pragma once
 #include "gik_collide.cuh"
 
@@ -11,6 +12,72 @@ namespace gik {
 
 constexpr int kCollideWarps = 4;
 constexpr int kMaxCand = 512;       // per-configuration candidate pairs kept for the narrow phase
+
+// tree FK of one configuration by one warp (level by level, one joint per lane) into oMi[nq][12]; q_of(j) = q_j.
+// Lane j first builds its joint's local transform jointPlacement * Rot(axis, q_j), then the joints of depth d (all
+// independent) are composed with their parents' world placements of depth d - 1.
+template <typename T, typename QF>
+__device__ __forceinline__ void warp_tree_fk(const DevScene<T>* sc, int lane, QF q_of, T (*oMi)[12]) {
+  const int nq = sc->tree.nq;
+  T L[12];
+  int par = -1, dep = -1;
+  if (lane < nq) {
+    joint_placement(sc->tree, lane, (const T*)nullptr, q_of(lane), L);
+    par = sc->tree.parent[lane]; dep = sc->tree.depth[lane];
+  }
+  for (int d = 0; d <= sc->tree.max_depth; ++d) {
+    if (dep == d) {
+      if (par < 0) {
+#pragma unroll
+        for (int k = 0; k < 12; ++k) oMi[lane][k] = L[k];
+      } else {
+        se3_mul12(&oMi[par][0], L, &oMi[lane][0]);
+      }
+    }
+    __syncwarp();
+  }
+}
+
+// Does some pair (pa[k], pb[k]), k < n_pairs, intersect with its first shape inflated by `margin`?  Warp-uniform.
+// oMg: the warp's geometry placements; cand: the warp's kMaxCand-entry candidate list.  The broad phase runs over all
+// pairs first (bounding spheres), compacting the survivors, so that the narrow phase (GJK, a few hundred instructions,
+// data dependent) runs on FULL warps of candidates instead of on the one or two lanes of each 32-pair round that happen
+// to survive.
+template <typename T>
+__device__ __forceinline__ bool warp_any_pair_hits(const DevScene<T>* sc, const uint8_t* pa, const uint8_t* pb, int n_pairs,
+                                                   const T (*oMg)[12], uint16_t* cand, T margin, int lane) {
+  bool hit = false;
+  int n_cand = 0;
+  for (int k0 = 0; k0 < n_pairs && !hit; k0 += 32) {
+    const int k = k0 + lane;
+    bool pass = false;
+    if (k < n_pairs) {
+      const int a = pa[k], b = pb[k];
+      const T dx = oMg[a][9] - oMg[b][9], dy = oMg[a][10] - oMg[b][10], dz = oMg[a][11] - oMg[b][11];
+      const T reach = sc->g[a].bound + sc->g[b].bound + margin;
+      pass = dx * dx + dy * dy + dz * dz <= reach * reach;
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, pass);
+    if (n_cand + __popc(m) > kMaxCand) {
+      // list full (never with the reference scene): test this round's survivors in place
+      if (pass) hit = gjk_intersect(make_shape(sc->g[pa[k]], oMg[pa[k]]), make_shape(sc->g[pb[k]], oMg[pb[k]]), margin);
+      hit = __any_sync(0xffffffffu, hit);
+    } else {
+      if (pass) cand[n_cand + __popc(m & ((1u << lane) - 1u))] = (uint16_t)k;
+      n_cand += __popc(m);
+    }
+  }
+  __syncwarp();
+  for (int c0 = 0; c0 < n_cand && !hit; c0 += 32) {
+    if (c0 + lane < n_cand) {
+      const int k = cand[c0 + lane];
+      const int a = pa[k], b = pb[k];
+      hit = gjk_intersect(make_shape(sc->g[a], oMg[a]), make_shape(sc->g[b], oMg[b]), margin);
+    }
+    hit = __any_sync(0xffffffffu, hit);
+  }
+  return hit;
+}
 
 template <typename T>
 __global__ void __launch_bounds__(kCollideWarps * 32)
@@ -22,86 +89,18 @@ gik_collision_kernel(const DevScene<T>* __restrict__ sc, const uint8_t* __restri
   __shared__ T s_oMg[kCollideWarps][GIK_MAX_GEOMS][12];
   __shared__ uint16_t s_cand[kCollideWarps][kMaxCand];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int nq = sc->tree.nq, ng = sc->n_geoms;
+  const int ng = sc->n_geoms;
   const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   // `sel` (optional): test only the columns sel[0 .. n_sel) of the [.][n] arrays; results go to out[sel[.]]
   const int64_t count = sel ? (n_sel_dev ? *n_sel_dev : n_sel) : n;
   for (int64_t w_i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w_i < count; w_i += warps) {
     const int64_t i = sel ? __ldg(sel + w_i) : w_i;
-    if (q) {
-      // tree FK, level by level: lane j first builds its joint's local transform jointPlacement * Rot(axis, q_j), then
-      // the joints of depth d (all independent) are composed with their parents' world placements of depth d - 1
-      T L[12];
-      int par = -1, dep = -1;
-      if (lane < nq) {
-        joint_placement(sc->tree, lane, (const T*)nullptr, __ldg(q + (int64_t)lane * n + i), L);
-        par = sc->tree.parent[lane]; dep = sc->tree.depth[lane];
-      }
-      for (int d = 0; d <= sc->tree.max_depth; ++d) {
-        if (dep == d) {
-          if (par < 0) {
-#pragma unroll
-            for (int k = 0; k < 12; ++k) s_oMi[w][lane][k] = L[k];
-          } else {
-            se3_mul12(&s_oMi[w][par][0], L, &s_oMi[w][lane][0]);
-          }
-        }
-        __syncwarp();
-      }
-    }
-    for (int g = lane; g < ng; g += 32) {
-      const DevGeom<T>& G = sc->g[g];
-      T P[12];
-      if (g == sc->cube_geom && cube_pose) {
-#pragma unroll
-        for (int k = 0; k < 12; ++k) P[k] = __ldg(cube_pose + (int64_t)k * n + i);
-      } else {
-#pragma unroll
-        for (int k = 0; k < 9; ++k) P[k] = G.R[k];
-        P[9] = G.p[0]; P[10] = G.p[1]; P[11] = G.p[2];
-      }
-      if (G.joint >= 0 && q) se3_mul12(&s_oMi[w][G.joint][0], P, &s_oMg[w][g][0]);
-      else {
-#pragma unroll
-        for (int k = 0; k < 12; ++k) s_oMg[w][g][k] = P[k];
-      }
-    }
+    // q = nullptr (the cube-only test): no FK, the robot's geometries keep their local placements
+    if (q) warp_tree_fk(sc, lane, [&](int j) { return __ldg(q + (int64_t)j * n + i); }, s_oMi[w]);
+    for (int g = lane; g < ng; g += 32)
+      place_geom(sc, g, cube_pose, n, i, q ? s_oMi[w] : nullptr, s_oMg[w][g]);
     __syncwarp();
-    // broad phase over all pairs first (bounding spheres), compacting the survivors into a per-warp list, so that the
-    // narrow phase (GJK, a few hundred instructions, data dependent) runs on FULL warps of candidates instead of on
-    // the one or two lanes of each 32-pair round that happen to survive
-    bool hit = false;
-    int n_cand = 0;
-    for (int k0 = 0; k0 < n_pairs && !hit; k0 += 32) {
-      const int k = k0 + lane;
-      bool pass = false;
-      if (k < n_pairs) {
-        const int a = pa[k], b = pb[k];
-        const T* Ma = &s_oMg[w][a][0];
-        const T* Mb = &s_oMg[w][b][0];
-        const T dx = Ma[9] - Mb[9], dy = Ma[10] - Mb[10], dz = Ma[11] - Mb[11];
-        const T reach = sc->g[a].bound + sc->g[b].bound + margin;
-        pass = dx * dx + dy * dy + dz * dz <= reach * reach;
-      }
-      const unsigned m = __ballot_sync(0xffffffffu, pass);
-      if (n_cand + __popc(m) > kMaxCand) {
-        // list full (never with the reference scene): test this round's survivors in place
-        if (pass) hit = gjk_intersect(make_shape(sc->g[pa[k]], &s_oMg[w][pa[k]][0]), make_shape(sc->g[pb[k]], &s_oMg[w][pb[k]][0]), margin);
-        hit = __any_sync(0xffffffffu, hit);
-      } else {
-        if (pass) s_cand[w][n_cand + __popc(m & ((1u << lane) - 1u))] = (uint16_t)k;
-        n_cand += __popc(m);
-      }
-    }
-    __syncwarp();
-    for (int c0 = 0; c0 < n_cand && !hit; c0 += 32) {
-      if (c0 + lane < n_cand) {
-        const int k = s_cand[w][c0 + lane];
-        const int a = pa[k], b = pb[k];
-        hit = gjk_intersect(make_shape(sc->g[a], &s_oMg[w][a][0]), make_shape(sc->g[b], &s_oMg[w][b][0]), margin);
-      }
-      hit = __any_sync(0xffffffffu, hit);
-    }
+    const bool hit = warp_any_pair_hits(sc, pa, pb, n_pairs, s_oMg[w], s_cand[w], margin, lane);
     if (lane == 0) out[i] = (uint8_t)((hit ? 1 : 0) ^ (invert ? 1 : 0));
     __syncwarp();
   }
@@ -122,45 +121,11 @@ gik_distance_kernel(const DevScene<T>* __restrict__ sc, const uint8_t* __restric
   __shared__ T s_oMi[kCollideWarps][GIK_MAX_NQ][12];
   __shared__ T s_oMg[kCollideWarps][GIK_MAX_GEOMS][12];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int nq = sc->tree.nq, ng = sc->n_geoms;
+  const int ng = sc->n_geoms;
   const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += warps) {
-    {                                               // tree FK level by level, then the geometry placements (as gik_collision_kernel)
-      T L[12];
-      int par = -1, dep = -1;
-      if (lane < nq) {
-        joint_placement(sc->tree, lane, (const T*)nullptr, __ldg(q + (int64_t)lane * n + i), L);
-        par = sc->tree.parent[lane]; dep = sc->tree.depth[lane];
-      }
-      for (int d = 0; d <= sc->tree.max_depth; ++d) {
-        if (dep == d) {
-          if (par < 0) {
-#pragma unroll
-            for (int k = 0; k < 12; ++k) s_oMi[w][lane][k] = L[k];
-          } else {
-            se3_mul12(&s_oMi[w][par][0], L, &s_oMi[w][lane][0]);
-          }
-        }
-        __syncwarp();
-      }
-    }
-    for (int g = lane; g < ng; g += 32) {
-      const DevGeom<T>& G = sc->g[g];
-      T P[12];
-      if (g == sc->cube_geom && cube_pose) {
-#pragma unroll
-        for (int k = 0; k < 12; ++k) P[k] = __ldg(cube_pose + (int64_t)k * n + i);
-      } else {
-#pragma unroll
-        for (int k = 0; k < 9; ++k) P[k] = G.R[k];
-        P[9] = G.p[0]; P[10] = G.p[1]; P[11] = G.p[2];
-      }
-      if (G.joint >= 0) se3_mul12(&s_oMi[w][G.joint][0], P, &s_oMg[w][g][0]);
-      else {
-#pragma unroll
-        for (int k = 0; k < 12; ++k) s_oMg[w][g][k] = P[k];
-      }
-    }
+    warp_tree_fk(sc, lane, [&](int j) { return __ldg(q + (int64_t)j * n + i); }, s_oMi[w]);
+    for (int g = lane; g < ng; g += 32) place_geom(sc, g, cube_pose, n, i, s_oMi[w], s_oMg[w][g]);
     __syncwarp();
     T best = d_max;                                 // running minimum, warp-uniform
     for (int k0 = 0; k0 < n_pairs && best > T(0); k0 += 32) {
@@ -231,48 +196,6 @@ __global__ void __launch_bounds__(256) gik_compact_pending_kernel(int64_t n, con
   }
 }
 
-// tree FK of one configuration by one warp (level by level, one joint per lane) into oMi[nq][12]; q_of(j) = q_j
-template <typename T, typename QF>
-__device__ __forceinline__ void warp_tree_fk(const DevScene<T>* sc, int lane, QF q_of, T (*oMi)[12]) {
-  const int nq = sc->tree.nq;
-  T L[12];
-  int par = -1, dep = -1;
-  if (lane < nq) {
-    joint_placement(sc->tree, lane, (const T*)nullptr, q_of(lane), L);
-    par = sc->tree.parent[lane]; dep = sc->tree.depth[lane];
-  }
-  for (int d = 0; d <= sc->tree.max_depth; ++d) {
-    if (dep == d) {
-      if (par < 0) {
-#pragma unroll
-        for (int k = 0; k < 12; ++k) oMi[lane][k] = L[k];
-      } else {
-        se3_mul12(&oMi[par][0], L, &oMi[lane][0]);
-      }
-    }
-    __syncwarp();
-  }
-}
-
-// world placement of geometry g: oMi[parent] * placement (pin.updateGeometryPlacements); the cube takes the problem's pose
-template <typename T>
-__device__ __forceinline__ void place_geom(const DevScene<T>* sc, int g, const T* cube12, const T (*oMi)[12], T* out) {
-  const DevGeom<T>& G = sc->g[g];
-  T P[12];
-  if (g == sc->cube_geom && cube12) {
-#pragma unroll
-    for (int k = 0; k < 12; ++k) P[k] = cube12[k];
-  } else {
-#pragma unroll
-    for (int k = 0; k < 9; ++k) P[k] = G.R[k];
-    P[9] = G.p[0]; P[10] = G.p[1]; P[11] = G.p[2];
-  }
-  if (G.joint >= 0) se3_mul12(&oMi[G.joint][0], P, out);
-  else {
-#pragma unroll
-    for (int k = 0; k < 12; ++k) out[k] = P[k];
-  }
-}
 
 // ---------------------------------------------------------------------------------------------------------------
 // The reference's keep-descending-while-colliding tail (inverse_geometry.py:70, 97-98), ONE WARP PER PENDING PROBLEM.
@@ -330,7 +253,7 @@ gik_tail_kernel(const __grid_constant__ DevTable<T> tab, const DevScene<T>* __re
 #pragma unroll
     for (int sl = 0; sl < 2; ++sl) {
       const int g = lane + 32 * sl;
-      if (g < ng) place_geom(sc, g, cube, s_oMi[w], Pf[sl]);
+      if (g < ng) place_geom(sc, g, cube, 1, 0, s_oMi[w], Pf[sl]);
     }
     __syncwarp();
     if (lane < nq) s_q[w][lane] = q[(int64_t)lane * n + i];
@@ -341,7 +264,7 @@ gik_tail_kernel(const __grid_constant__ DevTable<T> tab, const DevScene<T>* __re
       const int g = lane + 32 * sl;
       if (g < ng) {
         T Pc[12];
-        place_geom(sc, g, cube, s_oMi[w], Pc);
+        place_geom(sc, g, cube, 1, 0, s_oMi[w], Pc);
         T dR = T(0), dp = T(0);
 #pragma unroll
         for (int k = 0; k < 9; ++k) { const T d = Pc[k] - Pf[sl][k]; dR += d * d; }
@@ -453,8 +376,8 @@ gik_tail_kernel(const __grid_constant__ DevTable<T> tab, const DevScene<T>* __re
             const int k = s_cand[w][c0 + lane];
             const int a = pa[k], b = pb[k];
             T Ma[12], Mb[12];
-            place_geom(sc, a, cube, s_oMi[w], Ma);
-            place_geom(sc, b, cube, s_oMi[w], Mb);
+            place_geom(sc, a, cube, 1, 0, s_oMi[w], Ma);
+            place_geom(sc, b, cube, 1, 0, s_oMi[w], Mb);
             hit = narrow_hits(sc->g[a], Ma, sc->g[b], Mb, T(0));
           }
           collide = __any_sync(0xffffffffu, hit);
@@ -495,17 +418,11 @@ gik_tail_kernel(const __grid_constant__ DevTable<T> tab, const DevScene<T>* __re
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-namespace gik {
-constexpr int kTrajPairCap = GIK_MAX_PAIRS + 2;   // list 3: at most list 0 plus the cube's two own pairs
-}
-
 struct gik_scene_dev {
   gik::DevScene<float>* sc32 = nullptr;
   gik::DevScene<double>* sc64 = nullptr;
-  // [3 lists][2][GIK_MAX_PAIRS]: all pairs | table/obstacle pairs | cube vs table, obstacle; then list 3 as
-  // [2][kTrajPairCap]: the trajectory check's pairs (gik_traj.cuh)
-  uint8_t* pairs = nullptr;
-  int n_list[4] = {0, 0, 0, 0};
+  uint8_t (*pairs)[2][gik::kPairListCap] = nullptr;   // gik::PairLists::pairs on the device
+  int n_list[gik::kNumPairLists] = {};
 };
 
 namespace {
@@ -520,9 +437,12 @@ template <typename T> gik::DevScene<T>* scene_of(gik_scene_dev* sd);
 template <> gik::DevScene<float>* scene_of<float>(gik_scene_dev* sd) { return sd->sc32; }
 template <> gik::DevScene<double>* scene_of<double>(gik_scene_dev* sd) { return sd->sc64; }
 
-// list: 0 all pairs, 1 table/obstacle pairs, 2 cube's own pairs
+// one pair list of the attached scene on the device: pair k = (a[k], b[k]), k < n
+struct DevPairList { const uint8_t *a, *b; int n; };
+DevPairList pair_list(const gik_scene_dev* sd, gik::PairList l) { return {sd->pairs[l][0], sd->pairs[l][1], sd->n_list[l]}; }
+
 template <typename T>
-int collide_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, int list, double margin, int invert,
+int collide_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, gik::PairList list, double margin, int invert,
                 uint8_t* out, void* stream, const int64_t* sel = nullptr, int64_t n_sel = 0,
                 const int64_t* n_sel_dev = nullptr) {
   if (bad_handle(h)) return GIK_E_HANDLE;
@@ -531,22 +451,23 @@ int collide_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, int l
   if (!h->scene) return GIK_E_NOSCENE;
   if (n == 0 || (sel && !n_sel_dev && n_sel == 0)) return GIK_OK;
   if (n_sel < 0) return GIK_E_SIZE;
-  if (!out || (list != 2 && !q) || (list == 2 && !cube_pose)) return GIK_E_NULL;
+  const bool cube_only = list == gik::kListCube;
+  if (!out || (!cube_only && !q) || (cube_only && !cube_pose)) return GIK_E_NULL;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  gik_scene_dev* sd = h->scene;
   const int64_t work = (sel && !n_sel_dev) ? n_sel : n;     // device-side count: size the grid for the upper bound
   int64_t blocks = (work + gik::kCollideWarps - 1) / gik::kCollideWarps;
   const int64_t cap = (int64_t)h->sm_count * 16;
   if (blocks > cap) blocks = cap;
-  const uint8_t* pa = sd->pairs + (size_t)list * 2 * GIK_MAX_PAIRS;
+  const DevPairList pl = pair_list(h->scene, list);
   gik::gik_collision_kernel<T><<<(int)blocks, gik::kCollideWarps * 32, 0, (cudaStream_t)stream>>>(
-      scene_of<T>(sd), pa, pa + GIK_MAX_PAIRS, sd->n_list[list], n, q, cube_pose, (T)margin, out, invert, sel, n_sel, n_sel_dev);
+      scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, q, cube_pose, (T)margin, out, invert, sel, n_sel, n_sel_dev);
   return (int)cudaGetLastError();
 }
 
 template <typename T>
-int distance_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, int list, double d_max, T* out, void* stream) {
+int distance_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, gik::PairList list, double d_max, T* out,
+                 void* stream) {
   if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0) return GIK_E_SIZE;
   if (!(d_max > 0.0)) return GIK_E_PARAM;
@@ -555,14 +476,13 @@ int distance_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, int 
   if (!out || !q) return GIK_E_NULL;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  gik_scene_dev* sd = h->scene;
   int64_t blocks = (n + gik::kCollideWarps - 1) / gik::kCollideWarps;
   const int64_t cap = (int64_t)h->sm_count * 16;
   if (blocks > cap) blocks = cap;
-  const uint8_t* pa = sd->pairs + (size_t)list * 2 * GIK_MAX_PAIRS;
+  const DevPairList pl = pair_list(h->scene, list);
   const int rounds = sizeof(T) == 4 ? 20 : 40;       // d_max / 2^rounds: below the arithmetic's own resolution
   gik::gik_distance_kernel<T><<<(int)blocks, gik::kCollideWarps * 32, 0, (cudaStream_t)stream>>>(
-      scene_of<T>(sd), pa, pa + GIK_MAX_PAIRS, sd->n_list[list], n, q, cube_pose, (T)d_max, rounds, out);
+      scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, q, cube_pose, (T)d_max, rounds, out);
   return (int)cudaGetLastError();
 }
 
@@ -623,7 +543,7 @@ int solve_success_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose,
   if (blocks > (int64_t)h->sm_count * 8) blocks = (int64_t)h->sm_count * 8;
   gik::gik_compact_converged_kernel<<<(int)blocks, 256, 0, st>>>(n, conv, success, sc.sel1, sc.sel1 + 1);
   if ((e = cudaGetLastError()) != cudaSuccess) return (int)e;
-  rc = collide_api<T>(h, n, q_out, pose, 0, 0.0, 1, success, stream, sc.sel1 + 1, 0, sc.sel1);
+  rc = collide_api<T>(h, n, q_out, pose, gik::kListAll, 0.0, 1, success, stream, sc.sel1 + 1, 0, sc.sel1);
   if (rc || (prm->flags & GIK_F_NO_DESCEND)) return rc;
   // ---- the tail
   gik::gik_compact_pending_kernel<<<(int)blocks, 256, 0, st>>>(n, conv, success, iters, prm->max_iters, sc.sel2, sc.sel2 + 1);
@@ -640,8 +560,7 @@ int solve_success_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose,
     rc = launch_solve<T, MODE_BATCH>(h, a, &p2, stream, /*force=*/true);
     if (rc) return rc;
   }
-  gik_scene_dev* sd = h->scene;
-  const uint8_t* pa = sd->pairs;
+  const DevPairList pl = pair_list(h->scene, gik::kListAll);
   int64_t tb = (n + gik::kCollideWarps - 1) / gik::kCollideWarps;
   const int64_t cap = (int64_t)h->sm_count * 16;
   if (tb > cap) tb = cap;
@@ -651,7 +570,7 @@ int solve_success_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose,
   // queue[0] / queue[5]: work counters of the two stages; queue[1..4]: statistics
   auto launch_tail = [&](auto kern, int64_t blocks_, const int64_t* list, unsigned long long* q_) {
     kern<<<(int)blocks_, gik::kCollideWarps * 32, 0, st>>>(
-        table_of<T>(h), scene_of<T>(sd), pa, pa + GIK_MAX_PAIRS, sd->n_list[0], n, list + 1, list, pose, (const T*)sc.q_fin,
+        table_of<T>(h), scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, list + 1, list, pose, (const T*)sc.q_fin,
         (const T*)sc.resid_fin, q_out, success, conv, iters, resid, eps2, (T)prm->dt, (T)prm->damping, prm->max_iters, safety,
         q_, sc.queue + 1, sc.sel3, sc.sel3 + 1);
   };
@@ -679,52 +598,21 @@ int gik_scene_attach(gik_handle_t h, const gik_scene_t* scene) {
   if (!sd) return (int)cudaErrorMemoryAllocation;
   gik::DevScene<float>* h32 = new (std::nothrow) gik::DevScene<float>();
   gik::DevScene<double>* h64 = new (std::nothrow) gik::DevScene<double>();
-  const size_t pair_bytes = (size_t)6 * GIK_MAX_PAIRS + 2 * gik::kTrajPairCap;
-  uint8_t* hp = new (std::nothrow) uint8_t[pair_bytes]();
-  cudaError_t e = (h32 && h64 && hp) ? cudaSuccess : cudaErrorMemoryAllocation;
+  gik::PairLists* hl = new (std::nothrow) gik::PairLists();
+  cudaError_t e = (h32 && h64 && hl) ? cudaSuccess : cudaErrorMemoryAllocation;
   if (e == cudaSuccess) {
     gik::fill_dev_scene(h->host, *scene, *h32);
     gik::fill_dev_scene(h->host, *scene, *h64);
-    for (int k = 0; k < scene->n_pairs; ++k) {
-      const uint8_t a = scene->pair_a[k], b = scene->pair_b[k];
-      hp[sd->n_list[0]] = a; hp[GIK_MAX_PAIRS + sd->n_list[0]++] = b;
-      if ((int)b == scene->table_geom || (int)b == scene->obstacle_geom) {          // tools.py:42
-        hp[2 * GIK_MAX_PAIRS + sd->n_list[1]] = a; hp[3 * GIK_MAX_PAIRS + sd->n_list[1]++] = b;
-      }
-    }
-    const int env[2] = {scene->table_geom, scene->obstacle_geom};                    // setup_pinocchio.py:66-70
-    for (int k = 0; k < 2; ++k)
-      if (env[k] >= 0 && scene->cube_geom >= 0) {
-        hp[4 * GIK_MAX_PAIRS + sd->n_list[2]] = (uint8_t)env[k]; hp[5 * GIK_MAX_PAIRS + sd->n_list[2]++] = (uint8_t)scene->cube_geom;
-      }
-    // list 3 (gik_traj_check_*): list 0 without the pairs of the cube with a geometry on either hand joint -- the grasp
-    // error judges that contact, GJK would only measure the millimetre between the fingers and the cube -- plus the
-    // pairs of list 2 that list 0 lacks
-    uint8_t* l3a = hp + 6 * GIK_MAX_PAIRS;
-    uint8_t* l3b = l3a + gik::kTrajPairCap;
-    auto on_hand = [&](int g) {
-      return scene->geoms[g].joint == h->host.hand_joint[0] || scene->geoms[g].joint == h->host.hand_joint[1];
-    };
-    for (int k = 0; k < sd->n_list[0]; ++k) {
-      const int a = hp[k], b = hp[GIK_MAX_PAIRS + k];
-      if ((a == scene->cube_geom && on_hand(b)) || (b == scene->cube_geom && on_hand(a))) continue;
-      l3a[sd->n_list[3]] = (uint8_t)a; l3b[sd->n_list[3]++] = (uint8_t)b;
-    }
-    for (int k = 0; k < sd->n_list[2]; ++k) {
-      const int a = hp[4 * GIK_MAX_PAIRS + k], b = hp[5 * GIK_MAX_PAIRS + k];
-      bool listed = false;
-      for (int j = 0; j < sd->n_list[3] && !listed; ++j)
-        listed = (l3a[j] == a && l3b[j] == b) || (l3a[j] == b && l3b[j] == a);
-      if (!listed) { l3a[sd->n_list[3]] = (uint8_t)a; l3b[sd->n_list[3]++] = (uint8_t)b; }
-    }
+    gik::build_pair_lists(h->host, *scene, *hl);
+    for (int l = 0; l < gik::kNumPairLists; ++l) sd->n_list[l] = hl->n[l];
     if ((e = cudaMalloc(&sd->sc32, sizeof(*h32))) == cudaSuccess &&
         (e = cudaMalloc(&sd->sc64, sizeof(*h64))) == cudaSuccess &&
-        (e = cudaMalloc(&sd->pairs, pair_bytes)) == cudaSuccess &&
+        (e = cudaMalloc(&sd->pairs, sizeof(hl->pairs))) == cudaSuccess &&
         (e = cudaMemcpy(sd->sc32, h32, sizeof(*h32), cudaMemcpyHostToDevice)) == cudaSuccess &&
         (e = cudaMemcpy(sd->sc64, h64, sizeof(*h64), cudaMemcpyHostToDevice)) == cudaSuccess)
-      e = cudaMemcpy(sd->pairs, hp, pair_bytes, cudaMemcpyHostToDevice);
+      e = cudaMemcpy(sd->pairs, hl->pairs, sizeof(hl->pairs), cudaMemcpyHostToDevice);
   }
-  delete h32; delete h64; delete[] hp;
+  delete h32; delete h64; delete hl;
   if (e != cudaSuccess) { free_scene(sd); return (int)e; }
   cudaDeviceSynchronize();          // a previous scene may still be in use by enqueued kernels
   free_scene(h->scene);
@@ -732,15 +620,15 @@ int gik_scene_attach(gik_handle_t h, const gik_scene_t* scene) {
   return GIK_OK;
 }
 
-int gik_collision_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, uint8_t* out, void* s) { return collide_api<float>(h, n, q, cube, 0, 0.0, 0, out, s); }
-int gik_collision_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, uint8_t* out, void* s) { return collide_api<double>(h, n, q, cube, 0, 0.0, 0, out, s); }
+int gik_collision_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, uint8_t* out, void* s) { return collide_api<float>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s); }
+int gik_collision_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, uint8_t* out, void* s) { return collide_api<double>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s); }
 int gik_collision_sel_f32(gik_handle_t h, int64_t n, int64_t n_sel, const int64_t* sel, const float* q, const float* cube, uint8_t* out, void* s) {
   if (!sel) return GIK_E_NULL;
-  return collide_api<float>(h, n, q, cube, 0, 0.0, 0, out, s, sel, n_sel);
+  return collide_api<float>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s, sel, n_sel);
 }
 int gik_collision_sel_f64(gik_handle_t h, int64_t n, int64_t n_sel, const int64_t* sel, const double* q, const double* cube, uint8_t* out, void* s) {
   if (!sel) return GIK_E_NULL;
-  return collide_api<double>(h, n, q, cube, 0, 0.0, 0, out, s, sel, n_sel);
+  return collide_api<double>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s, sel, n_sel);
 }
 int gik_solve_success_f32(gik_handle_t h, int64_t n, const float* q_init, const float* pose, const gik_params_t* p, float* q_out,
                           uint8_t* success, uint8_t* conv, int32_t* iters, float* resid, void* scratch, void* s) {
@@ -754,11 +642,11 @@ size_t gik_solve_success_scratch_bytes(gik_handle_t h, int64_t n, int elem_size)
   if (bad_handle(h) || n < 0 || (elem_size != 4 && elem_size != 8)) return 0;
   return carve_scratch(nullptr, n, h->host.nq, elem_size).bytes;
 }
-int gik_clearance_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, double thr, uint8_t* out, void* s) { return collide_api<float>(h, n, q, cube, 1, thr, 1, out, s); }
-int gik_clearance_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, double thr, uint8_t* out, void* s) { return collide_api<double>(h, n, q, cube, 1, thr, 1, out, s); }
-int gik_obstacle_distance_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, double d_max, float* dist, void* s) { return distance_api<float>(h, n, q, cube, 1, d_max, dist, s); }
-int gik_obstacle_distance_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, double d_max, double* dist, void* s) { return distance_api<double>(h, n, q, cube, 1, d_max, dist, s); }
-int gik_cube_collision_f32(gik_handle_t h, int64_t n, const float* cube, uint8_t* out, void* s) { return collide_api<float>(h, n, (const float*)nullptr, cube, 2, 0.0, 0, out, s); }
-int gik_cube_collision_f64(gik_handle_t h, int64_t n, const double* cube, uint8_t* out, void* s) { return collide_api<double>(h, n, (const double*)nullptr, cube, 2, 0.0, 0, out, s); }
+int gik_clearance_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, double thr, uint8_t* out, void* s) { return collide_api<float>(h, n, q, cube, gik::kListEnv, thr, 1, out, s); }
+int gik_clearance_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, double thr, uint8_t* out, void* s) { return collide_api<double>(h, n, q, cube, gik::kListEnv, thr, 1, out, s); }
+int gik_obstacle_distance_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, double d_max, float* dist, void* s) { return distance_api<float>(h, n, q, cube, gik::kListEnv, d_max, dist, s); }
+int gik_obstacle_distance_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, double d_max, double* dist, void* s) { return distance_api<double>(h, n, q, cube, gik::kListEnv, d_max, dist, s); }
+int gik_cube_collision_f32(gik_handle_t h, int64_t n, const float* cube, uint8_t* out, void* s) { return collide_api<float>(h, n, (const float*)nullptr, cube, gik::kListCube, 0.0, 0, out, s); }
+int gik_cube_collision_f64(gik_handle_t h, int64_t n, const double* cube, uint8_t* out, void* s) { return collide_api<double>(h, n, (const double*)nullptr, cube, gik::kListCube, 0.0, 0, out, s); }
 
 }  // extern "C"

@@ -196,4 +196,53 @@ inline void fill_dev_scene(const gik_table_t& t, const gik_scene_t& s, DevScene<
   }
 }
 
+// ---- the pair lists of a scene: each collision query scans one of them ----
+enum PairList {
+  kListAll = 0,    // every pair of the scene: collision(q)
+  kListEnv = 1,    // the pairs whose second geometry is the table or the obstacle: distanceToObstacle, clearance
+  kListCube = 2,   // the cube against the table and the obstacle: the cube-only test
+  kListTraj = 3,   // the trajectory check's pairs (gik_traj.cuh)
+  kNumPairLists = 4
+};
+constexpr int kPairListCap = GIK_MAX_PAIRS + 2;   // kListTraj: at most every pair plus the cube's two own pairs
+
+struct PairLists {
+  uint8_t pairs[kNumPairLists][2][kPairListCap];   // pair k of list l: (pairs[l][0][k], pairs[l][1][k])
+  int32_t n[kNumPairLists];
+};
+
+// The scene must have passed validate_scene.
+inline void build_pair_lists(const gik_table_t& t, const gik_scene_t& s, PairLists& L) {
+  memset(&L, 0, sizeof(L));
+  auto add = [&](int l, int a, int b) {
+    L.pairs[l][0][L.n[l]] = (uint8_t)a;
+    L.pairs[l][1][L.n[l]++] = (uint8_t)b;
+  };
+  for (int k = 0; k < s.n_pairs; ++k) {
+    const int a = s.pair_a[k], b = s.pair_b[k];
+    add(kListAll, a, b);
+    if (b == s.table_geom || b == s.obstacle_geom) add(kListEnv, a, b);          // tools.py:42
+  }
+  const int env[2] = {s.table_geom, s.obstacle_geom};                            // setup_pinocchio.py:66-70
+  for (int e : env)
+    if (e >= 0 && s.cube_geom >= 0) add(kListCube, e, s.cube_geom);
+  // kListTraj: kListAll without the pairs of the cube with a geometry on either hand joint -- the grasp error judges
+  // that contact, GJK would only measure the millimetre between the fingers and the cube -- plus the pairs of kListCube
+  // that kListAll lacks
+  auto on_hand = [&](int g) { return s.geoms[g].joint == t.hand_joint[0] || s.geoms[g].joint == t.hand_joint[1]; };
+  for (int k = 0; k < L.n[kListAll]; ++k) {
+    const int a = L.pairs[kListAll][0][k], b = L.pairs[kListAll][1][k];
+    if ((a == s.cube_geom && on_hand(b)) || (b == s.cube_geom && on_hand(a))) continue;
+    add(kListTraj, a, b);
+  }
+  for (int k = 0; k < L.n[kListCube]; ++k) {
+    const int a = L.pairs[kListCube][0][k], b = L.pairs[kListCube][1][k];
+    const uint8_t* ta = L.pairs[kListTraj][0];
+    const uint8_t* tb = L.pairs[kListTraj][1];
+    bool listed = false;
+    for (int j = 0; j < L.n[kListTraj] && !listed; ++j) listed = (ta[j] == a && tb[j] == b) || (ta[j] == b && tb[j] == a);
+    if (!listed) add(kListTraj, a, b);
+  }
+}
+
 }  // namespace gik

@@ -7,10 +7,10 @@
 // every sample (n, k) of every trajectory is checked on the device: one warp per sample, trajectory-major, so the M
 // warps of one trajectory share its control points through the read-only cache.  Lane j evaluates q_j, the warp walks
 // the tree (warp_tree_fk), one lane derives both hand frames, the cube placement each hand implies and the grasp error,
-// the lanes place the geometries with the left hand's cube (place_geom) and the pairs of list 3 go through the same
-// broad phase with compaction and GJK on full warps of candidates as gik_collision_kernel.  Per trajectory only min /
-// max reductions are kept (atomicMin of (sample << 3 | bits), atomicMax of the error's bits), so the outputs do not
-// depend on the launch configuration or on the order in which warps finish.
+// the lanes place the geometries with the left hand's cube (place_geom) and the pairs of list 3 (kListTraj) go through
+// gik_collision_kernel's any-hit pair test (warp_any_pair_hits, gik_collide_impl.cuh).  Per trajectory only min / max
+// reductions are kept (atomicMin of (sample << 3 | bits), atomicMax of the error's bits), so the outputs do not depend
+// on the launch configuration or on the order in which warps finish.
 //
 // The per-sample arithmetic is GIK_HD: tests/test_traj_check_cpu.py compiles it with g++ against numpy.
 #pragma once
@@ -160,41 +160,11 @@ gik_traj_check_kernel(const __grid_constant__ TrajConst<T> tc, const DevScene<T>
     // collisions of list 3 with the cube at C_L.  Without per-sample flags, a sample after the trajectory's first bad
     // one so far cannot change any output (the key is a minimum): its pair tests are skipped (a relaxed read).
     if (sample_flags || k <= (ld_relaxed(key + n) >> 3)) {
-      for (int g = lane; g < ng; g += 32) place_geom(sc, g, &s_cube[w][0], s_oMi[w], &s_oMg[w][g][0]);
+      for (int g = lane; g < ng; g += 32) place_geom(sc, g, s_cube[w], 1, 0, s_oMi[w], s_oMg[w][g]);
       __syncwarp();
-      bool hit = false;
-      int n_cand = 0;
-      for (int k0 = 0; k0 < n_pairs && !hit; k0 += 32) {
-        const int p = k0 + lane;
-        bool pass = false;
-        if (p < n_pairs) {
-          const int a = pa[p], b = pb[p];
-          const T* Ma = &s_oMg[w][a][0];
-          const T* Mb = &s_oMg[w][b][0];
-          const T dx = Ma[9] - Mb[9], dy = Ma[10] - Mb[10], dz = Ma[11] - Mb[11];
-          const T reach = sc->g[a].bound + sc->g[b].bound;
-          pass = dx * dx + dy * dy + dz * dz <= reach * reach;
-        }
-        const unsigned m = __ballot_sync(0xffffffffu, pass);
-        if (n_cand + __popc(m) > kMaxCand) {
-          // list full (never with the reference scene): test this round's survivors in place
-          if (pass) hit = gjk_intersect(make_shape(sc->g[pa[p]], &s_oMg[w][pa[p]][0]), make_shape(sc->g[pb[p]], &s_oMg[w][pb[p]][0]), T(0));
-          hit = __any_sync(0xffffffffu, hit);
-        } else {
-          if (pass) s_cand[w][n_cand + __popc(m & ((1u << lane) - 1u))] = (uint16_t)p;
-          n_cand += __popc(m);
-        }
-      }
-      __syncwarp();
-      for (int c0 = 0; c0 < n_cand && !hit; c0 += 32) {
-        if (c0 + lane < n_cand) {
-          const int p = s_cand[w][c0 + lane];
-          const int a = pa[p], b = pb[p];
-          hit = gjk_intersect(make_shape(sc->g[a], &s_oMg[w][a][0]), make_shape(sc->g[b], &s_oMg[w][b][0]), T(0));
-        }
-        hit = __any_sync(0xffffffffu, hit);
-      }
-      if (hit) bits |= 4u;
+      // margin -0: x + (-0) == x for every x, so the compiler drops the margin's add from the broad phase, and -0 > 0
+      // is as false as +0 > 0 in the narrow phase: the plain intersection test, at no extra cost
+      if (warp_any_pair_hits(sc, pa, pb, n_pairs, s_oMg[w], s_cand[w], T(-0.0), lane)) bits |= 4u;
     }
     if (lane == 0) {
       if (bits) atomicMin(key + n, (int32_t)(((unsigned)k << 3) | bits));
@@ -228,7 +198,6 @@ int traj_check_api(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_sam
   cudaStream_t st = (cudaStream_t)stream;
   gik::TrajConst<T> tc;
   gik::fill_traj_const(h->host, limit_tol, tc);
-  gik_scene_dev* sd = h->scene;
   int64_t rb = (n_traj + 255) / 256;
   if (rb > (int64_t)h->sm_count * 8) rb = (int64_t)h->sm_count * 8;
   gik::gik_traj_init_kernel<T><<<(int)rb, 256, 0, st>>>(n_traj, first_bad, grasp_err);
@@ -237,9 +206,9 @@ int traj_check_api(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_sam
   const int64_t total = n_traj * n_samples;
   int64_t blocks = (total + gik::kTrajWarps - 1) / gik::kTrajWarps;
   if (blocks > (int64_t)h->sm_count * 16) blocks = (int64_t)h->sm_count * 16;
-  const uint8_t* pa = sd->pairs + (size_t)6 * GIK_MAX_PAIRS;
+  const DevPairList pl = pair_list(h->scene, gik::kListTraj);
   gik::gik_traj_check_kernel<T><<<(int)blocks, gik::kTrajWarps * 32, 0, st>>>(
-      tc, scene_of<T>(sd), pa, pa + gik::kTrajPairCap, sd->n_list[3], n_traj, n_ctrl, n_samples, weights, ctrl,
+      tc, scene_of<T>(h->scene), pl.a, pl.b, pl.n, n_traj, n_ctrl, n_samples, weights, ctrl,
       (T)grasp_tol, first_bad, grasp_err, sample_flags);
   if ((e = cudaGetLastError()) != cudaSuccess) return (int)e;
   gik::gik_traj_finish_kernel<<<(int)rb, 256, 0, st>>>(n_traj, first_bad, valid, reason);

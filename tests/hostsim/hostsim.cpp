@@ -107,37 +107,28 @@ static int solve_impl(const gik_table_t* tab, int64_t n, const T* q_init, const 
   return 0;
 }
 
-// collision predicate, sequential over pairs (the kernel deals the same pairs to the lanes of a warp)
+// collision predicate over one pair list (PairList: 0 all pairs, 1 table/obstacle pairs, 2 the cube's own pairs),
+// sequential over pairs (the kernel deals the same pairs to the lanes of a warp)
 template <typename T>
 static int collide_impl(const gik_table_t* tab, const gik_scene_t* scn, int64_t n, const T* q, const T* cube, int list,
                         double margin, uint8_t* out) {
+  if (list < 0 || list >= kNumPairLists) return GIK_E_PARAM;
   int rc = validate_table(*tab);
   if (rc == 0) rc = validate_scene(*tab, *scn);
   if (rc) return rc;
   static DevScene<T> sc;
+  static PairLists L;
   fill_dev_scene(*tab, *scn, sc);
+  build_pair_lists(*tab, *scn, L);
+  const uint8_t *pa = L.pairs[list][0], *pb = L.pairs[list][1];
   for (int64_t i = 0; i < n; ++i) {
     T oMi[GIK_MAX_NQ][12], oMg[GIK_MAX_GEOMS][12];
     if (q)
       for (int j = 0; j < sc.tree.nq; ++j)
         joint_placement(sc.tree, j, sc.tree.parent[j] < 0 ? (const T*)nullptr : oMi[sc.tree.parent[j]], q[(int64_t)j * n + i], oMi[j]);
-    for (int g = 0; g < sc.n_geoms; ++g) {
-      T P[12];
-      for (int k = 0; k < 9; ++k) P[k] = sc.g[g].R[k];
-      for (int k = 0; k < 3; ++k) P[9 + k] = sc.g[g].p[k];
-      if (g == sc.cube_geom && cube) for (int k = 0; k < 12; ++k) P[k] = cube[(int64_t)k * n + i];
-      if (sc.g[g].joint >= 0 && q) se3_mul12(oMi[sc.g[g].joint], P, oMg[g]);
-      else for (int k = 0; k < 12; ++k) oMg[g][k] = P[k];
-    }
+    for (int g = 0; g < sc.n_geoms; ++g) place_geom(&sc, g, cube, n, i, q ? oMi : nullptr, oMg[g]);
     bool hit = false;
-    const int np = list == 2 ? 2 : scn->n_pairs;
-    for (int k = 0; k < np && !hit; ++k) {
-      int a, b;
-      if (list == 2) { a = k == 0 ? scn->table_geom : scn->obstacle_geom; b = scn->cube_geom; }
-      else { a = scn->pair_a[k]; b = scn->pair_b[k]; }
-      if (list == 1 && b != scn->table_geom && b != scn->obstacle_geom) continue;
-      hit = pair_hits(sc.g[a], oMg[a], sc.g[b], oMg[b], (T)margin);
-    }
+    for (int k = 0; k < L.n[list] && !hit; ++k) hit = pair_hits(sc.g[pa[k]], oMg[pa[k]], sc.g[pb[k]], oMg[pb[k]], (T)margin);
     out[i] = hit ? 1 : 0;
   }
   return 0;
@@ -168,6 +159,17 @@ void hostsim_atan2_pos_f64(int64_t n, const double* y, const double* x, double* 
 }
 void hostsim_atan2_pos_f32(int64_t n, const float* y, const float* x, float* out) {
   for (int64_t i = 0; i < n; ++i) out[i] = atan2_pos(y[i], x[i]);
+}
+// pair list `list` of the scene (gik_scene_attach's lists) -> a[n], b[n] with room for kPairListCap; returns n, < 0: error
+int hostsim_pair_lists(const gik_table_t* t, const gik_scene_t* s, int list, uint8_t* a, uint8_t* b) {
+  if (list < 0 || list >= kNumPairLists) return GIK_E_PARAM;
+  int rc = validate_table(*t);
+  if (rc == 0) rc = validate_scene(*t, *s);
+  if (rc) return rc;
+  static PairLists L;
+  build_pair_lists(*t, *s, L);
+  for (int k = 0; k < L.n[list]; ++k) { a[k] = L.pairs[list][0][k]; b[k] = L.pairs[list][1][k]; }
+  return L.n[list];
 }
 int hostsim_collide_f32(const gik_table_t* t, const gik_scene_t* s, int64_t n, const float* q, const float* cube, int list, double m, uint8_t* o) { return collide_impl<float>(t, s, n, q, cube, list, m, o); }
 int hostsim_collide_f64(const gik_table_t* t, const gik_scene_t* s, int64_t n, const double* q, const double* cube, int list, double m, uint8_t* o) { return collide_impl<double>(t, s, n, q, cube, list, m, o); }

@@ -1,5 +1,6 @@
 """Collision predicate on the CPU: the scene flattener, the oracle (alternating projections) against engine-independent
-exact answers, and the product's GJK (csrc/gik_collide.cuh compiled for the host) against the oracle."""
+exact answers, the product's GJK and geometry placement (csrc/gik_collide.cuh compiled for the host) against the
+oracle, and the scene's pair lists (csrc/gik_table.h) against a numpy restatement."""
 import json
 import os
 
@@ -195,3 +196,45 @@ def test_full_scene_gjk_vs_oracle(table, table_c, scene_c, c_oracle, hostsim):
     got = hostsim.collide(table_c, scene_c, None, Pc, np.float64, mode=2)
     sure = (dc == 0) | (dc > 1e-6)
     assert (got[sure] == (dc[sure] == 0)).all() and 0.1 < got.mean() < 0.9
+
+
+def _pair_list_scenes(scene):
+    """The packaged scene and variants that reach every rule of the pair-list builder."""
+    import copy
+
+    def variant(**kw):
+        s = copy.copy(scene)
+        for k, v in kw.items():
+            setattr(s, k, v)
+        return s
+
+    pairs = np.asarray(scene.pairs)
+    assert tuple(pairs[-1]) == (scene.obstacle, scene.cube)
+    return {"packaged": scene,
+            "no_obstacle": variant(obstacle=-1),
+            "no_cube": variant(cube=-1),
+            "lists_table_cube": variant(pairs=np.concatenate([pairs, [[scene.table, scene.cube]]])),
+            "cube_obstacle_reversed": variant(pairs=np.concatenate([pairs[:-1], [[scene.cube, scene.obstacle]]])),
+            "no_pairs": variant(pairs=np.zeros((0, 2), np.int64))}
+
+
+@pytest.mark.parametrize("which", ["packaged", "no_obstacle", "no_cube", "lists_table_cube", "cube_obstacle_reversed",
+                                   "no_pairs"])
+def test_pair_lists_match_restatement(table, table_c, scene, hostsim, which):
+    # the C builder of gik_scene_attach's four pair lists (csrc/gik_table.h) against a numpy restatement of its rules,
+    # order and orientation included
+    import ctypes
+    from gik_b200.scene import GIK_MAX_PAIRS
+    from traj_oracle import list3_pairs
+    sc = _pair_list_scenes(scene)[which]
+    pairs = np.asarray(sc.pairs, np.int64).reshape(-1, 2)
+    env = [e for e in (sc.table, sc.obstacle) if e >= 0 and sc.cube >= 0]
+    want = [pairs,                                                            # 0: all pairs
+            pairs[(pairs[:, 1] == sc.table) | (pairs[:, 1] == sc.obstacle)],  # 1: second geometry table / obstacle
+            np.array([(e, sc.cube) for e in env], np.int64).reshape(-1, 2),   # 2: the cube against table, obstacle
+            list3_pairs(sc, tuple(int(j) for j in table.hand_joint))]         # 3: the trajectory check's pairs
+    f = hostsim.lib.hostsim_pair_lists
+    for lst, ref in enumerate(want):
+        a, b = np.zeros(GIK_MAX_PAIRS + 2, np.uint8), np.zeros(GIK_MAX_PAIRS + 2, np.uint8)
+        n = f(ctypes.byref(table_c), ctypes.byref(sc.to_c()), lst, hostsim._p(a), hostsim._p(b))
+        assert n >= 0 and np.array_equal(np.stack([a[:n], b[:n]], axis=1), ref), (lst, n)

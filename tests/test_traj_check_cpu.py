@@ -1,6 +1,7 @@
 """The trajectory check's per-sample arithmetic (csrc/gik_traj.cuh) on the CPU: the GIK_HD Bernstein sum, hand frames,
 cube-from-hand and grasp error compiled with g++ in fp64 and fp32 against numpy and the C oracle; maketraj_paths on CPU
-tensors against maketraj; list 3 of the packaged scene; the argument checks of the C entries (no GPU needed)."""
+tensors against maketraj; list 3 of the packaged scene, restated and as the C builder makes it; the argument checks of
+the C entries (no GPU needed)."""
 import ctypes
 import os
 import subprocess
@@ -263,11 +264,16 @@ def test_maketraj_paths_equals_maketraj_per_path():
         assert np.abs(ctrl[i].numpy() - ref).max() < 1e-9 * max(1.0, np.abs(ref).max()), (i, n)
 
 
-def test_list3_of_the_packaged_scene(table):
+def test_list3_of_the_packaged_scene(table, table_c, hostsim):
     import gik_b200
+    from gik_b200.scene import GIK_MAX_PAIRS
     sc = gik_b200.nextage_scene()
     hands = tuple(int(j) for j in table.hand_joint)
     L3 = list3_pairs(sc, hands)
+    # the list gik_scene_attach uploads (csrc/gik_table.h, build_pair_lists) is this restatement, in its order
+    a, b = np.zeros(GIK_MAX_PAIRS + 2, np.uint8), np.zeros(GIK_MAX_PAIRS + 2, np.uint8)
+    n = hostsim.lib.hostsim_pair_lists(ctypes.byref(table_c), ctypes.byref(sc.to_c()), 3, _p(a), _p(b))
+    assert n >= 0 and np.array_equal(np.stack([a[:n], b[:n]], axis=1), L3)
     on_hand = [g for g, geom in enumerate(sc.geoms) if geom.joint in hands]
     cube_hand = [(a, b) for a, b in sc.pairs if (a == sc.cube and b in on_hand) or (b == sc.cube and a in on_hand)]
     assert len(on_hand) == 4 and len(cube_hand) == 4
