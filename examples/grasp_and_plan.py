@@ -48,6 +48,14 @@ def main():
     t4 = time.perf_counter()
     print(f"check: valid {verdict['valid']}, first bad sample {verdict['first_bad']} (reason {verdict['reason']}: "
           f"1 limits, 2 grasp, 4 collision), max grasp error {verdict['grasp_err']:.2e}  ({(t4 - t3) * 1e3:.1f} ms)")
+    P = np.array(q_of_t.control_points_)[None]
+    refined = gik_b200.refine_trajectories_batch(torch.as_tensor(P))
+    P[0] = refined["ctrl"][0].cpu().numpy()
+    verdict = gik_b200.check_trajectory(gik_b200.Bezier(list(P[0]), t_min=q_of_t.T_min_, t_max=q_of_t.T_max_))
+    t5 = time.perf_counter()
+    print(f"refined: {int(refined['accepted'][0])} steps, check: valid {verdict['valid']}, first bad sample "
+          f"{verdict['first_bad']} (reason {verdict['reason']}), max grasp error {verdict['grasp_err']:.2e}  "
+          f"({(t5 - t4) * 1e3:.1f} ms)")
     return 0
 
 

@@ -435,6 +435,41 @@ int gik_traj_check_f64(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n
                        const double* ctrl, double limit_tol, double grasp_tol, uint8_t* valid, int32_t* first_bad,
                        uint8_t* reason, double* grasp_err, uint8_t* sample_flags, void* stream);
 
+/* Trajectory refinement onto the grasp: the left hand leads, the right arm follows.  Same trajectories and weights as
+ * gik_traj_check_* (ctrl [n_traj][n_ctrl][nq], weights [n_samples][n_ctrl]).  With r_k = log6(C_L^-1 C_R) at sample k
+ * (the residual whose norm the check's bit 1 judges, C_h = H_h * hook_h^-1 from the IK kernels' hand chain), it lowers
+ * F = sum_k ||r_k||^2 by changing only the right-arm columns (act_q[7..12]) of the free control points 3 .. n_ctrl-4.
+ * The three pinned control points at each end and every other column are copied bit for bit.  Levenberg-Marquardt:
+ *   1. at the accepted X: q_k = sum_i weights[k][i] * ctrl[i] (i ascending), r_k, and the model Jacobian
+ *      J_k = Ad(hook_R) J_R, J_R = the right-arm columns of RARM_EFF's LOCAL Jacobian (gik_jac_*): C_R(q + dq) =
+ *      C_R exp(Ad(hook_R) J_R dq), so r_k moves by J_k dq to first order when Jlog6 is ignored, as the IK step does;
+ *   2. H = sum_k (w_k w_k^T) (x) (J_k^T J_k), g = sum_k w_k (x) J_k^T r_k over the free control points' weights w_k,
+ *      in fp64 whatever the storage type;
+ *   3. (H + lambda diag H) delta = -g by Cholesky in fp64 (pivots floored);
+ *   4. X' = clamp(X + delta) to the box [min(lower, x0), max(upper, x0)] per value, x0 = its input value: a control
+ *      point that starts inside the limits stays inside (and by the convex hull property so does the curve), one that
+ *      starts outside never moves further out;
+ *   5. F(X') < F(X): accept and lambda /= 10; otherwise reject (H and g are reused) and lambda *= 10;
+ *   6. stop after max_iters trial steps, when max_k ||r_k|| <= tol, or when lambda exceeds 1e10.
+ * Acceptance is judged on the exact F, so F never increases.  Limits enter only through the box, collisions not at all:
+ * gik_traj_check_* stays the judge of both.  lambda starts at `damping`.
+ * Outputs: ctrl_out [n_traj][n_ctrl][nq] (may equal ctrl: in place), and per trajectory obj_before / obj_after (fp64 F
+ * at the input and the output), grasp_err (max_k ||r_k|| at the output, +inf if it is NaN), iters (trial steps) and
+ * accepted (accepted steps).  A trajectory whose F is not finite is copied through with iters = 0.  One CTA per
+ * trajectory and no floating-point atomics: the outputs are identical between runs and do not depend on the batch.
+ * Needs no scene.
+ * Errors: GIK_E_SIZE (n_traj < 0, n_ctrl < 7 or > 26, n_samples < 2 or > 2^28 - 1), GIK_E_PARAM (max_iters < 0, tol
+ * negative or NaN, damping not a finite positive number), GIK_E_NULL (a pointer is NULL and n_traj > 0), GIK_E_HANDLE;
+ * n_traj = 0 is a no-op. */
+int gik_traj_refine_f32(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_samples, const float* weights,
+                        const float* ctrl, int32_t max_iters, double tol, double damping, float* ctrl_out,
+                        double* obj_before, double* obj_after, float* grasp_err, int32_t* iters, int32_t* accepted,
+                        void* stream);
+int gik_traj_refine_f64(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_samples, const double* weights,
+                        const double* ctrl, int32_t max_iters, double tol, double damping, double* ctrl_out,
+                        double* obj_before, double* obj_after, double* grasp_err, int32_t* iters, int32_t* accepted,
+                        void* stream);
+
 #ifdef __cplusplus
 }
 #endif

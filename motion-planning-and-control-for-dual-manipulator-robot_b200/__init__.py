@@ -14,7 +14,7 @@ from .path import (computepath, edge_num_steps, project_edges_batch, project_pat
                    sample_grasp_poses_batch, se3_interpolate)
 from .planner import computepath_batch, shortcut_paths_batch                          # noqa: F401
 from .trajectory import (Bezier, check_trajectories_batch, check_trajectory, maketraj, maketraj_batch,  # noqa: F401
-                         maketraj_paths)
+                         maketraj_paths, refine_trajectories_batch)
 from . import tools                                                                   # noqa: F401
 from . import experiments                                                             # noqa: F401
 from . import dist                                                                     # noqa: F401

@@ -1691,4 +1691,5 @@ const char* gik_version(void) { return "gik 0.1 (sm_100a)"; }
 #include "gik_tree.cuh"
 #include "gik_shortcut.cuh"
 #include "gik_traj.cuh"
+#include "gik_traj_refine.cuh"
 static void gik_free_scene_of(gik_handle_s* h) { free_scene(h->scene); h->scene = nullptr; }

@@ -380,6 +380,30 @@ class GraspIK:
             self.launches += 3
         return valid, first_bad, reason, grasp_err, flags
 
+    def refine_trajectories(self, ctrl: torch.Tensor, weights, *, max_iters: int, tol: float, damping: float):
+        """Refine many Bezier trajectories onto the grasp (gik_traj_refine_*, semantics in include/gik.h): the right
+        arm's free control points follow the left hand.  ctrl [N, n_ctrl, nq] on this device; weights [M, n_ctrl]:
+        Bernstein weights of the samples (trajectory.sample_weights).  -> (ctrl_out [N, n_ctrl, nq], obj_before f64 [N],
+        obj_after f64 [N], grasp_err [N] (max over the samples at the output), iters i32 [N], accepted i32 [N])."""
+        self._chk_dev(ctrl)
+        dt = ctrl.dtype
+        N, n_ctrl, nq = ctrl.shape
+        W = torch.as_tensor(weights, dtype=dt, device=self.device).contiguous()
+        if nq != self.nq or W.dim() != 2 or W.shape[1] != n_ctrl:
+            raise ValueError(f"refine_trajectories: expected ctrl [N, n_ctrl, {self.nq}] and weights [M, n_ctrl]")
+        out = torch.empty_like(ctrl, memory_format=torch.contiguous_format)
+        f64 = lambda: torch.empty((N,), dtype=torch.float64, device=self.device)       # noqa: E731
+        i32 = lambda: torch.empty((N,), dtype=torch.int32, device=self.device)         # noqa: E731
+        obj_before, obj_after, iters, accepted = f64(), f64(), i32(), i32()
+        grasp_err = torch.empty((N,), dtype=dt, device=self.device)
+        f = getattr(self._lib, f"gik_traj_refine_{_sfx(dt)}")
+        _cabi.check(f(self._h, N, n_ctrl, W.shape[0], self._ptr(W), self._ptr(ctrl.contiguous()), int(max_iters),
+                      float(tol), float(damping), self._ptr(out), self._ptr(obj_before), self._ptr(obj_after),
+                      self._ptr(grasp_err), self._ptr(iters), self._ptr(accepted), self._stream()), "gik_traj_refine")
+        if N:
+            self.launches += 1
+        return out, obj_before, obj_after, grasp_err, iters, accepted
+
     # ------------------------------------------------------------------ RRT-connect trees on the device (csrc/gik_tree.cuh)
     # verts [n_trees][nq][cap], cubes [n_trees][12][cap], parent i32 [n_trees][cap], n_verts i32 [n_trees]
     def _chk_tree(self, verts, n_verts, cubes=None, parent=None):

@@ -177,6 +177,33 @@ def check_trajectories_batch(ctrl, *, n_samples=CHECK_SAMPLES, grasp_tol=GRASP_T
     return out
 
 
+REFINE_ITERS = 8         # Levenberg-Marquardt trial steps: see DESIGN.md "Trajectory refinement" for the table behind it
+REFINE_TOL = 0.5 * GRASP_TOL   # stop once max_k ||r_k|| <= this: half the check's grasp tolerance (the pinned end
+                               # points alone leave ~2e-3 on planned trajectories, so a tighter tol only adds steps)
+REFINE_DAMPING = 1e-3    # initial lambda of (H + lambda diag H)
+
+
+def refine_trajectories_batch(ctrl, *, n_samples=CHECK_SAMPLES, max_iters=REFINE_ITERS, tol=REFINE_TOL, solver=None):
+    """Refine fitted trajectories onto the grasp: the left hand leads, the right arm follows.  ctrl [N, n_ctrl, nq]
+    (maketraj_batch / maketraj_paths; 7 <= n_ctrl <= 26).  One gik_traj_refine_* call (semantics in include/gik.h)
+    moves only the right-arm columns of the free control points so that the grasp error check_trajectories_batch
+    measures at u_k = k / (n_samples - 1) drops: Levenberg-Marquardt on sum_k ||log6(C_L^-1 C_R)||^2, every step kept
+    inside the joint limits (a control point already outside them never moves further out).  Collisions are not
+    considered: check the output.  `solver` as in check_trajectories_batch.  -> dict of tensors on the solver's
+    device: ctrl (the refined control points), obj_before / obj_after fp64 [N] (the objective at input and output),
+    grasp_err [N] (max over the samples at the output), iters int32 [N] (trial steps), accepted int32 [N]."""
+    import torch
+    from .ops import default_solver
+    ctrl = torch.as_tensor(ctrl)
+    s = solver if solver is not None else default_solver(ctrl.device if ctrl.is_cuda else None)
+    ctrl = ctrl.to(s.device)
+    W = sample_weights(ctrl.shape[-2], int(n_samples))
+    out, before, after, grasp_err, iters, accepted = s.refine_trajectories(ctrl, W, max_iters=max_iters, tol=tol,
+                                                                            damping=REFINE_DAMPING)
+    return {"ctrl": out, "obj_before": before, "obj_after": after, "grasp_err": grasp_err, "iters": iters,
+            "accepted": accepted}
+
+
 def check_trajectory(q_of_t, *, n_samples=CHECK_SAMPLES, grasp_tol=GRASP_TOL, limit_tol=LIMIT_TOL, per_sample=False,
                      solver=None, dtype=None):
     """check_trajectories_batch for one reference-style Bezier (maketraj's q_of_t): sampled at n_samples evenly spaced
