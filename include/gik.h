@@ -13,7 +13,8 @@
  *     kinematic table.  Launches are asynchronous on `stream`; the caller synchronises.
  *   - Return value: 0 = ok, negative = invalid argument / unsupported model (GIK_E_*),
  *     positive = a cudaError_t value.  No exceptions cross the ABI.
- *   - A handle is immutable after gik_create: concurrent calls on different streams are safe.
+ *   - A handle is immutable after gik_create, but for its launch counter (atomic): concurrent calls on different
+ *     streams are safe.
  *   - Batch layout is structure-of-arrays, component-major: element (c, i) of a [C][n] array lives at
  *     ptr[c * n + i], so consecutive problems are consecutive addresses.
  *       q      : [nq][n]           joint configuration, pinocchio order (q index = joint id - 1)
@@ -43,6 +44,14 @@ extern "C" {
 #define GIK_E_PARAM           -5   /* bad solver parameter (eps<=0, dt<=0, max_iters<0, damping<0) */
 #define GIK_E_HANDLE          -6   /* bad or destroyed handle */
 #define GIK_E_NOSCENE         -7   /* collision entry called before gik_scene_attach */
+/* Every entry checks its arguments in one order and returns the first fault it finds:
+ *   1. sizes (GIK_E_SIZE)
+ *   2. parameters (GIK_E_PARAM; a NULL gik_params_t* is GIK_E_NULL here)
+ *   3. required pointers, when the call has work to do (GIK_E_NULL)
+ *   4. the handle (GIK_E_HANDLE)
+ *   5. the collision scene, for the entries that use one (GIK_E_NOSCENE)
+ * A call with nothing to do then returns GIK_OK without touching the device.  Checks that need the handle's table
+ * (gik_scene_attach's validation of the scene) come after the handle check. */
 
 /* Host-side flattened kinematic model: what the reference obtains from
  * RobotWrapper.BuildFromURDF + translaterobot (setup_pinocchio.py:28-32,73-75) and from the cube's
@@ -294,6 +303,8 @@ int gik_solve_launch_dims(gik_handle_t h, int elem_size, int64_t n, int32_t* blo
 /* Name of the kernel gik_solve_* launches for n problems with params.flags = flags (static string; "" on bad
  * arguments).  For reports: bench.py's roofline.kernel. */
 const char* gik_solve_kernel_name(gik_handle_t h, int elem_size, int64_t n, int flags);
+/* Number of kernels the entries have launched through this handle since gik_create, in *count. */
+int gik_launch_count(gik_handle_t h, int64_t* count);
 
 const char* gik_strerror(int code);
 const char* gik_version(void);

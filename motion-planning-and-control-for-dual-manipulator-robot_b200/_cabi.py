@@ -117,6 +117,7 @@ def lib() -> ctypes.CDLL:
     L.gik_solve_launch_dims.argtypes = [_P, ctypes.c_int, _I64, ctypes.POINTER(_I32), ctypes.POINTER(_I32)]
     L.gik_solve_kernel_name.argtypes = [_P, ctypes.c_int, _I64, ctypes.c_int]
     L.gik_solve_kernel_name.restype = ctypes.c_char_p
+    L.gik_launch_count.argtypes = [_P, ctypes.POINTER(_I64)]
     L.gik_strerror.argtypes = [ctypes.c_int]; L.gik_strerror.restype = ctypes.c_char_p
     L.gik_version.restype = ctypes.c_char_p
     _lib = L
@@ -134,7 +135,7 @@ EXPORTS = [
     "gik_tree_paths_f32", "gik_tree_paths_f64", "gik_path_shortcut_f32", "gik_path_shortcut_f64", "gik_traj_check_f32", "gik_traj_check_f64",
     "gik_traj_refine_f32", "gik_traj_refine_f64",
     "gik_flops_per_iter", "gik_flops_per_iter_executed", "gik_bytes_per_solve", "gik_measure_fma_peak", "gik_solve_launch_dims",
-    "gik_solve_kernel_name",
+    "gik_solve_kernel_name", "gik_launch_count",
     "gik_strerror", "gik_version",
 ]
 

@@ -79,24 +79,20 @@ namespace {
 template <typename T>
 int bezier_fit_api(gik_handle_t h, int64_t n_paths, int32_t n_points, int32_t dim, int32_t n_ctrl, const T* pinv, const T* basis,
                    const T* w0, const T* w1, const T* q0, const T* q1, const T* path, T* ctrl, T* cost, void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n_paths < 0 || n_points < 1 || dim < 1 || n_ctrl < 7) return GIK_E_SIZE;
-  if (n_paths == 0) return GIK_OK;
-  if (!pinv || !basis || !w0 || !w1 || !q0 || !q1 || !path || !ctrl || !cost) return GIK_E_NULL;
-  DeviceGuard g(h->device);
-  if (g.err != cudaSuccess) return (int)g.err;
   const int n_free = n_ctrl - 6;
   const size_t smem = sizeof(T) * ((size_t)2 * n_free * n_points + 2 * (size_t)n_points +
                                    (size_t)gik::kBezierWarps * (n_points + n_free) * dim);
   if (smem > 200 * 1024) return GIK_E_SIZE;
+  if (n_paths > 0 && (!pinv || !basis || !w0 || !w1 || !q0 || !q1 || !path || !ctrl || !cost)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
+  if (n_paths == 0) return GIK_OK;
+  DeviceGuard g(h->device);
+  if (g.err != cudaSuccess) return (int)g.err;
   cudaError_t e = cudaFuncSetAttribute(gik::gik_bezier_fit_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  int64_t blocks = (n_paths + gik::kBezierWarps - 1) / gik::kBezierWarps;
-  const int64_t cap = (int64_t)h->sm_count * 4;
-  if (blocks > cap) blocks = cap;
-  gik::gik_bezier_fit_kernel<T><<<(int)blocks, gik::kBezierWarps * 32, smem, (cudaStream_t)stream>>>(
-      n_paths, n_points, dim, n_ctrl, pinv, basis, w0, w1, q0, q1, path, ctrl, cost);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_bezier_fit_kernel<T>, capped_grid(h, n_paths, gik::kBezierWarps, 4), gik::kBezierWarps * 32, smem,
+                (cudaStream_t)stream, n_paths, n_points, dim, n_ctrl, pinv, basis, w0, w1, q0, q1, path, ctrl, cost);
 }
 
 }  // namespace

@@ -441,49 +441,43 @@ template <> gik::DevScene<double>* scene_of<double>(gik_scene_dev* sd) { return 
 struct DevPairList { const uint8_t *a, *b; int n; };
 DevPairList pair_list(const gik_scene_dev* sd, gik::PairList l) { return {sd->pairs[l][0], sd->pairs[l][1], sd->n_list[l]}; }
 
+// select: test only the columns listed in sel -- n_sel of them, or *n_sel_dev when that device-side count is given
 template <typename T>
 int collide_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, gik::PairList list, double margin, int invert,
-                uint8_t* out, void* stream, const int64_t* sel = nullptr, int64_t n_sel = 0,
+                uint8_t* out, void* stream, bool select = false, const int64_t* sel = nullptr, int64_t n_sel = 0,
                 const int64_t* n_sel_dev = nullptr) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
-  if (n < 0) return GIK_E_SIZE;
+  if (n < 0 || n_sel < 0) return GIK_E_SIZE;
   if (!(margin >= 0.0)) return GIK_E_PARAM;
+  if (select && !sel) return GIK_E_NULL;
+  const int64_t work = (select && !n_sel_dev) ? n_sel : n;     // device-side count: size the grid for the upper bound
+  const bool idle = n == 0 || work == 0;
+  if (!idle && (!out || (list == gik::kListCube ? !cube_pose : !q))) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (!h->scene) return GIK_E_NOSCENE;
-  if (n == 0 || (sel && !n_sel_dev && n_sel == 0)) return GIK_OK;
-  if (n_sel < 0) return GIK_E_SIZE;
-  const bool cube_only = list == gik::kListCube;
-  if (!out || (!cube_only && !q) || (cube_only && !cube_pose)) return GIK_E_NULL;
+  if (idle) return GIK_OK;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  const int64_t work = (sel && !n_sel_dev) ? n_sel : n;     // device-side count: size the grid for the upper bound
-  int64_t blocks = (work + gik::kCollideWarps - 1) / gik::kCollideWarps;
-  const int64_t cap = (int64_t)h->sm_count * 16;
-  if (blocks > cap) blocks = cap;
   const DevPairList pl = pair_list(h->scene, list);
-  gik::gik_collision_kernel<T><<<(int)blocks, gik::kCollideWarps * 32, 0, (cudaStream_t)stream>>>(
-      scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, q, cube_pose, (T)margin, out, invert, sel, n_sel, n_sel_dev);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_collision_kernel<T>, capped_grid(h, work, gik::kCollideWarps, 16), gik::kCollideWarps * 32, 0,
+                (cudaStream_t)stream, scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, q, cube_pose, (T)margin, out, invert,
+                sel, n_sel, n_sel_dev);
 }
 
 template <typename T>
 int distance_api(gik_handle_t h, int64_t n, const T* q, const T* cube_pose, gik::PairList list, double d_max, T* out,
                  void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0) return GIK_E_SIZE;
   if (!(d_max > 0.0)) return GIK_E_PARAM;
+  if (n > 0 && (!out || !q)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (!h->scene) return GIK_E_NOSCENE;
   if (n == 0) return GIK_OK;
-  if (!out || !q) return GIK_E_NULL;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  int64_t blocks = (n + gik::kCollideWarps - 1) / gik::kCollideWarps;
-  const int64_t cap = (int64_t)h->sm_count * 16;
-  if (blocks > cap) blocks = cap;
   const DevPairList pl = pair_list(h->scene, list);
   const int rounds = sizeof(T) == 4 ? 20 : 40;       // d_max / 2^rounds: below the arithmetic's own resolution
-  gik::gik_distance_kernel<T><<<(int)blocks, gik::kCollideWarps * 32, 0, (cudaStream_t)stream>>>(
-      scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, q, cube_pose, (T)d_max, rounds, out);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_distance_kernel<T>, capped_grid(h, n, gik::kCollideWarps, 16), gik::kCollideWarps * 32, 0,
+                (cudaStream_t)stream, scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, q, cube_pose, (T)d_max, rounds, out);
 }
 
 }  // namespace
@@ -524,11 +518,14 @@ static SuccessScratch carve_scratch(void* base, int64_t n, int nq, int esz) {
 template <typename T>
 int solve_success_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const gik_params_t* prm, T* q_out,
                       uint8_t* success, uint8_t* conv, int32_t* iters, T* resid, void* scratch, void* stream) {
+  if (n < 0) return GIK_E_SIZE;
+  if (int rc = check_params(prm)) return rc;
+  if (n > 0 && (!q_init || !pose || !q_out || !success || !conv || !iters || !resid || !scratch)) return GIK_E_NULL;
   if (bad_handle(h)) return GIK_E_HANDLE;
   if (!h->scene) return GIK_E_NOSCENE;
-  if (n > 0 && (!success || !conv || !scratch || !iters || !resid)) return GIK_E_NULL;
+  if (n == 0) return GIK_OK;
   int rc = solve_api<T>(h, n, q_init, pose, prm, q_out, conv, iters, resid, stream);
-  if (rc || n == 0) return rc;
+  if (rc) return rc;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
   cudaStream_t st = (cudaStream_t)stream;
@@ -539,15 +536,15 @@ int solve_success_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose,
   if (e == cudaSuccess) e = cudaMemsetAsync(sc.sel3, 0, sizeof(int64_t), st);
   if (e == cudaSuccess) e = cudaMemsetAsync(sc.queue, 0, 8 * 8, st);
   if (e != cudaSuccess) return (int)e;
-  int64_t blocks = (n + 255) / 256;
-  if (blocks > (int64_t)h->sm_count * 8) blocks = (int64_t)h->sm_count * 8;
-  gik::gik_compact_converged_kernel<<<(int)blocks, 256, 0, st>>>(n, conv, success, sc.sel1, sc.sel1 + 1);
-  if ((e = cudaGetLastError()) != cudaSuccess) return (int)e;
-  rc = collide_api<T>(h, n, q_out, pose, gik::kListAll, 0.0, 1, success, stream, sc.sel1 + 1, 0, sc.sel1);
+  const int blocks = capped_grid(h, n, 256, 8);
+  if ((rc = launch(h, gik::gik_compact_converged_kernel, blocks, 256, 0, st, n, conv, success, sc.sel1, sc.sel1 + 1)))
+    return rc;
+  rc = collide_api<T>(h, n, q_out, pose, gik::kListAll, 0.0, 1, success, stream, true, sc.sel1 + 1, 0, sc.sel1);
   if (rc || (prm->flags & GIK_F_NO_DESCEND)) return rc;
   // ---- the tail
-  gik::gik_compact_pending_kernel<<<(int)blocks, 256, 0, st>>>(n, conv, success, iters, prm->max_iters, sc.sel2, sc.sel2 + 1);
-  if ((e = cudaGetLastError()) != cudaSuccess) return (int)e;
+  if ((rc = launch(h, gik::gik_compact_pending_kernel, blocks, 256, 0, st, n, conv, success, iters, prm->max_iters, sc.sel2,
+                   sc.sel2 + 1)))
+    return rc;
   {
     SolveArgs<T> a{};
     a.q_init = q_out; a.pose = pose; a.iters = sc.iters_fin; a.resid = (T*)sc.resid_fin;
@@ -561,35 +558,28 @@ int solve_success_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose,
     if (rc) return rc;
   }
   const DevPairList pl = pair_list(h->scene, gik::kListAll);
-  int64_t tb = (n + gik::kCollideWarps - 1) / gik::kCollideWarps;
-  const int64_t cap = (int64_t)h->sm_count * 16;
-  if (tb > cap) tb = cap;
   const T safety = (T)1.5;
-  const bool wrist = use_wrist<T>(h, prm);
   const T eps2 = (T)(prm->eps * prm->eps);
   // queue[0] / queue[5]: work counters of the two stages; queue[1..4]: statistics
-  auto launch_tail = [&](auto kern, int64_t blocks_, const int64_t* list, unsigned long long* q_) {
-    kern<<<(int)blocks_, gik::kCollideWarps * 32, 0, st>>>(
-        table_of<T>(h), scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, list + 1, list, pose, (const T*)sc.q_fin,
-        (const T*)sc.resid_fin, q_out, success, conv, iters, resid, eps2, (T)prm->dt, (T)prm->damping, prm->max_iters, safety,
-        q_, sc.queue + 1, sc.sel3, sc.sel3 + 1);
+  auto launch_tail = [&](auto kern, int per_sm, const int64_t* list, unsigned long long* q_) {
+    return launch(h, kern, capped_grid(h, n, gik::kCollideWarps, per_sm), gik::kCollideWarps * 32, 0, st,
+                  table_of<T>(h), scene_of<T>(h->scene), pl.a, pl.b, pl.n, n, list + 1, list, pose, (const T*)sc.q_fin,
+                  (const T*)sc.resid_fin, q_out, success, conv, iters, resid, eps2, (T)prm->dt, (T)prm->damping,
+                  prm->max_iters, safety, q_, sc.queue + 1, sc.sel3, sc.sel3 + 1);
   };
-  const int64_t cap2 = (int64_t)h->sm_count * 2;
-  if (wrist) {
-    launch_tail(gik::gik_tail_kernel<T, true, 0>, tb, sc.sel2, sc.queue);
-    launch_tail(gik::gik_tail_kernel<T, true, 1>, tb < cap2 ? tb : cap2, sc.sel3, sc.queue + 5);
-  } else {
-    launch_tail(gik::gik_tail_kernel<T, false, 0>, tb, sc.sel2, sc.queue);
-    launch_tail(gik::gik_tail_kernel<T, false, 1>, tb < cap2 ? tb : cap2, sc.sel3, sc.queue + 5);
+  if (use_wrist<T>(h, prm)) {
+    if ((rc = launch_tail(gik::gik_tail_kernel<T, true, 0>, 16, sc.sel2, sc.queue))) return rc;
+    return launch_tail(gik::gik_tail_kernel<T, true, 1>, 2, sc.sel3, sc.queue + 5);
   }
-  return (int)cudaGetLastError();
+  if ((rc = launch_tail(gik::gik_tail_kernel<T, false, 0>, 16, sc.sel2, sc.queue))) return rc;
+  return launch_tail(gik::gik_tail_kernel<T, false, 1>, 2, sc.sel3, sc.queue + 5);
 }
 
 extern "C" {
 
 int gik_scene_attach(gik_handle_t h, const gik_scene_t* scene) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (!scene) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   int rc = gik::validate_scene(h->host, *scene);
   if (rc) return rc;
   DeviceGuard g(h->device);
@@ -623,12 +613,10 @@ int gik_scene_attach(gik_handle_t h, const gik_scene_t* scene) {
 int gik_collision_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, uint8_t* out, void* s) { return collide_api<float>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s); }
 int gik_collision_f64(gik_handle_t h, int64_t n, const double* q, const double* cube, uint8_t* out, void* s) { return collide_api<double>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s); }
 int gik_collision_sel_f32(gik_handle_t h, int64_t n, int64_t n_sel, const int64_t* sel, const float* q, const float* cube, uint8_t* out, void* s) {
-  if (!sel) return GIK_E_NULL;
-  return collide_api<float>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s, sel, n_sel);
+  return collide_api<float>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s, true, sel, n_sel);
 }
 int gik_collision_sel_f64(gik_handle_t h, int64_t n, int64_t n_sel, const int64_t* sel, const double* q, const double* cube, uint8_t* out, void* s) {
-  if (!sel) return GIK_E_NULL;
-  return collide_api<double>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s, sel, n_sel);
+  return collide_api<double>(h, n, q, cube, gik::kListAll, 0.0, 0, out, s, true, sel, n_sel);
 }
 int gik_solve_success_f32(gik_handle_t h, int64_t n, const float* q_init, const float* pose, const gik_params_t* p, float* q_out,
                           uint8_t* success, uint8_t* conv, int32_t* iters, float* resid, void* scratch, void* s) {
@@ -639,7 +627,7 @@ int gik_solve_success_f64(gik_handle_t h, int64_t n, const double* q_init, const
   return solve_success_api<double>(h, n, q_init, pose, p, q_out, success, conv, iters, resid, scratch, s);
 }
 size_t gik_solve_success_scratch_bytes(gik_handle_t h, int64_t n, int elem_size) {
-  if (bad_handle(h) || n < 0 || (elem_size != 4 && elem_size != 8)) return 0;
+  if (n < 0 || (elem_size != 4 && elem_size != 8) || bad_handle(h)) return 0;
   return carve_scratch(nullptr, n, h->host.nq, elem_size).bytes;
 }
 int gik_clearance_f32(gik_handle_t h, int64_t n, const float* q, const float* cube, double thr, uint8_t* out, void* s) { return collide_api<float>(h, n, q, cube, gik::kListEnv, thr, 1, out, s); }

@@ -13,6 +13,8 @@
 #include <stdlib.h>
 #include <atomic>
 #include <new>
+#include <type_traits>
+#include <utility>
 
 #include "gik_table.h"
 
@@ -1066,6 +1068,7 @@ struct gik_handle_s {
   struct gik_scene_dev* scene;       // collision scene (gik_scene_attach), or null
   unsigned long long* queues;        // device: kQueueSlots work-queue heads, one per launch in flight
   std::atomic<uint32_t> next_queue;
+  std::atomic<int64_t> launches;     // kernels launched through this handle (gik_launch_count)
 };
 static constexpr uint32_t kQueueSlots = 1024;   // launches that may be in flight on one handle at once
 static constexpr uint32_t kMagic = 0x67696b31u;  // "gik1"
@@ -1085,6 +1088,22 @@ struct DeviceGuard {
     if (prev >= 0 && cudaGetDevice(&cur) == cudaSuccess && cur != prev) cudaSetDevice(prev);
   }
 };
+
+// Every kernel launch of the C ABI goes through here (gik_measure_fma_peak, which has no handle, aside): the launch is
+// counted on the handle for gik_launch_count, and its error returned.
+template <typename... P, typename... A>
+int launch(gik_handle_t h, void (*kern)(P...), int blocks, int threads, size_t smem, cudaStream_t st, A&&... args) {
+  kern<<<blocks, threads, smem, st>>>(std::forward<A>(args)...);
+  const cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) h->launches.fetch_add(1, std::memory_order_relaxed);
+  return (int)e;
+}
+
+// Grid of a launch over `work` items, `per_block` items per block, at most `per_sm` blocks per SM
+inline int capped_grid(gik_handle_t h, int64_t work, int per_block, int per_sm) {
+  const int64_t blocks = (work + per_block - 1) / per_block, most = (int64_t)h->sm_count * per_sm;
+  return (int)(blocks < most ? blocks : most);
+}
 
 inline bool bad_handle(gik_handle_t h) { return h == nullptr || h->magic != kMagic; }
 
@@ -1190,15 +1209,6 @@ int choose_launch(gik_handle_t h, int64_t n, int flags, bool wrist, int reserve,
   return with_kernel<T, MODE>(*k, [&](auto kern) { return grid_dims(h, kern, n, 16, blocks, per_warp, nullptr, reserve); });
 }
 
-template <typename T>
-void launch_kernel(void (*kern)(DevTable<T>, SolveArgs<T>), int blocks, cudaStream_t st, gik_handle_t h, const SolveArgs<T>& a) {
-  kern<<<blocks, kThreads, 0, st>>>(table_of<T>(h), a);
-}
-void launch_kernel(void (*kern)(DevTable<float>, PackedTable, SolveArgs<float>), int blocks, cudaStream_t st, gik_handle_t h,
-                   const SolveArgs<float>& a) {
-  kern<<<blocks, kThreads, 0, st>>>(h->tab32, h->pt32, a);
-}
-
 // force: a continuation launch that must run every problem to the iteration cap -- eps^2 = 0 can never be undercut
 template <typename T, int MODE>
 int launch_solve(gik_handle_t h, SolveArgs<T>& a, const gik_params_t* prm, void* stream, bool force = false) {
@@ -1228,8 +1238,10 @@ int launch_solve(gik_handle_t h, SolveArgs<T>& a, const gik_params_t* prm, void*
   cudaError_t qe = cudaMemsetAsync(a.queue, 0, sizeof(unsigned long long), (cudaStream_t)stream);
   if (qe != cudaSuccess) return (int)qe;
   return with_kernel<T, MODE>(k, [&](auto kern) {
-    launch_kernel(kern, blocks, (cudaStream_t)stream, h, a);
-    return (int)cudaGetLastError();
+    if constexpr (std::is_same_v<decltype(kern), void (*)(DevTable<float>, PackedTable, SolveArgs<float>)>)   // packed fp32
+      return launch(h, kern, blocks, kThreads, 0, (cudaStream_t)stream, h->tab32, h->pt32, a);
+    else
+      return launch(h, kern, blocks, kThreads, 0, (cudaStream_t)stream, table_of<T>(h), a);
   });
 }
 
@@ -1260,12 +1272,11 @@ void set_soa(SolveArgs<T>& a, int64_t n_in, int64_t n_out) {
 template <typename T>
 int rows_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const gik_params_t* prm, T* q_out, uint8_t* conv,
              int32_t* iters, T* resid, const unsigned long long* ready, void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0) return GIK_E_SIZE;
-  int rc = check_params(prm);
-  if (rc) return rc;
+  if (int rc = check_params(prm)) return rc;
+  if (n > 0 && (!q_init || !pose || !q_out || !conv)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n == 0) return GIK_OK;
-  if (!q_init || !pose || !q_out || !conv) return GIK_E_NULL;
   SolveArgs<T> a{};
   a.q_init = q_init; a.pose = pose; a.iters = iters; a.resid = resid;
   a.q_dst[0] = q_out; a.conv_dst[0] = conv; a.n_dst = 1; a.out_off = 0;
@@ -1280,12 +1291,11 @@ int rows_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const gi
 template <typename T>
 int solve_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const gik_params_t* prm, T* q_out,
               uint8_t* conv, int32_t* iters, T* resid, void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0) return GIK_E_SIZE;
-  int rc = check_params(prm);
-  if (rc) return rc;
+  if (int rc = check_params(prm)) return rc;
+  if (n > 0 && (!q_init || !pose || !q_out || !conv)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n == 0) return GIK_OK;
-  if (!q_init || !pose || !q_out || !conv) return GIK_E_NULL;
   SolveArgs<T> a{};
   a.q_init = q_init; a.pose = pose; a.iters = iters; a.resid = resid;
   a.q_dst[0] = q_out; a.conv_dst[0] = conv; a.n_dst = 1; a.out_off = 0;
@@ -1298,14 +1308,16 @@ template <typename T>
 int scatter_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const gik_params_t* prm, int32_t n_peers,
                 T* const* q_all, uint8_t* const* conv_all, int64_t n_total, int64_t offset, int32_t* iters, T* resid,
                 void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0 || n_peers < 1 || n_peers > GIK_MAX_PEERS || offset < 0 || n_total < 0 || offset + n > n_total) return GIK_E_SIZE;
   int rc = check_params(prm);
   if (rc) return rc;
+  if (n > 0) {
+    if (!q_init || !pose || !q_all || !conv_all) return GIK_E_NULL;
+    for (int p = 0; p < n_peers; ++p)
+      if (!q_all[p] || !conv_all[p]) return GIK_E_NULL;
+  }
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n == 0) return GIK_OK;
-  if (!q_init || !pose || !q_all || !conv_all) return GIK_E_NULL;
-  for (int p = 0; p < n_peers; ++p)
-    if (!q_all[p] || !conv_all[p]) return GIK_E_NULL;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
   // The lanes store into ONE array -- this rank's own, i.e. the one whose memory lives on this device -- and the chunk
@@ -1350,10 +1362,7 @@ int scatter_api(gik_handle_t h, int64_t n, const T* q_init, const T* pose, const
   }
   rc = launch_solve<T, MODE_BATCH>(h, a, prm, stream);
   if (stats) cudaEventRecord(ev[1], st);
-  if (rc == GIK_OK) {
-    gik_push_rest_kernel<T><<<h->sm_count * 4, 128, 0, st>>>(a, h->host.nq, stats ? 2 : 0);
-    rc = (int)cudaGetLastError();
-  }
+  if (rc == GIK_OK) rc = launch(h, gik_push_rest_kernel<T>, h->sm_count * 4, 128, 0, st, a, h->host.nq, stats ? 2 : 0);
   if (stats) {
     cudaEventRecord(ev[2], st);
     uint8_t* hp = (uint8_t*)malloc((size_t)n_chunks);
@@ -1430,12 +1439,11 @@ template <typename T>
 int edges_api(gik_handle_t h, int64_t n, int32_t max_steps, const T* q_start, const T* pose_a, const T* pose_b,
               const int32_t* num_steps, const gik_params_t* prm, T* q_path, int32_t* n_valid,
               int32_t* iters_total, void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0 || max_steps < 0) return GIK_E_SIZE;
-  int rc = check_params(prm);
-  if (rc) return rc;
+  if (int rc = check_params(prm)) return rc;
+  if (n > 0 && (!q_start || !pose_a || !pose_b || !num_steps || !q_path || !n_valid)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n == 0) return GIK_OK;
-  if (!q_start || !pose_a || !pose_b || !num_steps || !q_path || !n_valid) return GIK_E_NULL;
   SolveArgs<T> a{};
   a.q_init = q_start; a.pose = pose_a; a.pose_b = pose_b; a.num_steps = num_steps; a.q_out = q_path;
   a.n_valid = n_valid; a.iters = iters_total; a.max_steps = max_steps; a.n = n;
@@ -1445,33 +1453,27 @@ int edges_api(gik_handle_t h, int64_t n, int32_t max_steps, const T* q_start, co
 
 template <typename T>
 int fk_api(gik_handle_t h, int64_t n, const T* q, T* frames, void* stream, bool jac) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n < 0) return GIK_E_SIZE;
+  if (n > 0 && (!q || !frames)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n == 0) return GIK_OK;
-  if (!q || !frames) return GIK_E_NULL;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  int64_t blocks = (n + 127) / 128;
-  if (blocks > (int64_t)h->sm_count * 16) blocks = (int64_t)h->sm_count * 16;
-  if (jac) gik_jac_kernel<T><<<(int)blocks, 128, 0, (cudaStream_t)stream>>>(table_of<T>(h), n, q, frames);
-  else gik_fk_kernel<T><<<(int)blocks, 128, 0, (cudaStream_t)stream>>>(table_of<T>(h), n, q, frames);
-  return (int)cudaGetLastError();
+  return launch(h, jac ? gik_jac_kernel<T> : gik_fk_kernel<T>, capped_grid(h, n, 128, 16), 128, 0, (cudaStream_t)stream,
+                table_of<T>(h), n, q, frames);
 }
 
 template <typename T>
 int best_of_api(gik_handle_t h, int64_t n_place, int32_t n_restart, const T* q, const uint8_t* conv,
                 const T* resid, T* q_best, uint8_t* conv_best, int32_t* which, void* stream) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n_place < 0 || n_restart < 1) return GIK_E_SIZE;
+  if (n_place > 0 && (!q || !conv || !resid || !q_best || !conv_best)) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   if (n_place == 0) return GIK_OK;
-  if (!q || !conv || !resid || !q_best || !conv_best) return GIK_E_NULL;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  int64_t blocks = (n_place + 3) / 4;
-  if (blocks > (int64_t)h->sm_count * 16) blocks = (int64_t)h->sm_count * 16;
-  gik_best_of_kernel<T><<<(int)blocks, 128, 0, (cudaStream_t)stream>>>(h->host.nq, n_place, n_restart, q, conv,
-                                                                       resid, q_best, conv_best, which);
-  return (int)cudaGetLastError();
+  return launch(h, gik_best_of_kernel<T>, capped_grid(h, n_place, 4, 16), 128, 0, (cudaStream_t)stream, h->host.nq, n_place,
+                n_restart, q, conv, resid, q_best, conv_best, which);
 }
 
 template <typename T>
@@ -1536,6 +1538,7 @@ int gik_create(const gik_table_t* host_table, int device, gik_handle_t* out) {
     if (g.err != cudaSuccess) { delete h; return (int)g.err; }
   }
   h->next_queue.store(0);
+  h->launches.store(0);
   h->scene = nullptr;
   h->magic = kMagic;
   *out = h;
@@ -1636,10 +1639,10 @@ int gik_measure_fma_peak(int device, int elem_size, int repeats, double* tflops)
 }
 
 int gik_solve_launch_dims(gik_handle_t h, int elem_size, int64_t n, int32_t* blocks, int32_t* threads) {
-  if (bad_handle(h)) return GIK_E_HANDLE;
-  if (!blocks || !threads) return GIK_E_NULL;
   if (n < 0) return GIK_E_SIZE;
   if (elem_size != 4 && elem_size != 8) return GIK_E_PARAM;
+  if (!blocks || !threads) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
   SolveKernel k;
   int b = 0;
   const int rc = batch_launch(h, elem_size, n, 0, &k, &b);
@@ -1648,8 +1651,15 @@ int gik_solve_launch_dims(gik_handle_t h, int elem_size, int64_t n, int32_t* blo
   return GIK_OK;
 }
 
+int gik_launch_count(gik_handle_t h, int64_t* count) {
+  if (!count) return GIK_E_NULL;
+  if (bad_handle(h)) return GIK_E_HANDLE;
+  *count = h->launches.load(std::memory_order_relaxed);
+  return GIK_OK;
+}
+
 const char* gik_solve_kernel_name(gik_handle_t h, int elem_size, int64_t n, int flags) {
-  if (bad_handle(h) || n < 0 || (elem_size != 4 && elem_size != 8)) return "";
+  if (n < 0 || (elem_size != 4 && elem_size != 8) || bad_handle(h)) return "";
   SolveKernel k;
   int b = 0;
   if (batch_launch(h, elem_size, n, flags, &k, &b)) return "";

@@ -196,7 +196,6 @@ gik_path_shortcut_write_kernel(int nq, int64_t Q, int K, const int64_t* __restri
 #if defined(__CUDACC__)
 namespace {
 
-// Argument checks come before the handle check and before any CUDA call (sizes, parameters, pointers, then the handle).
 template <typename T>
 int path_shortcut_api(gik_handle_t h, int64_t n_paths, int32_t n_cand, int32_t max_steps, const int64_t* offsets,
                       const T* q, const T* cube, const int32_t* pair_i, const int32_t* pair_j, const int32_t* num_steps,
@@ -212,21 +211,16 @@ int path_shortcut_api(gik_handle_t h, int64_t n_paths, int32_t n_cand, int32_t m
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
   cudaStream_t st = (cudaStream_t)stream;
-  int64_t blocks = (n_paths + gik::kShortcutWarps - 1) / gik::kShortcutWarps;
-  const int64_t most = (int64_t)h->sm_count * 16;
-  if (blocks > most) blocks = most;
+  const int blocks = capped_grid(h, n_paths, gik::kShortcutWarps, 16);
   if (!q_out) {
-    gik::gik_path_shortcut_select_kernel<T><<<(int)blocks, gik::kShortcutWarps * 32, 0, st>>>(
-        h->host.nq, n_paths, n_cand, max_steps, offsets, q, pair_i, pair_j, num_steps, n_valid, q_path, join_tol, chosen,
-        length, offsets_out);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    gik::gik_tree_scan_kernel<<<1, gik::kScanThreads, 0, st>>>(n_paths, offsets_out);
-    return (int)cudaGetLastError();
+    if (int rc = launch(h, gik::gik_path_shortcut_select_kernel<T>, blocks, gik::kShortcutWarps * 32, 0, st, h->host.nq,
+                        n_paths, n_cand, max_steps, offsets, q, pair_i, pair_j, num_steps, n_valid, q_path, join_tol, chosen,
+                        length, offsets_out))
+      return rc;
+    return launch(h, gik::gik_tree_scan_kernel, 1, gik::kScanThreads, 0, st, n_paths, offsets_out);
   }
-  gik::gik_path_shortcut_write_kernel<T><<<(int)blocks, gik::kShortcutWarps * 32, 0, st>>>(
-      h->host.nq, n_paths, n_cand, offsets, q, cube, pair_i, pair_j, num_steps, q_path, chosen, offsets_out, q_out, cube_out);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_path_shortcut_write_kernel<T>, blocks, gik::kShortcutWarps * 32, 0, st, h->host.nq, n_paths, n_cand,
+                offsets, q, cube, pair_i, pair_j, num_steps, q_path, chosen, offsets_out, q_out, cube_out);
 }
 
 }  // namespace

@@ -181,7 +181,6 @@ gik_traj_check_kernel(const __grid_constant__ TrajConst<T> tc, const DevScene<T>
 #if defined(__CUDACC__)
 namespace {
 
-// Sizes, tolerances and pointers are checked before the handle and before any CUDA call.
 template <typename T>
 int traj_check_api(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_samples, const T* weights, const T* ctrl,
                    double limit_tol, double grasp_tol, uint8_t* valid, int32_t* first_bad, uint8_t* reason, T* grasp_err,
@@ -198,21 +197,14 @@ int traj_check_api(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_sam
   cudaStream_t st = (cudaStream_t)stream;
   gik::TrajConst<T> tc;
   gik::fill_traj_const(h->host, limit_tol, tc);
-  int64_t rb = (n_traj + 255) / 256;
-  if (rb > (int64_t)h->sm_count * 8) rb = (int64_t)h->sm_count * 8;
-  gik::gik_traj_init_kernel<T><<<(int)rb, 256, 0, st>>>(n_traj, first_bad, grasp_err);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return (int)e;
-  const int64_t total = n_traj * n_samples;
-  int64_t blocks = (total + gik::kTrajWarps - 1) / gik::kTrajWarps;
-  if (blocks > (int64_t)h->sm_count * 16) blocks = (int64_t)h->sm_count * 16;
+  const int rb = capped_grid(h, n_traj, 256, 8);
+  if (int rc = launch(h, gik::gik_traj_init_kernel<T>, rb, 256, 0, st, n_traj, first_bad, grasp_err)) return rc;
   const DevPairList pl = pair_list(h->scene, gik::kListTraj);
-  gik::gik_traj_check_kernel<T><<<(int)blocks, gik::kTrajWarps * 32, 0, st>>>(
-      tc, scene_of<T>(h->scene), pl.a, pl.b, pl.n, n_traj, n_ctrl, n_samples, weights, ctrl,
-      (T)grasp_tol, first_bad, grasp_err, sample_flags);
-  if ((e = cudaGetLastError()) != cudaSuccess) return (int)e;
-  gik::gik_traj_finish_kernel<<<(int)rb, 256, 0, st>>>(n_traj, first_bad, valid, reason);
-  return (int)cudaGetLastError();
+  if (int rc = launch(h, gik::gik_traj_check_kernel<T>, capped_grid(h, n_traj * n_samples, gik::kTrajWarps, 16),
+                      gik::kTrajWarps * 32, 0, st, tc, scene_of<T>(h->scene), pl.a, pl.b, pl.n, n_traj, n_ctrl, n_samples,
+                      weights, ctrl, (T)grasp_tol, first_bad, grasp_err, sample_flags))
+    return rc;
+  return launch(h, gik::gik_traj_finish_kernel, rb, 256, 0, st, n_traj, first_bad, valid, reason);
 }
 
 }  // namespace

@@ -371,7 +371,6 @@ gik_traj_refine_kernel(const __grid_constant__ DevTable<T> tab, const __grid_con
 #if defined(__CUDACC__)
 namespace {
 
-// Sizes, parameters and pointers are checked before the handle and before any CUDA call.
 template <typename T>
 int traj_refine_api(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_samples, const T* weights, const T* ctrl,
                     int32_t max_iters, double tol, double damping, T* ctrl_out, double* obj_before, double* obj_after,
@@ -393,12 +392,10 @@ int traj_refine_api(gik_handle_t h, int64_t n_traj, int32_t n_ctrl, int32_t n_sa
   int occ = 0;
   e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, gik::kRefineThreads, smem);
   if (e != cudaSuccess) return (int)e;
-  int64_t blocks = (int64_t)h->sm_count * (occ > 0 ? occ : 1);
-  if (blocks > n_traj) blocks = n_traj;
   gik::RefineArgs<T> a{n_traj, n_ctrl, n_samples, max_iters, tol, damping, weights, ctrl, ctrl_out, obj_before,
                        obj_after, grasp_err, iters, accepted};
-  kern<<<(int)blocks, gik::kRefineThreads, smem, (cudaStream_t)stream>>>(table_of<T>(h), a);
-  return (int)cudaGetLastError();
+  return launch(h, kern, capped_grid(h, n_traj, 1, occ > 0 ? occ : 1), gik::kRefineThreads, smem, (cudaStream_t)stream,
+                table_of<T>(h), a);
 }
 
 }  // namespace

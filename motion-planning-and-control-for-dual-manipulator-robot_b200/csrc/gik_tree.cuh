@@ -253,7 +253,6 @@ gik_tree_path_write_kernel(int nq, int64_t Q, int64_t cap, const T* verts, const
 #if defined(__CUDACC__)
 namespace {
 
-// Argument checks come before the handle check and before any CUDA call (sizes, then pointers, then the handle).
 inline int tree_blocks(int64_t n, int per_block) { return (int)((n + per_block - 1) / per_block); }
 
 template <typename T>
@@ -265,12 +264,8 @@ int tree_nearest_api(gik_handle_t h, int64_t n_trees, int32_t cap, const T* vert
   if (n_targets == 0) return GIK_OK;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  int64_t blocks = (n_targets + gik::kTreeWarps - 1) / gik::kTreeWarps;
-  const int64_t most = (int64_t)h->sm_count * 16;
-  if (blocks > most) blocks = most;
-  gik::gik_tree_nearest_kernel<T><<<(int)blocks, gik::kTreeWarps * 32, 0, (cudaStream_t)stream>>>(
-      h->host.nq, n_trees, cap, verts, n_verts, n_targets, targets, target_tree, nearest);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_tree_nearest_kernel<T>, capped_grid(h, n_targets, gik::kTreeWarps, 16), gik::kTreeWarps * 32, 0,
+                (cudaStream_t)stream, h->host.nq, n_trees, cap, verts, n_verts, n_targets, targets, target_tree, nearest);
 }
 
 template <typename T>
@@ -286,10 +281,9 @@ int tree_grow_api(gik_handle_t h, int64_t n_trees, int32_t cap, T* verts, T* cub
   if (n_edges == 0) return GIK_OK;
   DeviceGuard g(h->device);
   if (g.err != cudaSuccess) return (int)g.err;
-  gik::gik_tree_grow_kernel<T><<<tree_blocks(n_edges, 128), 128, 0, (cudaStream_t)stream>>>(
-      h->host.nq, n_trees, cap, max_steps, verts, cubes, parent, n_verts, overflow, n_edges, edge_tree, near, q_start, pose_a,
-      pose_b, num_steps, n_valid, q_path, seg_end);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_tree_grow_kernel<T>, tree_blocks(n_edges, 128), 128, 0, (cudaStream_t)stream, h->host.nq, n_trees,
+                cap, max_steps, verts, cubes, parent, n_verts, overflow, n_edges, edge_tree, near, q_start, pose_a, pose_b,
+                num_steps, n_valid, q_path, seg_end);
 }
 
 template <typename T>
@@ -306,15 +300,13 @@ int tree_paths_api(gik_handle_t h, int64_t n_queries, int32_t cap, const T* vert
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = tree_blocks(n_queries, 128);
   if (!q) {
-    gik::gik_tree_path_len_kernel<<<blocks, 128, 0, st>>>(n_queries, cap, parent, n_verts, start_end, goal_end, offsets);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (int)e;
-    gik::gik_tree_scan_kernel<<<1, gik::kScanThreads, 0, st>>>(n_queries, offsets);
-    return (int)cudaGetLastError();
+    if (int rc = launch(h, gik::gik_tree_path_len_kernel, blocks, 128, 0, st, n_queries, cap, parent, n_verts, start_end,
+                        goal_end, offsets))
+      return rc;
+    return launch(h, gik::gik_tree_scan_kernel, 1, gik::kScanThreads, 0, st, n_queries, offsets);
   }
-  gik::gik_tree_path_write_kernel<T><<<blocks, 128, 0, st>>>(h->host.nq, n_queries, cap, verts, cubes, parent, n_verts,
-                                                              start_end, goal_end, offsets, q, cube);
-  return (int)cudaGetLastError();
+  return launch(h, gik::gik_tree_path_write_kernel<T>, blocks, 128, 0, st, h->host.nq, n_queries, cap, verts, cubes, parent,
+                n_verts, start_end, goal_end, offsets, q, cube);
 }
 
 }  // namespace

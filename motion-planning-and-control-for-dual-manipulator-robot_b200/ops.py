@@ -78,7 +78,6 @@ class GraspIK:
         ct = self.table.to_c()
         _cabi.check(self._lib.gik_create(ctypes.byref(ct), self.device.index, ctypes.byref(self._h)), "gik_create")
         self.nq = self.table.nq
-        self.launches = 0   # kernels of this library launched through this handle
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -94,6 +93,42 @@ class GraspIK:
     # ------------------------------------------------------------------ helpers
     def _stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    @property
+    def launches(self) -> int:
+        """Kernels of this library launched through this handle (gik_launch_count)."""
+        count = ctypes.c_int64()
+        _cabi.check(self._lib.gik_launch_count(self._h, ctypes.byref(count)), "gik_launch_count")
+        return count.value
+
+    def _call(self, entry: str, dtype, *args):
+        """Call gik_<entry>_f32 / _f64 (chosen by dtype) with the handle first and the current stream last; raise on an
+        error code."""
+        f = getattr(self._lib, f"gik_{entry}_{_sfx(dtype)}")
+        _cabi.check(f(self._h, *args, self._stream()), f"gik_{entry}")
+
+    def _arg(self, t, shape, dtype, name, *, copy=False) -> torch.Tensor:
+        """A tensor handed to an entry: on this handle's device, of `dtype`, exactly `shape` (None: any size) and
+        contiguous -- or, with `copy`, made contiguous.  TypeError for the dtype, ValueError otherwise."""
+        if not torch.is_tensor(t) or not t.is_cuda or t.device != self.device:
+            raise ValueError(f"{name}: expected a tensor on {self.device}, got {getattr(t, 'device', type(t).__name__)}")
+        if t.dtype != dtype:
+            raise TypeError(f"{name}: expected {dtype}, got {t.dtype}")
+        if t.dim() != len(shape) or any(s is not None and s != d for s, d in zip(shape, t.shape)):
+            want = "[" + "][".join("*" if s is None else str(s) for s in shape) + "]"
+            raise ValueError(f"{name}: expected shape {want}, got {list(t.shape)}")
+        if not t.is_contiguous():
+            if not copy:
+                raise ValueError(f"{name} must be contiguous")
+            t = t.contiguous()
+        return t
+
+    def _q_cube(self, q_soa, cube_pose_soa):
+        """q [nq][n] and the optional cube_pose [12][n] (converted to q's dtype) of the collision entries."""
+        q = self._arg(q_soa, (self.nq, None), q_soa.dtype, "q", copy=True)
+        if cube_pose_soa is None:
+            return q, None
+        return q, self._arg(cube_pose_soa.to(q.dtype), (12, q.shape[1]), q.dtype, "cube_pose", copy=True)
 
     # GIK_F_LANE_KERNEL / GIK_F_PAIR_KERNEL / GIK_F_SCALAR_LANE (fp32: "lane" = packed FFMA2 kernel, "lane1" = scalar)
     _KERNEL_FLAGS = {None: 0, "auto": 0, "lane": 2, "pair": 4, "lane1": 2 | 8}
@@ -118,11 +153,6 @@ class GraspIK:
         flags = self._params(1e-3, 1e-2, 1, 0.0, kernel).flags
         return self._lib.gik_solve_kernel_name(self._h, esz, int(n), flags).decode()
 
-    def _chk_dev(self, *ts):
-        for t in ts:
-            if t is not None and (not t.is_cuda or t.device != self.device):
-                raise ValueError(f"tensor on {t.device}, handle on {self.device}")
-
     @staticmethod
     def _ptr(t):
         return ctypes.c_void_p(0 if t is None else t.data_ptr())
@@ -134,22 +164,16 @@ class GraspIK:
     # ------------------------------------------------------------------ SoA entry points (no copies)
     def fk_soa(self, q_soa: torch.Tensor) -> torch.Tensor:
         """q [nq][n] -> frames [2][12][n]  (gik_fk_*)."""
-        self._chk_dev(q_soa)
-        n = q_soa.shape[1]
-        out = torch.empty((2, 12, n), dtype=q_soa.dtype, device=self.device)
-        f = getattr(self._lib, f"gik_fk_{_sfx(q_soa.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(q_soa.contiguous()), self._ptr(out), self._stream()), "gik_fk")
-        self.launches += 1
+        q = self._arg(q_soa, (self.nq, None), q_soa.dtype, "q", copy=True)
+        out = torch.empty((2, 12, q.shape[1]), dtype=q.dtype, device=self.device)
+        self._call("fk", q.dtype, q.shape[1], self._ptr(q), self._ptr(out))
         return out
 
     def jac_soa(self, q_soa: torch.Tensor) -> torch.Tensor:
         """q [nq][n] -> jac [2][6][nq][n]  (gik_jac_*)."""
-        self._chk_dev(q_soa)
-        n = q_soa.shape[1]
-        out = torch.empty((2, 6, self.nq, n), dtype=q_soa.dtype, device=self.device)
-        f = getattr(self._lib, f"gik_jac_{_sfx(q_soa.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(q_soa.contiguous()), self._ptr(out), self._stream()), "gik_jac")
-        self.launches += 1
+        q = self._arg(q_soa, (self.nq, None), q_soa.dtype, "q", copy=True)
+        out = torch.empty((2, 6, self.nq, q.shape[1]), dtype=q.dtype, device=self.device)
+        self._call("jac", q.dtype, q.shape[1], self._ptr(q), self._ptr(out))
         return out
 
     def solve_soa(self, q_init: torch.Tensor, pose: torch.Tensor, *, eps=EPSILON, dt=DT, max_iters=MAX_ITERS,
@@ -159,27 +183,24 @@ class GraspIK:
         `kernel`: None = launcher's choice by batch size, "lane" / "pair" force a thread mapping (same results).
         `early_stop`: fast preset (GIK_F_EARLY_STOP) -- stalled problems are abandoned early; flags and converged q
         are unchanged, the q / iters of FAILED problems are not the reference's."""
-        self._chk_dev(q_init, pose)
-        if q_init.dtype != pose.dtype:
-            raise TypeError("q_init and pose must share a dtype")
-        if not (q_init.is_contiguous() and pose.is_contiguous()):
-            raise ValueError("SoA inputs must be contiguous")
+        ft = q_init.dtype
+        q_init = self._arg(q_init, (self.nq, None), ft, "q_init")
         n = q_init.shape[1]
-        if q_init.shape[0] != self.nq or pose.shape != (12, n):
-            raise ValueError(f"expected q_init [{self.nq}][n] and pose [12][n], got {tuple(q_init.shape)}, {tuple(pose.shape)}")
+        pose = self._arg(pose, (12, n), ft, "pose")
         if out is None:
             q = torch.empty_like(q_init)
             conv = torch.empty((n,), dtype=torch.uint8, device=self.device)
             iters = torch.empty((n,), dtype=torch.int32, device=self.device)
-            resid = torch.empty((2, n), dtype=q_init.dtype, device=self.device)
+            resid = torch.empty((2, n), dtype=ft, device=self.device)
         else:
             q, conv, iters, resid = out
+            self._arg(q, (self.nq, n), ft, "out q")
+            self._arg(conv, (n,), torch.uint8, "out converged")
+            self._arg(iters, (n,), torch.int32, "out iters")
+            self._arg(resid, (2, n), ft, "out resid")
         prm = self._params(eps, dt, max_iters, damping, kernel, early_stop)
-        f = getattr(self._lib, f"gik_solve_{_sfx(q_init.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(q_init), self._ptr(pose), ctypes.byref(prm), self._ptr(q),
-                      self._ptr(conv), self._ptr(iters), self._ptr(resid), self._stream()), "gik_solve")
-        if n:
-            self.launches += 1
+        self._call("solve", ft, n, self._ptr(q_init), self._ptr(pose), ctypes.byref(prm), self._ptr(q), self._ptr(conv),
+                   self._ptr(iters), self._ptr(resid))
         return q, conv, iters, resid
 
     def solve_scatter_soa(self, q_init: torch.Tensor, pose: torch.Tensor, q_ptrs, conv_ptrs, n_total: int, offset: int,
@@ -188,64 +209,62 @@ class GraspIK:
         result arrays of ALL ranks.  `q_ptrs` / `conv_ptrs`: device addresses (ints) of each rank's [nq][n_total] q
         array and [n_total] flag array as mapped on THIS device (see dist.SymmetricResults).  Returns the local
         (iters [n], resid [2][n]); the caller runs the cross-rank barrier."""
-        self._chk_dev(q_init, pose)
-        if not (q_init.is_contiguous() and pose.is_contiguous()) or q_init.dtype != pose.dtype:
-            raise ValueError("SoA inputs must be contiguous and share a dtype")
+        ft = q_init.dtype
+        q_init = self._arg(q_init, (self.nq, None), ft, "q_init")
         n = q_init.shape[1]
-        if q_init.shape[0] != self.nq or pose.shape != (12, n):
-            raise ValueError("expected q_init [nq][n] and pose [12][n]")
+        pose = self._arg(pose, (12, n), ft, "pose")
         if len(q_ptrs) != len(conv_ptrs) or not q_ptrs:
             raise ValueError("need one q and one flag pointer per rank")
         if out is None:
             iters = torch.empty((n,), dtype=torch.int32, device=self.device)
-            resid = torch.empty((2, n), dtype=q_init.dtype, device=self.device)
+            resid = torch.empty((2, n), dtype=ft, device=self.device)
         else:
             iters, resid = out
+            self._arg(iters, (n,), torch.int32, "out iters")
+            self._arg(resid, (2, n), ft, "out resid")
         P = len(q_ptrs)
         qa = (ctypes.c_void_p * P)(*[int(p) for p in q_ptrs])
         ca = (ctypes.c_void_p * P)(*[int(p) for p in conv_ptrs])
         prm = self._params(eps, dt, max_iters, damping, kernel)
-        f = getattr(self._lib, f"gik_solve_scatter_{_sfx(q_init.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(q_init), self._ptr(pose), ctypes.byref(prm), P, qa, ca, int(n_total),
-                      int(offset), self._ptr(iters), self._ptr(resid), self._stream()), "gik_solve_scatter")
-        if n:
-            self.launches += 2 if P > 1 else 1          # solve kernel (+ its pusher blocks) and the tail kernel
+        self._call("solve_scatter", ft, n, self._ptr(q_init), self._ptr(pose), ctypes.byref(prm), P, qa, ca, int(n_total),
+                   int(offset), self._ptr(iters), self._ptr(resid))
         return iters, resid
 
     def best_of_soa(self, q, conv, resid, n_place: int, n_restart: int):
         """Problem (p, r) at column p * n_restart + r.  -> (q_best [nq][n_place], conv u8, which i32)."""
-        self._chk_dev(q, conv, resid)
+        N = n_place * n_restart
+        q = self._arg(q, (self.nq, N), q.dtype, "q", copy=True)
+        conv = self._arg(conv, (N,), torch.uint8, "converged", copy=True)
+        resid = self._arg(resid, (2, N), q.dtype, "resid", copy=True)
         qb = torch.empty((self.nq, n_place), dtype=q.dtype, device=self.device)
         cb = torch.empty((n_place,), dtype=torch.uint8, device=self.device)
         wh = torch.empty((n_place,), dtype=torch.int32, device=self.device)
-        f = getattr(self._lib, f"gik_best_of_{_sfx(q.dtype)}")
-        _cabi.check(f(self._h, n_place, n_restart, self._ptr(q), self._ptr(conv), self._ptr(resid), self._ptr(qb),
-                      self._ptr(cb), self._ptr(wh), self._stream()), "gik_best_of")
-        if n_place:
-            self.launches += 1
+        self._call("best_of", q.dtype, n_place, n_restart, self._ptr(q), self._ptr(conv), self._ptr(resid), self._ptr(qb),
+                   self._ptr(cb), self._ptr(wh))
         return qb, cb, wh
 
     def project_edges_soa(self, q_start, pose_a, pose_b, num_steps, max_steps: int, *, eps=EPSILON, dt=DT,
                           max_iters=MAX_ITERS, damping=0.0, kernel=None, out=None):
         """q_start [nq][E], pose_a/b [12][E], num_steps i32 [E] -> (q_path [max_steps][nq][E], n_valid i32 [E],
         iters_total i32 [E]).  Rows >= n_valid[e] of q_path are zero."""
-        self._chk_dev(q_start, pose_a, pose_b, num_steps)
+        ft = q_start.dtype
+        q_start = self._arg(q_start, (self.nq, None), ft, "q_start", copy=True)
         E = q_start.shape[1]
-        if num_steps.dtype != torch.int32:
-            raise TypeError("num_steps must be int32")
+        pose_a = self._arg(pose_a, (12, E), ft, "pose_a", copy=True)
+        pose_b = self._arg(pose_b, (12, E), ft, "pose_b", copy=True)
+        num_steps = self._arg(num_steps, (E,), torch.int32, "num_steps", copy=True)
         if out is None:
-            path = torch.zeros((max_steps, self.nq, E), dtype=q_start.dtype, device=self.device)
+            path = torch.zeros((max_steps, self.nq, E), dtype=ft, device=self.device)
             nv = torch.empty((E,), dtype=torch.int32, device=self.device)
             itt = torch.empty((E,), dtype=torch.int32, device=self.device)
         else:
             path, nv, itt = out
+            self._arg(path, (max_steps, self.nq, E), ft, "out q_path")
+            self._arg(nv, (E,), torch.int32, "out n_valid")
+            self._arg(itt, (E,), torch.int32, "out iters_total")
         prm = self._params(eps, dt, max_iters, damping, kernel)
-        f = getattr(self._lib, f"gik_project_edges_{_sfx(q_start.dtype)}")
-        _cabi.check(f(self._h, E, max_steps, self._ptr(q_start.contiguous()), self._ptr(pose_a.contiguous()),
-                      self._ptr(pose_b.contiguous()), self._ptr(num_steps.contiguous()), ctypes.byref(prm),
-                      self._ptr(path), self._ptr(nv), self._ptr(itt), self._stream()), "gik_project_edges")
-        if E:
-            self.launches += 1
+        self._call("project_edges", ft, E, max_steps, self._ptr(q_start), self._ptr(pose_a), self._ptr(pose_b),
+                   self._ptr(num_steps), ctypes.byref(prm), self._ptr(path), self._ptr(nv), self._ptr(itt))
         return path, nv, itt
 
     # ------------------------------------------------------------------ collision predicate (SURVEY 8f-1)
@@ -279,78 +298,60 @@ class GraspIK:
         -> colliding u8 [n].  `sel` (int64 [m], device): test only those columns (gik_collision_sel_*); the other
         entries of the result are 0."""
         self._need_scene()
-        self._chk_dev(q_soa, cube_pose_soa, sel)
-        n = q_soa.shape[1]
-        cp = None if cube_pose_soa is None else cube_pose_soa.to(q_soa.dtype).contiguous()
+        q, cp = self._q_cube(q_soa, cube_pose_soa)
+        n = q.shape[1]
         if sel is not None:
+            sel = self._arg(sel.to(torch.int64), (None,), torch.int64, "sel", copy=True)
             out = torch.zeros((n,), dtype=torch.uint8, device=self.device)
-            if sel.numel() == 0:
-                return out
-            f = getattr(self._lib, f"gik_collision_sel_{_sfx(q_soa.dtype)}")
-            sel = sel.to(torch.int64).contiguous()
-            _cabi.check(f(self._h, n, sel.numel(), self._ptr(sel), self._ptr(q_soa.contiguous()), self._ptr(cp), self._ptr(out),
-                          self._stream()), "gik_collision_sel")
-            self.launches += 1
+            if sel.numel():
+                self._call("collision_sel", q.dtype, n, sel.numel(), self._ptr(sel), self._ptr(q), self._ptr(cp),
+                           self._ptr(out))
             return out
         out = torch.empty((n,), dtype=torch.uint8, device=self.device)
-        f = getattr(self._lib, f"gik_collision_{_sfx(q_soa.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(q_soa.contiguous()), self._ptr(cp), self._ptr(out), self._stream()), "gik_collision")
-        if n:
-            self.launches += 1
+        self._call("collision", q.dtype, n, self._ptr(q), self._ptr(cp), self._ptr(out))
         return out
 
     def clearance_soa(self, q_soa: torch.Tensor, cube_pose_soa: torch.Tensor | None = None, threshold: float = 0.04) -> torch.Tensor:
         """distanceToObstacle(robot, q) >= threshold (tools.py:38-51, path.py:61-62) -> clear u8 [n]."""
         self._need_scene()
-        self._chk_dev(q_soa, cube_pose_soa)
-        n = q_soa.shape[1]
-        out = torch.empty((n,), dtype=torch.uint8, device=self.device)
-        f = getattr(self._lib, f"gik_clearance_{_sfx(q_soa.dtype)}")
-        cp = None if cube_pose_soa is None else cube_pose_soa.to(q_soa.dtype).contiguous()
-        _cabi.check(f(self._h, n, self._ptr(q_soa.contiguous()), self._ptr(cp), float(threshold), self._ptr(out),
-                      self._stream()), "gik_clearance")
-        if n:
-            self.launches += 1
+        q, cp = self._q_cube(q_soa, cube_pose_soa)
+        out = torch.empty((q.shape[1],), dtype=torch.uint8, device=self.device)
+        self._call("clearance", q.dtype, q.shape[1], self._ptr(q), self._ptr(cp), float(threshold), self._ptr(out))
         return out
 
     def obstacle_distance_soa(self, q_soa: torch.Tensor, cube_pose_soa: torch.Tensor | None = None, d_max: float = 2.0) -> torch.Tensor:
         """distanceToObstacle(robot, q) (tools.py:38-51) as a value -> dist [n] in q's dtype: smallest distance between
         the robot (and cube) and the table / obstacle, capped at d_max, 0 on intersection (gik_obstacle_distance_*)."""
         self._need_scene()
-        self._chk_dev(q_soa, cube_pose_soa)
-        n = q_soa.shape[1]
-        out = torch.empty((n,), dtype=q_soa.dtype, device=self.device)
-        f = getattr(self._lib, f"gik_obstacle_distance_{_sfx(q_soa.dtype)}")
-        cp = None if cube_pose_soa is None else cube_pose_soa.to(q_soa.dtype).contiguous()
-        _cabi.check(f(self._h, n, self._ptr(q_soa.contiguous()), self._ptr(cp), float(d_max), self._ptr(out),
-                      self._stream()), "gik_obstacle_distance")
-        if n:
-            self.launches += 1
+        q, cp = self._q_cube(q_soa, cube_pose_soa)
+        out = torch.empty((q.shape[1],), dtype=q.dtype, device=self.device)
+        self._call("obstacle_distance", q.dtype, q.shape[1], self._ptr(q), self._ptr(cp), float(d_max), self._ptr(out))
         return out
 
     def bezier_fit(self, q0: torch.Tensor, q1: torch.Tensor, path: torch.Tensor, pinv, basis, w0, w1):
         """The least-squares fit of `maketraj` (control.py:63-195) for many paths in one launch (gik_bezier_fit_*).
         q0, q1 [N, dim], path [N, n_points, dim] on this device; pinv [n_free, n_points], basis [n_points, n_free],
         w0 / w1 [n_points]: the factored design matrix (trajectory.fit_operands).  -> (ctrl [N, n_free + 6, dim], cost [N])."""
-        self._chk_dev(q0, q1, path)
-        dt = path.dtype
-        if dt not in (torch.float32, torch.float64) or q0.dtype != dt or q1.dtype != dt:
-            raise TypeError("q0, q1 and path must share a float32 / float64 dtype")
+        ft = path.dtype
+        path = self._arg(path, (None, None, None), ft, "path", copy=True)
         N, n_points, dim = path.shape
+        q0 = self._arg(q0, (N, dim), ft, "q0", copy=True)
+        q1 = self._arg(q1, (N, dim), ft, "q1", copy=True)
         n_free = int(pinv.shape[0])
-        if q0.shape != (N, dim) or q1.shape != (N, dim) or tuple(pinv.shape) != (n_free, n_points) or \
-                tuple(basis.shape) != (n_points, n_free) or w0.shape[0] != n_points or w1.shape[0] != n_points:
-            raise ValueError("bezier_fit: inconsistent shapes")
-        ops = [torch.as_tensor(x, dtype=dt, device=self.device).contiguous() for x in (pinv, basis, w0, w1)]
-        ctrl = torch.empty((N, n_free + 6, dim), dtype=dt, device=self.device)
-        cost = torch.empty((N,), dtype=dt, device=self.device)
-        f = getattr(self._lib, f"gik_bezier_fit_{_sfx(dt)}")
-        _cabi.check(f(self._h, N, n_points, dim, n_free + 6, *[self._ptr(x) for x in ops], self._ptr(q0.contiguous()),
-                      self._ptr(q1.contiguous()), self._ptr(path.contiguous()), self._ptr(ctrl), self._ptr(cost), self._stream()),
-                    "gik_bezier_fit")
-        if N:
-            self.launches += 1
+        ops = [self._arg(torch.as_tensor(x, dtype=ft, device=self.device), shape, ft, name, copy=True)
+               for x, shape, name in ((pinv, (n_free, n_points), "pinv"), (basis, (n_points, n_free), "basis"),
+                                      (w0, (n_points,), "w0"), (w1, (n_points,), "w1"))]
+        ctrl = torch.empty((N, n_free + 6, dim), dtype=ft, device=self.device)
+        cost = torch.empty((N,), dtype=ft, device=self.device)
+        self._call("bezier_fit", ft, N, n_points, dim, n_free + 6, *[self._ptr(x) for x in ops], self._ptr(q0), self._ptr(q1),
+                   self._ptr(path), self._ptr(ctrl), self._ptr(cost))
         return ctrl, cost
+
+    def _traj_args(self, ctrl, weights):
+        """ctrl [N, n_ctrl, nq] and weights [M, n_ctrl] (converted to ctrl's dtype) of the trajectory entries."""
+        ctrl = self._arg(ctrl, (None, None, self.nq), ctrl.dtype, "ctrl", copy=True)
+        W = torch.as_tensor(weights, dtype=ctrl.dtype, device=self.device)
+        return ctrl, self._arg(W, (None, ctrl.shape[1]), ctrl.dtype, "weights", copy=True)
 
     def check_trajectories(self, ctrl: torch.Tensor, weights, *, limit_tol: float, grasp_tol: float, per_sample=False):
         """Validity of many Bezier trajectories at the sample times of `weights` (gik_traj_check_*, semantics in
@@ -360,24 +361,15 @@ class GraspIK:
         [N] (flags of the first bad sample: 1 limits | 2 grasp | 4 collision), grasp_err [N] (max over the samples),
         sample_flags u8 [N, M] or None)."""
         self._need_scene()
-        self._chk_dev(ctrl)
-        dt = ctrl.dtype
-        N, n_ctrl, nq = ctrl.shape
-        W = torch.as_tensor(weights, dtype=dt, device=self.device).contiguous()
-        if nq != self.nq or W.dim() != 2 or W.shape[1] != n_ctrl:
-            raise ValueError(f"check_trajectories: expected ctrl [N, n_ctrl, {self.nq}] and weights [M, n_ctrl]")
-        M = W.shape[0]
+        ctrl, W = self._traj_args(ctrl, weights)
+        (N, n_ctrl, _), M = ctrl.shape, W.shape[0]
         valid = torch.empty((N,), dtype=torch.uint8, device=self.device)
         first_bad = torch.empty((N,), dtype=torch.int32, device=self.device)
         reason = torch.empty((N,), dtype=torch.uint8, device=self.device)
-        grasp_err = torch.empty((N,), dtype=dt, device=self.device)
+        grasp_err = torch.empty((N,), dtype=ctrl.dtype, device=self.device)
         flags = torch.empty((N, M), dtype=torch.uint8, device=self.device) if per_sample else None
-        f = getattr(self._lib, f"gik_traj_check_{_sfx(dt)}")
-        _cabi.check(f(self._h, N, n_ctrl, M, self._ptr(W), self._ptr(ctrl.contiguous()), float(limit_tol),
-                      float(grasp_tol), self._ptr(valid), self._ptr(first_bad), self._ptr(reason), self._ptr(grasp_err),
-                      self._ptr(flags), self._stream()), "gik_traj_check")
-        if N:
-            self.launches += 3
+        self._call("traj_check", ctrl.dtype, N, n_ctrl, M, self._ptr(W), self._ptr(ctrl), float(limit_tol), float(grasp_tol),
+                   self._ptr(valid), self._ptr(first_bad), self._ptr(reason), self._ptr(grasp_err), self._ptr(flags))
         return valid, first_bad, reason, grasp_err, flags
 
     def refine_trajectories(self, ctrl: torch.Tensor, weights, *, max_iters: int, tol: float, damping: float):
@@ -385,56 +377,41 @@ class GraspIK:
         arm's free control points follow the left hand.  ctrl [N, n_ctrl, nq] on this device; weights [M, n_ctrl]:
         Bernstein weights of the samples (trajectory.sample_weights).  -> (ctrl_out [N, n_ctrl, nq], obj_before f64 [N],
         obj_after f64 [N], grasp_err [N] (max over the samples at the output), iters i32 [N], accepted i32 [N])."""
-        self._chk_dev(ctrl)
-        dt = ctrl.dtype
-        N, n_ctrl, nq = ctrl.shape
-        W = torch.as_tensor(weights, dtype=dt, device=self.device).contiguous()
-        if nq != self.nq or W.dim() != 2 or W.shape[1] != n_ctrl:
-            raise ValueError(f"refine_trajectories: expected ctrl [N, n_ctrl, {self.nq}] and weights [M, n_ctrl]")
-        out = torch.empty_like(ctrl, memory_format=torch.contiguous_format)
+        ctrl, W = self._traj_args(ctrl, weights)
+        N, n_ctrl, _ = ctrl.shape
+        out = torch.empty_like(ctrl)
         f64 = lambda: torch.empty((N,), dtype=torch.float64, device=self.device)       # noqa: E731
         i32 = lambda: torch.empty((N,), dtype=torch.int32, device=self.device)         # noqa: E731
         obj_before, obj_after, iters, accepted = f64(), f64(), i32(), i32()
-        grasp_err = torch.empty((N,), dtype=dt, device=self.device)
-        f = getattr(self._lib, f"gik_traj_refine_{_sfx(dt)}")
-        _cabi.check(f(self._h, N, n_ctrl, W.shape[0], self._ptr(W), self._ptr(ctrl.contiguous()), int(max_iters),
-                      float(tol), float(damping), self._ptr(out), self._ptr(obj_before), self._ptr(obj_after),
-                      self._ptr(grasp_err), self._ptr(iters), self._ptr(accepted), self._stream()), "gik_traj_refine")
-        if N:
-            self.launches += 1
+        grasp_err = torch.empty((N,), dtype=ctrl.dtype, device=self.device)
+        self._call("traj_refine", ctrl.dtype, N, n_ctrl, W.shape[0], self._ptr(W), self._ptr(ctrl), int(max_iters),
+                   float(tol), float(damping), self._ptr(out), self._ptr(obj_before), self._ptr(obj_after),
+                   self._ptr(grasp_err), self._ptr(iters), self._ptr(accepted))
         return out, obj_before, obj_after, grasp_err, iters, accepted
 
     # ------------------------------------------------------------------ RRT-connect trees on the device (csrc/gik_tree.cuh)
-    # verts [n_trees][nq][cap], cubes [n_trees][12][cap], parent i32 [n_trees][cap], n_verts i32 [n_trees]
-    def _chk_tree(self, verts, n_verts, cubes=None, parent=None):
-        self._chk_dev(verts, n_verts, cubes, parent)
-        _sfx(verts.dtype)
-        n_trees, nq, cap = verts.shape
-        if nq != self.nq or n_verts.shape != (n_trees,) or n_verts.dtype != torch.int32 or \
-                (cubes is not None and (cubes.shape != (n_trees, 12, cap) or cubes.dtype != verts.dtype)) or \
-                (parent is not None and (parent.shape != (n_trees, cap) or parent.dtype != torch.int32)):
-            raise ValueError("trees: expected verts [n_trees][nq][cap], cubes [n_trees][12][cap] (same dtype), "
-                             "parent int32 [n_trees][cap], n_verts int32 [n_trees]")
-        if not all(t is None or t.is_contiguous() for t in (verts, n_verts, cubes, parent)):
-            raise ValueError("tree arrays must be contiguous")
+    # verts [n_trees][nq][cap], cubes [n_trees][12][cap], parent i32 [n_trees][cap], n_verts i32 [n_trees]; the trees
+    # are updated in place, so these are checked, never copied
+    def _tree(self, verts, n_verts, cubes=None, parent=None):
+        self._arg(verts, (None, self.nq, None), verts.dtype, "verts")
+        n_trees, _, cap = verts.shape
+        self._arg(n_verts, (n_trees,), torch.int32, "n_verts")
+        if cubes is not None:
+            self._arg(cubes, (n_trees, 12, cap), verts.dtype, "cubes")
+        if parent is not None:
+            self._arg(parent, (n_trees, cap), torch.int32, "parent")
         return n_trees, cap
 
     def tree_nearest(self, verts, n_verts, targets, target_tree) -> torch.Tensor:
         """Nearest vertex of tree target_tree[t] to each row of targets [n,nq] (gik_tree_nearest_*): squared distances
         in fp64, numpy's sum order and argmin's tie rule (lowest index).  -> nearest int32 [n] (-1: empty tree)."""
-        n_trees, cap = self._chk_tree(verts, n_verts)
-        self._chk_dev(targets, target_tree)
-        n = targets.shape[0]
-        tg = targets.to(verts.dtype).contiguous()
-        tt = target_tree.to(torch.int32).contiguous()
-        if tg.shape != (n, self.nq) or tt.shape != (n,):
-            raise ValueError("tree_nearest: expected targets [n][nq] and target_tree [n]")
+        n_trees, cap = self._tree(verts, n_verts)
+        tg = self._arg(targets.to(verts.dtype), (None, self.nq), verts.dtype, "targets", copy=True)
+        n = tg.shape[0]
+        tt = self._arg(target_tree.to(torch.int32), (n,), torch.int32, "target_tree", copy=True)
         out = torch.empty((n,), dtype=torch.int32, device=self.device)
-        f = getattr(self._lib, f"gik_tree_nearest_{_sfx(verts.dtype)}")
-        _cabi.check(f(self._h, n_trees, cap, self._ptr(verts), self._ptr(n_verts), n, self._ptr(tg), self._ptr(tt),
-                      self._ptr(out), self._stream()), "gik_tree_nearest")
-        if n:
-            self.launches += 1
+        self._call("tree_nearest", verts.dtype, n_trees, cap, self._ptr(verts), self._ptr(n_verts), n, self._ptr(tg),
+                   self._ptr(tt), self._ptr(out))
         return out
 
     def tree_grow(self, verts, cubes, parent, n_verts, overflow, edge_tree, near, q_start, pose_a, pose_b, num_steps,
@@ -445,27 +422,22 @@ class GraspIK:
         inputs and output, n_valid i32 [E] its step counts (< 0: no segment).  overflow u8 [n_trees] is set for a tree
         that would exceed its capacity (left unchanged).  -> seg_end int32 [E] (tree index of each segment's last
         vertex, -1 without a segment)."""
-        n_trees, cap = self._chk_tree(verts, n_verts, cubes, parent)
-        self._chk_dev(overflow, edge_tree, near, q_start, pose_a, pose_b, num_steps, n_valid, q_path)
+        n_trees, cap = self._tree(verts, n_verts, cubes, parent)
+        ft = verts.dtype
+        self._arg(overflow, (n_trees,), torch.uint8, "overflow")
+        q_start = self._arg(q_start, (self.nq, None), ft, "q_start", copy=True)
         E = q_start.shape[1]
-        S = q_path.shape[0]
-        dt = verts.dtype
-        if overflow.shape != (n_trees,) or overflow.dtype != torch.uint8:
-            raise ValueError("tree_grow: overflow must be uint8 [n_trees]")
-        if q_start.shape != (self.nq, E) or pose_a.shape != (12, E) or pose_b.shape != (12, E) or \
-                q_path.shape != (S, self.nq, E) or any(t.shape != (E,) for t in (edge_tree, near, num_steps, n_valid)):
-            raise ValueError("tree_grow: inconsistent edge shapes")
-        if any(t.dtype != dt for t in (q_start, pose_a, pose_b, q_path)) or \
-                any(t.dtype != torch.int32 for t in (edge_tree, near, num_steps, n_valid)):
-            raise TypeError("tree_grow: float arrays must share the trees' dtype, index arrays must be int32")
+        pose_a = self._arg(pose_a, (12, E), ft, "pose_a", copy=True)
+        pose_b = self._arg(pose_b, (12, E), ft, "pose_b", copy=True)
+        q_path = self._arg(q_path, (None, self.nq, E), ft, "q_path", copy=True)
+        edge_tree, near, num_steps, n_valid = [self._arg(t, (E,), torch.int32, name, copy=True) for t, name in
+                                               ((edge_tree, "edge_tree"), (near, "near"), (num_steps, "num_steps"),
+                                                (n_valid, "n_valid"))]
         seg_end = torch.empty((E,), dtype=torch.int32, device=self.device)
-        args = [x.contiguous() for x in (edge_tree, near, q_start, pose_a, pose_b, num_steps, n_valid, q_path)]
-        f = getattr(self._lib, f"gik_tree_grow_{_sfx(dt)}")
-        _cabi.check(f(self._h, n_trees, cap, self._ptr(verts), self._ptr(cubes), self._ptr(parent), self._ptr(n_verts),
-                      self._ptr(overflow), E, S, *[self._ptr(x) for x in args], self._ptr(seg_end), self._stream()),
-                    "gik_tree_grow")
-        if E:
-            self.launches += 1
+        self._call("tree_grow", ft, n_trees, cap, self._ptr(verts), self._ptr(cubes), self._ptr(parent), self._ptr(n_verts),
+                   self._ptr(overflow), E, q_path.shape[0],
+                   *[self._ptr(x) for x in (edge_tree, near, q_start, pose_a, pose_b, num_steps, n_valid, q_path)],
+                   self._ptr(seg_end))
         return seg_end
 
     def tree_paths(self, verts, cubes, parent, n_verts, start_end, goal_end):
@@ -473,24 +445,20 @@ class GraspIK:
         (-1 = did not connect): get_path(start) + get_path(goal)[::-1] (path.py:226-233, 317) as packed rows
         (gik_tree_paths_*).  -> (q [total][nq], cube [total][12], offsets int64 [Q+1]); query i owns rows
         offsets[i]:offsets[i+1].  One host synchronisation (reading the total)."""
-        n_trees, cap = self._chk_tree(verts, n_verts, cubes, parent)
+        n_trees, cap = self._tree(verts, n_verts, cubes, parent)
         Q = n_trees // 2
-        self._chk_dev(start_end, goal_end)
-        if n_trees != 2 * Q or start_end.shape != (Q,) or goal_end.shape != (Q,):
-            raise ValueError("tree_paths: expected 2Q trees and start_end / goal_end [Q]")
-        se, ge = start_end.to(torch.int32).contiguous(), goal_end.to(torch.int32).contiguous()
+        if n_trees != 2 * Q:
+            raise ValueError("tree_paths: expected 2Q trees")
+        se = self._arg(start_end.to(torch.int32), (Q,), torch.int32, "start_end", copy=True)
+        ge = self._arg(goal_end.to(torch.int32), (Q,), torch.int32, "goal_end", copy=True)
         offsets = torch.zeros((Q + 1,), dtype=torch.int64, device=self.device)
-        f = getattr(self._lib, f"gik_tree_paths_{_sfx(verts.dtype)}")
         tree = [self._ptr(x) for x in (verts, cubes, parent, n_verts, se, ge)]
-        _cabi.check(f(self._h, Q, cap, *tree, self._ptr(offsets), None, None, self._stream()), "gik_tree_paths")
+        self._call("tree_paths", verts.dtype, Q, cap, *tree, self._ptr(offsets), None, None)
         total = int(offsets[-1].item()) if Q else 0
         q = torch.empty((total, self.nq), dtype=verts.dtype, device=self.device)
         cube = torch.empty((total, 12), dtype=verts.dtype, device=self.device)
         if total:
-            _cabi.check(f(self._h, Q, cap, *tree, self._ptr(offsets), self._ptr(q), self._ptr(cube), self._stream()),
-                        "gik_tree_paths")
-        if Q:
-            self.launches += 3 if total else 2
+            self._call("tree_paths", verts.dtype, Q, cap, *tree, self._ptr(offsets), self._ptr(q), self._ptr(cube))
         return q, cube, offsets
 
     def path_shortcut(self, q, cube, offsets, pair_i, pair_j, num_steps, n_valid, q_path, *, join_tol: float):
@@ -499,45 +467,36 @@ class GraspIK:
         project_edges_soa launch: pair_i / pair_j / num_steps / n_valid int32 [Q, K] and q_path [S][nq][Q*K].
         -> (q [total'][nq], cube [total'][12], offsets int64 [Q+1], chosen int32 [Q] (-1 = none), length float64 [Q]
         (joint-space length of each output path)).  One host synchronisation (reading the new total)."""
-        self._chk_dev(q, cube, offsets, pair_i, pair_j, num_steps, n_valid, q_path)
-        dt = q.dtype
+        ft = q.dtype
+        q = self._arg(q, (None, self.nq), ft, "q", copy=True)
+        cube = self._arg(cube, (q.shape[0], 12), ft, "cube", copy=True)
+        offsets = self._arg(offsets, (None,), torch.int64, "offsets", copy=True)
         Q = offsets.shape[0] - 1
-        K = pair_i.shape[1] if pair_i.dim() == 2 else -1
-        S = q_path.shape[0]
-        if Q < 0 or offsets.dtype != torch.int64 or q.shape[1:] != (self.nq,) or cube.shape != (q.shape[0], 12) or \
-                any(t.shape != (Q, K) for t in (pair_i, pair_j, num_steps, n_valid)) or q_path.shape != (S, self.nq, Q * K):
-            raise ValueError("path_shortcut: expected q [total][nq], cube [total][12], offsets int64 [Q+1], candidate "
-                             "arrays [Q, K] and q_path [S][nq][Q*K]")
-        if cube.dtype != dt or q_path.dtype != dt or any(t.dtype != torch.int32 for t in (pair_i, pair_j, num_steps, n_valid)):
-            raise TypeError("path_shortcut: float arrays must share q's dtype, candidate arrays must be int32")
-        args = [x.contiguous() for x in (offsets, q, cube, pair_i, pair_j, num_steps, n_valid, q_path)]
+        pair_i = self._arg(pair_i, (Q, None), torch.int32, "pair_i", copy=True)
+        K = pair_i.shape[1]
+        pair_j, num_steps, n_valid = [self._arg(t, (Q, K), torch.int32, name, copy=True) for t, name in
+                                      ((pair_j, "pair_j"), (num_steps, "num_steps"), (n_valid, "n_valid"))]
+        q_path = self._arg(q_path, (None, self.nq, Q * K), ft, "q_path", copy=True)
         chosen = torch.empty((Q,), dtype=torch.int32, device=self.device)
         length = torch.empty((Q,), dtype=torch.float64, device=self.device)
         off_out = torch.empty((Q + 1,), dtype=torch.int64, device=self.device)
-        f = getattr(self._lib, f"gik_path_shortcut_{_sfx(dt)}")
-        head = [self._ptr(x) for x in args]
+        head = [self._ptr(x) for x in (offsets, q, cube, pair_i, pair_j, num_steps, n_valid, q_path)]
         tail = [self._ptr(chosen), self._ptr(length), self._ptr(off_out)]
-        _cabi.check(f(self._h, Q, K, S, *head, float(join_tol), *tail, None, None, self._stream()), "gik_path_shortcut")
+        self._call("path_shortcut", ft, Q, K, q_path.shape[0], *head, float(join_tol), *tail, None, None)
         total = int(off_out[-1].item()) if Q else 0
-        q_out = torch.empty((total, self.nq), dtype=dt, device=self.device)
-        cube_out = torch.empty((total, 12), dtype=dt, device=self.device)
+        q_out = torch.empty((total, self.nq), dtype=ft, device=self.device)
+        cube_out = torch.empty((total, 12), dtype=ft, device=self.device)
         if total:
-            _cabi.check(f(self._h, Q, K, S, *head, float(join_tol), *tail, self._ptr(q_out), self._ptr(cube_out),
-                          self._stream()), "gik_path_shortcut")
-        if Q:
-            self.launches += 3 if total else 2
+            self._call("path_shortcut", ft, Q, K, q_path.shape[0], *head, float(join_tol), *tail, self._ptr(q_out),
+                       self._ptr(cube_out))
         return q_out, cube_out, off_out, chosen, length
 
     def cube_collision_soa(self, cube_pose_soa: torch.Tensor) -> torch.Tensor:
         """The cube's own collision test (cube vs table / obstacle, path.py:51-52): cube_pose [12][n] -> u8 [n]."""
         self._need_scene()
-        self._chk_dev(cube_pose_soa)
-        n = cube_pose_soa.shape[1]
-        out = torch.empty((n,), dtype=torch.uint8, device=self.device)
-        f = getattr(self._lib, f"gik_cube_collision_{_sfx(cube_pose_soa.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(cube_pose_soa.contiguous()), self._ptr(out), self._stream()), "gik_cube_collision")
-        if n:
-            self.launches += 1
+        cp = self._arg(cube_pose_soa, (12, None), cube_pose_soa.dtype, "cube_pose", copy=True)
+        out = torch.empty((cp.shape[1],), dtype=torch.uint8, device=self.device)
+        self._call("cube_collision", cp.dtype, cp.shape[1], self._ptr(cp), self._ptr(out))
         return out
 
     def collision(self, q, cube_pose=None, *, dtype=None) -> torch.Tensor:
@@ -566,27 +525,23 @@ class GraspIK:
         -> (q [nq][n], success u8 [n], converged u8 [n], iters i32 [n], resid [2][n][, stats]); stats (device int64 [4]):
         problems decided as persistent collisions, problems replayed, replayed iterations, replays that succeeded."""
         self._need_scene()
-        self._chk_dev(q_init, pose)
-        if q_init.dtype != pose.dtype:
-            raise TypeError("q_init and pose must share a dtype")
+        ft = q_init.dtype
+        q_init = self._arg(q_init, (self.nq, None), ft, "q_init", copy=True)
         n = q_init.shape[1]
+        pose = self._arg(pose, (12, n), ft, "pose", copy=True)
         q = torch.empty_like(q_init)
         succ = torch.empty((n,), dtype=torch.uint8, device=self.device)
         conv = torch.empty((n,), dtype=torch.uint8, device=self.device)
         iters = torch.empty((n,), dtype=torch.int32, device=self.device)
-        resid = torch.empty((2, n), dtype=q_init.dtype, device=self.device)
-        esz = 4 if q_init.dtype == torch.float32 else 8
+        resid = torch.empty((2, n), dtype=ft, device=self.device)
+        esz = 4 if ft == torch.float32 else 8
         nbytes = int(self._lib.gik_solve_success_scratch_bytes(self._h, n, esz))
         scratch = torch.empty((max(nbytes, 8),), dtype=torch.uint8, device=self.device)
         prm = self._params(eps, dt, max_iters, damping, kernel, early_stop)
         if not descend_while_colliding:
             prm.flags |= 64                                                  # GIK_F_NO_DESCEND
-        f = getattr(self._lib, f"gik_solve_success_{_sfx(q_init.dtype)}")
-        _cabi.check(f(self._h, n, self._ptr(q_init.contiguous()), self._ptr(pose.contiguous()), ctypes.byref(prm),
-                      self._ptr(q), self._ptr(succ), self._ptr(conv), self._ptr(iters), self._ptr(resid),
-                      self._ptr(scratch), self._stream()), "gik_solve_success")
-        if n:
-            self.launches += 3 if not descend_while_colliding else 6
+        self._call("solve_success", ft, n, self._ptr(q_init), self._ptr(pose), ctypes.byref(prm), self._ptr(q),
+                   self._ptr(succ), self._ptr(conv), self._ptr(iters), self._ptr(resid), self._ptr(scratch))
         if return_stats:
             stats = scratch[nbytes - 256 + 8:nbytes - 256 + 40].view(torch.int64).clone() if n else torch.zeros(4, dtype=torch.int64, device=self.device)
             return q, succ, conv, iters, resid, stats
@@ -735,10 +690,8 @@ def solve_host(self, q_init, pose, *, dtype=torch.float32, eps=EPSILON, dt=DT, m
                     first_in.record(copy_stream)
         cur.wait_event(first_in)
         prm = self._params(eps, dt, max_iters, damping, kernel)
-        f = getattr(self._lib, f"gik_solve_rows_{_sfx(dtype)}")
-        _cabi.check(f(self._h, B, self._ptr(dq), self._ptr(dp), ctypes.byref(prm), self._ptr(q_out), self._ptr(c_out),
-                      self._ptr(it_out), self._ptr(r_out), self._ptr(ready), self._stream()), "gik_solve_rows")
-        self.launches += 1
+        self._call("solve_rows", dtype, B, self._ptr(dq), self._ptr(dp), ctypes.byref(prm), self._ptr(q_out),
+                   self._ptr(c_out), self._ptr(it_out), self._ptr(r_out), self._ptr(ready))
         cur.synchronize()          # results are host memory: the call returns when the kernel has stored them
         copy_stream.synchronize()
     return (q_out, c_out.view(torch.bool)) + ((SolveInfo(it_out, r_out),) if return_info else ())

@@ -53,7 +53,7 @@ def test_struct_sizes_match_the_c_header(tmp_path):
     assert sizes == [ctypes.sizeof(GikTable), ctypes.sizeof(_cabi.GikParams), ctypes.sizeof(GikGeom), ctypes.sizeof(GikScene)]
 
 
-def test_error_paths_without_gpu():
+def test_error_codes_without_gpu():
     from gik_b200 import _cabi
     lib = _cabi.lib()
     assert lib.gik_strerror(0) == b"ok"
@@ -63,10 +63,12 @@ def test_error_paths_without_gpu():
     h = ctypes.c_void_p()
     assert lib.gik_create(None, 0, ctypes.byref(h)) == -1              # GIK_E_NULL
     assert lib.gik_destroy(None) == -6                                 # GIK_E_HANDLE
-    assert lib.gik_solve_f32(None, 1, None, None, None, None, None, None, None, None) == -6
     p = _cabi.GikParams()
     lib.gik_default_params(ctypes.byref(p))
     assert (p.eps, p.dt, p.damping, p.max_iters, p.flags) == (1e-3, 1e-2, 0.0, 1000, 0)
+    x = ctypes.c_void_p(8)                                             # never dereferenced
+    assert lib.gik_solve_f32(None, 1, x, x, ctypes.byref(p), x, x, None, None, None) == -6
+    assert lib.gik_solve_f32(None, 1, None, None, None, None, None, None, None, None) == -1   # no params: checked first
 
 
 def test_create_rejects_bad_tables_before_touching_cuda(table):

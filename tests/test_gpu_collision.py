@@ -104,13 +104,15 @@ def test_golden_grasp_poses_are_collision_free(solver, golden):
     assert solver.collision(_t(Q, torch.float64)).any() is not None
 
 
-def test_collision_error_codes(table):
+def test_collision_error_codes_in_check_order(table):
     import ctypes
     import gik_b200
     from gik_b200 import _cabi
     s = gik_b200.GraspIK(table, "cuda:0")
     z = ctypes.c_void_p(0)
-    assert _cabi.lib().gik_collision_f32(s._h, 4, z, z, z, z) == -7           # GIK_E_NOSCENE
+    x = ctypes.c_void_p(8)                                                     # never dereferenced
+    assert _cabi.lib().gik_collision_f32(s._h, 4, x, z, x, z) == -7           # GIK_E_NOSCENE
+    assert _cabi.lib().gik_collision_f32(s._h, 4, z, z, z, z) == -1           # pointers are checked before the scene
     s.attach_scene()
     assert _cabi.lib().gik_collision_f32(s._h, 4, z, z, z, z) == -1           # GIK_E_NULL
     assert _cabi.lib().gik_collision_f32(s._h, 0, z, z, z, z) == 0
