@@ -411,6 +411,93 @@ int gik_path_shortcut_f64(gik_handle_t h, int64_t n_paths, int32_t n_cand, int32
                           void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
+ * Grasp roadmap: N vertices (q [N][nq], cube [N][12], row-major grasps) and directed edges built once in a static scene,
+ * then queried many times.  The roadmap's edges are CSR by source: row_ptr [N+1] int64, dst [E] int32 (target vertex),
+ * ns [E] int32 (the edge's steps), weight [E] fp64, step_ptr [E+1] int64 and steps [rows][nq]: steps 1 .. ns-1 of edge e
+ * at rows step_ptr[e] .. step_ptr[e+1]-1 (the step at cube_dst is not stored: q_dst replaces it, as a shortcut splice
+ * does).  ||.|| below is the fp64 norm of the fp64 difference, squares summed left to right; every sum is fp64, left to
+ * right, without contraction.
+ * A query batch of n_queries = Q queries has A = 2 ka + 1 attachment edges per query, ka = k_attach; slot s of query p
+ * is edge e = p * A + s of one gik_project_edges_* launch:
+ *   s < ka        (q_init, cube0) -> vertex att_vertex[e] (the ka vertices nearest cube0)
+ *   ka <= s < 2ka vertex att_vertex[e] -> (q_goal, cube1) (the ka vertices nearest cube1)
+ *   s = 2 ka      (q_init, cube0) -> (q_goal, cube1), att_vertex[e] = -1
+ * att_weight [Q][A] holds their gik_roadmap_edges_* weights (+inf = rejected).
+ * ------------------------------------------------------------------------------------------------------- */
+
+/* k nearest vertices by the fp64 Euclidean distance of cube translations: d = sqrt((dx^2 + dy^2) + dz^2) of the values
+ * 9..11 of each placement.  nbr [n_points][k] lists them nearest first, ties to the lower index.  points [n_points][12]
+ * (row-major); points = NULL: the points are the vertices themselves (n_points = n_vertices), each excluding itself.
+ * One warp per point.
+ * Errors: GIK_E_SIZE (k < 1, k > 32, k > n_vertices - 1, n_points < 0, points NULL and n_points != n_vertices), GIK_E_NULL
+ * (cube or nbr NULL and n_points > 0), GIK_E_HANDLE; n_points = 0 is a no-op. */
+int gik_knn_f32(gik_handle_t h, int32_t n_vertices, int32_t k, const float* cube, int64_t n_points, const float* points,
+                int32_t* nbr, void* stream);
+int gik_knn_f64(gik_handle_t h, int32_t n_vertices, int32_t k, const double* cube, int64_t n_points, const double* points,
+                int32_t* nbr, void* stream);
+
+/* Acceptance and weight of n_edges edges, each from q_from[e] towards q_to[e] ([n_edges][nq] rows): column e of one
+ * gik_project_edges_* launch (max_steps, q_path [max_steps][nq][n_edges]) with num_steps[e] = ns steps of which
+ * n_valid[e] = nv converged collision-free.  With s_m the q of step m, the edge is accepted when
+ *   1 <= ns <= max_steps, nv == ns and ||s_ns - q_to|| < join_tol,
+ * and then weight[e] = ||s_1 - q_from|| + sum_{m=1}^{ns-2} ||s_{m+1} - s_m|| + ||q_to - s_{ns-1}|| (ns = 1:
+ * ||q_to - q_from||), summed from 0 as gik_path_shortcut_* sums a path length; weight[e] = +inf when rejected.
+ * Errors: GIK_E_SIZE (n_edges < 0, max_steps < 0), GIK_E_PARAM (join_tol negative or NaN), GIK_E_NULL (a required pointer
+ * is NULL and n_edges > 0; q_path only when max_steps > 0), GIK_E_HANDLE; n_edges = 0 is a no-op. */
+int gik_roadmap_edges_f32(gik_handle_t h, int64_t n_edges, int32_t max_steps, const float* q_from, const float* q_to,
+                          const int32_t* num_steps, const int32_t* n_valid, const float* q_path, double join_tol,
+                          double* weight, void* stream);
+int gik_roadmap_edges_f64(gik_handle_t h, int64_t n_edges, int32_t max_steps, const double* q_from, const double* q_to,
+                          const int32_t* num_steps, const int32_t* n_valid, const double* q_path, double join_tol,
+                          double* weight, void* stream);
+
+/* Shortest paths of n_queries queries over one roadmap (n_vertices, n_edges, row_ptr / dst / weight), one CTA per query.
+ * Sources: the accepted start attachments a, dist[a] = their weight.  dist [Q][N] fp64 is the least fixed point of
+ * dist[v] = min(w(start -> v), min_u dist[u] + w(u, v)): the exact minimum over paths of the left-to-right fp64 sums, as
+ * Dijkstra computes it on the same weights (fp addition is monotone).  Then pred [Q][N]: -1 when a start attachment's
+ * weight equals dist[v] (the virtual start wins ties), else the smallest u with dist[u] + w(u, v) == dist[v], -2 when
+ * dist[v] = +inf.  The answer length[p] = min(w_direct, min_b dist[b] + w(b -> goal)) over the accepted goal attachments;
+ * goal_pred[p] = -1 when the direct edge achieves it (it wins ties), else the smallest such b; -2 and +inf when
+ * unconnected.  attach_start / attach_goal [Q] count the accepted start / goal attachments.  Entries of dst or
+ * att_vertex outside [0, N) are skipped.  No floating-point atomics: the outputs are identical between runs and do
+ * not depend on the other queries of the batch.  (Bellman-Ford rounds over the vertices lowered in the previous round,
+ * atomicMin on the distances' bit patterns, until a round lowers nothing; pred holds the round marks meanwhile.)
+ * Errors: GIK_E_SIZE (n_queries < 0, n_vertices < 1, k_attach < 0 or > 32, n_edges < 0), GIK_E_NULL (a required pointer
+ * is NULL and n_queries > 0; dst and weight only when n_edges > 0), GIK_E_HANDLE; n_queries = 0 is a no-op. */
+int gik_roadmap_sssp(gik_handle_t h, int64_t n_queries, int32_t n_vertices, int32_t k_attach, int64_t n_edges,
+                     const int64_t* row_ptr, const int32_t* dst, const double* weight, const int32_t* att_vertex,
+                     const double* att_weight, double* dist, int32_t* pred, int32_t* goal_pred, double* length,
+                     int32_t* attach_start, int32_t* attach_goal, void* stream);
+
+/* The paths of a query batch, packed as gik_tree_paths_* packs them: CSR rows offsets [Q+1] int64, q [total][nq],
+ * cube [total][12].  Query p's rows, from gik_roadmap_sssp_*'s pred / goal_pred: (q_init, cube0); for each segment
+ * (the start attachment, the roadmap edges along the predecessor chain, the goal attachment) its steps 1 .. ns-1, each
+ * with the placement edge_placement(cube_from, xi, m, ns) the edge kernel solved it for, then its end row (the vertex's
+ * q and cube; (q_goal, cube1) at the end).  The direct edge is one segment.  An unconnected query (or a chain that
+ * does not reach the start within N steps) has no rows.  vertices [Q] = roadmap vertices on the path.  Attachment
+ * steps are read from att_path [max_steps][nq][Q * A] with att_ns [Q][A] (the attachment edge launch).  steps may be
+ * NULL when no edge has more than one step.
+ * Two calls: with q = cube = NULL, offsets (offsets[Q] = the total, the one value the caller reads back) and vertices
+ * are written; then, with q and cube, the rows.
+ * Errors: GIK_E_SIZE (n_queries < 0, n_vertices < 1, k_attach < 0 or > 32, max_steps < 0, n_edges < 0), GIK_E_NULL (a
+ * required pointer is NULL and n_queries > 0; dst and ns only when n_edges > 0, att_path only when max_steps > 0; q
+ * without cube or the reverse), GIK_E_HANDLE; n_queries = 0 is a no-op. */
+int gik_roadmap_paths_f32(gik_handle_t h, int64_t n_queries, int32_t n_vertices, int32_t k_attach, int32_t max_steps,
+                          int64_t n_edges, const float* vq, const float* vcube, const int64_t* row_ptr, const int32_t* dst,
+                          const int32_t* ns, const int64_t* step_ptr, const float* steps, const float* q_init,
+                          const float* q_goal, const float* cube0, const float* cube1, const int32_t* att_vertex,
+                          const double* att_weight, const int32_t* att_ns, const float* att_path, const int32_t* pred,
+                          const int32_t* goal_pred, int64_t* offsets, int32_t* vertices, float* q, float* cube,
+                          void* stream);
+int gik_roadmap_paths_f64(gik_handle_t h, int64_t n_queries, int32_t n_vertices, int32_t k_attach, int32_t max_steps,
+                          int64_t n_edges, const double* vq, const double* vcube, const int64_t* row_ptr, const int32_t* dst,
+                          const int32_t* ns, const int64_t* step_ptr, const double* steps, const double* q_init,
+                          const double* q_goal, const double* cube0, const double* cube1, const int32_t* att_vertex,
+                          const double* att_weight, const int32_t* att_ns, const double* att_path, const int32_t* pred,
+                          const int32_t* goal_pred, int64_t* offsets, int32_t* vertices, double* q, double* cube,
+                          void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
  * Trajectory check: can a fitted trajectory be executed?  The reference finds out only by running its 1500 pybullet
  * control steps (control.py:416-463): between the path vertices the least-squares curve lies on no grasp manifold, and
  * its free control points are unconstrained.  This checks the curve itself at the controller's sample times.

@@ -13,6 +13,7 @@ from .inverse_geometry import apply_collision, computeqgrasppose, computeqgraspp
 from .path import (computepath, edge_num_steps, project_edges_batch, project_path, sample_cube_placements,  # noqa: F401
                    sample_grasp_poses_batch, se3_interpolate)
 from .planner import computepath_batch, shortcut_paths_batch                          # noqa: F401
+from .roadmap import Roadmap, build_roadmap, query_roadmap_batch                      # noqa: F401
 from .trajectory import (Bezier, check_trajectories_batch, check_trajectory, maketraj, maketraj_batch,  # noqa: F401
                          maketraj_paths, refine_trajectories_batch)
 from . import tools                                                                   # noqa: F401

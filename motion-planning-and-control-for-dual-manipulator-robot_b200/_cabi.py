@@ -32,7 +32,7 @@ class GikError(RuntimeError):
 def _sources():
     return [os.path.join(CSRC, f) for f in ("gik_kernels.cu", "gik_core.cuh", "gik_table.h", "gik_collide.cuh",
                                             "gik_collide_impl.cuh", "gik_bezier.cuh", "gik_tree.cuh",
-                                            "gik_shortcut.cuh", "gik_traj.cuh", "gik_traj_refine.cuh")] + \
+                                            "gik_shortcut.cuh", "gik_roadmap.cuh", "gik_traj.cuh", "gik_traj_refine.cuh")] + \
            [os.path.join(_HERE, "..", "include", "gik.h")]
 
 
@@ -104,9 +104,13 @@ def lib() -> ctypes.CDLL:
         getattr(L, f"gik_tree_grow_{sfx}").argtypes = [_P, _I64, _I32, _P, _P, _P, _P, _P, _I64, _I32] + [_P] * 10
         getattr(L, f"gik_tree_paths_{sfx}").argtypes = [_P, _I64, _I32] + [_P] * 10
         getattr(L, f"gik_path_shortcut_{sfx}").argtypes = [_P, _I64, _I32, _I32] + [_P] * 8 + [ctypes.c_double] + [_P] * 6
+        getattr(L, f"gik_knn_{sfx}").argtypes = [_P, _I32, _I32, _P, _I64, _P, _P, _P]
+        getattr(L, f"gik_roadmap_edges_{sfx}").argtypes = [_P, _I64, _I32] + [_P] * 5 + [ctypes.c_double, _P, _P]
+        getattr(L, f"gik_roadmap_paths_{sfx}").argtypes = [_P, _I64, _I32, _I32, _I32, _I64] + [_P] * 22
         getattr(L, f"gik_traj_check_{sfx}").argtypes = [_P, _I64, _I32, _I32, _P, _P, ctypes.c_double, ctypes.c_double] + [_P] * 6
         getattr(L, f"gik_traj_refine_{sfx}").argtypes = [_P, _I64, _I32, _I32, _P, _P, _I32, ctypes.c_double,
                                                           ctypes.c_double] + [_P] * 7
+    L.gik_roadmap_sssp.argtypes = [_P, _I64, _I32, _I32, _I64] + [_P] * 12
     L.gik_solve_success_scratch_bytes.argtypes = [_P, _I64, ctypes.c_int]
     L.gik_solve_success_scratch_bytes.restype = ctypes.c_size_t
     L.gik_flops_per_iter.restype = ctypes.c_size_t
@@ -134,6 +138,8 @@ EXPORTS = [
     "gik_tree_nearest_f32", "gik_tree_nearest_f64", "gik_tree_grow_f32", "gik_tree_grow_f64",
     "gik_tree_paths_f32", "gik_tree_paths_f64", "gik_path_shortcut_f32", "gik_path_shortcut_f64", "gik_traj_check_f32", "gik_traj_check_f64",
     "gik_traj_refine_f32", "gik_traj_refine_f64",
+    "gik_knn_f32", "gik_knn_f64", "gik_roadmap_edges_f32", "gik_roadmap_edges_f64", "gik_roadmap_sssp",
+    "gik_roadmap_paths_f32", "gik_roadmap_paths_f64",
     "gik_flops_per_iter", "gik_flops_per_iter_executed", "gik_bytes_per_solve", "gik_measure_fma_peak", "gik_solve_launch_dims",
     "gik_solve_kernel_name", "gik_launch_count",
     "gik_strerror", "gik_version",

@@ -102,9 +102,9 @@ class GraspIK:
         return count.value
 
     def _call(self, entry: str, dtype, *args):
-        """Call gik_<entry>_f32 / _f64 (chosen by dtype) with the handle first and the current stream last; raise on an
-        error code."""
-        f = getattr(self._lib, f"gik_{entry}_{_sfx(dtype)}")
+        """Call gik_<entry>_f32 / _f64 (chosen by dtype; None: gik_<entry>, an entry without a storage type) with the
+        handle first and the current stream last; raise on an error code."""
+        f = getattr(self._lib, f"gik_{entry}" if dtype is None else f"gik_{entry}_{_sfx(dtype)}")
         _cabi.check(f(self._h, *args, self._stream()), f"gik_{entry}")
 
     def _arg(self, t, shape, dtype, name, *, copy=False) -> torch.Tensor:
@@ -490,6 +490,113 @@ class GraspIK:
             self._call("path_shortcut", ft, Q, K, q_path.shape[0], *head, float(join_tol), *tail, self._ptr(q_out),
                        self._ptr(cube_out))
         return q_out, cube_out, off_out, chosen, length
+
+    # ------------------------------------------------------------------ grasp roadmap (csrc/gik_roadmap.cuh)
+    def knn(self, cube, k: int, points=None) -> torch.Tensor:
+        """The k vertices nearest each point by the fp64 distance of cube translations, nearest first, ties to the lower
+        index (gik_knn_*, semantics in include/gik.h).  cube [N,12] vertex placements; points [P,12] (converted to
+        cube's dtype), None: the vertices themselves, each excluding itself.  -> nbr int32 [P,k]."""
+        cube = self._arg(cube, (None, 12), cube.dtype, "cube", copy=True)
+        N = cube.shape[0]
+        if not 1 <= int(k) <= min(32, N - 1):
+            raise ValueError(f"knn: k must be in [1, min(32, N - 1)] with N = {N}, got {k}")
+        if points is not None:
+            points = self._arg(points.to(cube.dtype), (None, 12), cube.dtype, "points", copy=True)
+        P = N if points is None else points.shape[0]
+        nbr = torch.empty((P, int(k)), dtype=torch.int32, device=self.device)
+        self._call("knn", cube.dtype, N, int(k), self._ptr(cube), P, self._ptr(points), self._ptr(nbr))
+        return nbr
+
+    def roadmap_edges(self, q_from, q_to, num_steps, n_valid, q_path, *, join_tol: float) -> torch.Tensor:
+        """Acceptance and fp64 weight of the E edges of one project_edges_soa launch (gik_roadmap_edges_*, semantics in
+        include/gik.h): edge e from q_from[e] towards q_to[e] ([E,nq]), num_steps / n_valid int32 [E], q_path
+        [S][nq][E].  -> weight float64 [E], +inf for a rejected edge."""
+        ft = q_path.dtype
+        q_path = self._arg(q_path, (None, self.nq, None), ft, "q_path", copy=True)
+        E = q_path.shape[2]
+        q_from = self._arg(q_from, (E, self.nq), ft, "q_from", copy=True)
+        q_to = self._arg(q_to, (E, self.nq), ft, "q_to", copy=True)
+        num_steps = self._arg(num_steps, (E,), torch.int32, "num_steps", copy=True)
+        n_valid = self._arg(n_valid, (E,), torch.int32, "n_valid", copy=True)
+        weight = torch.empty((E,), dtype=torch.float64, device=self.device)
+        self._call("roadmap_edges", ft, E, q_path.shape[0], self._ptr(q_from), self._ptr(q_to), self._ptr(num_steps),
+                   self._ptr(n_valid), self._ptr(q_path), float(join_tol), self._ptr(weight))
+        return weight
+
+    def _csr(self, row_ptr, dst, weight=None, ns=None):
+        row_ptr = self._arg(row_ptr, (None,), torch.int64, "row_ptr", copy=True)
+        dst = self._arg(dst, (None,), torch.int32, "dst", copy=True)
+        E = dst.shape[0]
+        out = [row_ptr, dst]
+        if weight is not None:
+            out.append(self._arg(weight, (E,), torch.float64, "weight", copy=True))
+        if ns is not None:
+            out.append(self._arg(ns, (E,), torch.int32, "ns", copy=True))
+        return out
+
+    def roadmap_sssp(self, row_ptr, dst, weight, att_vertex, att_weight):
+        """Shortest paths of Q queries over one roadmap, one CTA per query (gik_roadmap_sssp, semantics in
+        include/gik.h).  row_ptr int64 [N+1], dst int32 [E], weight float64 [E]; att_vertex int32 [Q, 2ka+1] and
+        att_weight float64 [Q, 2ka+1]: the attachment slots.  -> (dist float64 [Q,N], pred int32 [Q,N], goal_pred int32
+        [Q], length float64 [Q], attach_start int32 [Q], attach_goal int32 [Q]).  dist and pred take 12 Q N bytes."""
+        row_ptr, dst, weight = self._csr(row_ptr, dst, weight)
+        N, E = row_ptr.shape[0] - 1, dst.shape[0]
+        att_vertex = self._arg(att_vertex, (None, None), torch.int32, "att_vertex", copy=True)
+        Q, A = att_vertex.shape
+        if A % 2 != 1:
+            raise ValueError(f"att_vertex: expected 2 * k_attach + 1 slots per query, got {A}")
+        att_weight = self._arg(att_weight, (Q, A), torch.float64, "att_weight", copy=True)
+        dist = torch.empty((Q, N), dtype=torch.float64, device=self.device)
+        pred = torch.empty((Q, N), dtype=torch.int32, device=self.device)
+        goal_pred, a_s, a_g = [torch.empty((Q,), dtype=torch.int32, device=self.device) for _ in range(3)]
+        length = torch.empty((Q,), dtype=torch.float64, device=self.device)
+        self._call("roadmap_sssp", None, Q, N, (A - 1) // 2, E, *[self._ptr(x) for x in (
+            row_ptr, dst, weight, att_vertex, att_weight, dist, pred, goal_pred, length, a_s, a_g)])
+        return dist, pred, goal_pred, length, a_s, a_g
+
+    def roadmap_paths(self, vq, vcube, row_ptr, dst, ns, step_ptr, steps, q_init, q_goal, cube0, cube1, att_vertex,
+                      att_weight, att_ns, att_path, pred, goal_pred):
+        """The paths of a query batch from roadmap_sssp's pred / goal_pred (gik_roadmap_paths_*, semantics in
+        include/gik.h): roadmap vq [N,nq], vcube [N,12], row_ptr / dst / ns / step_ptr / steps [rows,nq]; queries q_init /
+        q_goal [Q,nq], cube0 / cube1 [Q,12]; attachment slots att_vertex / att_ns int32 and att_weight float64 [Q, A],
+        att_path [S][nq][Q*A].  -> (q [total,nq], cube [total,12], offsets int64 [Q+1], vertices int32 [Q]).  One host
+        synchronisation (reading the total)."""
+        ft = vq.dtype
+        vq = self._arg(vq, (None, self.nq), ft, "vq", copy=True)
+        N = vq.shape[0]
+        vcube = self._arg(vcube, (N, 12), ft, "vcube", copy=True)
+        row_ptr, dst, ns = self._csr(row_ptr, dst, ns=ns)
+        if row_ptr.shape[0] != N + 1:
+            raise ValueError(f"row_ptr: expected shape [{N + 1}], got {list(row_ptr.shape)}")
+        E = dst.shape[0]
+        step_ptr = self._arg(step_ptr, (E + 1,), torch.int64, "step_ptr", copy=True)
+        steps = self._arg(steps, (None, self.nq), ft, "steps", copy=True)
+        q_init = self._arg(q_init, (None, self.nq), ft, "q_init", copy=True)
+        Q = q_init.shape[0]
+        q_goal = self._arg(q_goal, (Q, self.nq), ft, "q_goal", copy=True)
+        cube0 = self._arg(cube0, (Q, 12), ft, "cube0", copy=True)
+        cube1 = self._arg(cube1, (Q, 12), ft, "cube1", copy=True)
+        att_vertex = self._arg(att_vertex, (Q, None), torch.int32, "att_vertex", copy=True)
+        A = att_vertex.shape[1]
+        if A % 2 != 1:
+            raise ValueError(f"att_vertex: expected 2 * k_attach + 1 slots per query, got {A}")
+        att_weight = self._arg(att_weight, (Q, A), torch.float64, "att_weight", copy=True)
+        att_ns = self._arg(att_ns, (Q, A), torch.int32, "att_ns", copy=True)
+        att_path = self._arg(att_path, (None, self.nq, Q * A), ft, "att_path", copy=True)
+        pred = self._arg(pred, (Q, N), torch.int32, "pred", copy=True)
+        goal_pred = self._arg(goal_pred, (Q,), torch.int32, "goal_pred", copy=True)
+        offsets = torch.zeros((Q + 1,), dtype=torch.int64, device=self.device)
+        vertices = torch.zeros((Q,), dtype=torch.int32, device=self.device)
+        head = [Q, N, (A - 1) // 2, att_path.shape[0], E] + [self._ptr(x) for x in (
+            vq, vcube, row_ptr, dst, ns, step_ptr, steps if steps.numel() else None, q_init, q_goal, cube0, cube1,
+            att_vertex, att_weight, att_ns, att_path, pred, goal_pred, offsets, vertices)]
+        self._call("roadmap_paths", ft, *head, None, None)
+        total = int(offsets[-1].item()) if Q else 0
+        q = torch.empty((total, self.nq), dtype=ft, device=self.device)
+        cube = torch.empty((total, 12), dtype=ft, device=self.device)
+        if total:
+            self._call("roadmap_paths", ft, *head, self._ptr(q), self._ptr(cube))
+        return q, cube, offsets, vertices
 
     def cube_collision_soa(self, cube_pose_soa: torch.Tensor) -> torch.Tensor:
         """The cube's own collision test (cube vs table / obstacle, path.py:51-52): cube_pose [12][n] -> u8 [n]."""
