@@ -1,7 +1,7 @@
 """Scalar device functions checked without a GPU.  atan2_pos: the host build of csrc/gik_core.cuh runs the same
 polynomial as the device.  fp64 sincos: device-only code (constant-bank coefficients), so its algorithm is re-executed
 here in numpy from the coefficients PARSED OUT of the header -- an edited coefficient or reduction constant fails this
-test before it reaches a GPU (on the box tools/probes/f64_trig.cu measures the real thing against the CUDA library)."""
+test before it reaches a GPU (test_gpu_device_functions.py measures the device forms themselves on the GPU)."""
 import os
 import re
 
